@@ -11,6 +11,9 @@ one rkFDUpdate for every environment (5 dynamics evaluations + RKG combination, 
   python bench.py --impl reference --gpus N --steps K ...    the CPU restatement of the reference on all
                                                              host cores (the reference itself is un-buildable
                                                              here: ZEDA/ZM/Zeo/RoKi absent)
+  python bench.py ... --dump-outputs DIR                     also writes what the last timed step computed as
+                                                             DIR/<name>.npy (seeded inputs: runs of two builds
+                                                             compare output for output)
 Prints ONE JSON line on rank 0.
 """
 import argparse
@@ -50,7 +53,8 @@ def _default_states(world, ch, B, seed):
 # BASELINE.json configurations that fit one GPU (SURVEY.md section 8d).  Per config: the world, environments per GPU,
 # untimed settle steps from the synthetic initial states, ALGORITHMIC bytes / flop per env-step (section 8d's figures; None
 # where the survey gives no closed formula), the CPU samples (environments per host core, steps) of the cpu_baseline leg
-# and of one "step" of the reference arm.  C3 is the configuration BASELINE.json's metric is quoted on: the default.
+# and of one "step" of the reference arm; `slow` marks steps of tens of ms.  C3 is the configuration BASELINE.json's metric
+# is quoted on: the default.
 CONFIGS = {
     "C2": dict(label="C2: arm7 (7-DoF, DC motors, joint friction), no contact (pure ABA kernel)",
                world=lambda ch: ch.world_c2(), envs=65536, settle=0, states=_default_states,
@@ -60,12 +64,12 @@ CONFIGS = {
                alg_bytes=1054.0, alg_flop=20471.0, cpu=(1024, 400), ref=(512, 100)),
     "C4": dict(label="C4: legged tree (floating trunk + two 3-joint legs, 12 DoF, box soles) standing, volume-based contact (rkfd_volume)",
                world=lambda ch: ch.world_c4_volume(), envs=131072, settle=10, states=_c4_states,
-               alg_bytes=66.0 * 12 + 74.0 * 16, alg_flop=None, cpu=(8, 40), ref=(4, 10), max_steps=10),
+               alg_bytes=66.0 * 12 + 74.0 * 16, alg_flop=None, cpu=(8, 40), ref=(4, 10), slow=True),
     "C4-mighty": dict(label="C4 on the reference's own model: mighty.ztk (25 links, 26 DoF, 701 collision vertices; tests/golden/flat_mighty_on_floor.txt) "
                             "standing on floor.ztk, volume-based contact (rkfd_volume) on the soles",
                       world=lambda ch: ch.world_from_flat(ch.load_flat(os.path.join(ROOT, "tests", "golden", "flat_mighty_on_floor.txt"))),
                       envs=32768, settle=10, states=lambda world, ch, B, seed: _mighty_states(world, ch, B, seed),
-                      alg_bytes=66.0 * 26 + 74.0 * 701, alg_flop=None, cpu=(8, 40), ref=(4, 10), max_steps=10),
+                      alg_bytes=66.0 * 26 + 74.0 * 701, alg_flop=None, cpu=(8, 40), ref=(4, 10), slow=True),
     "C5-mlcp": dict(label="C5: arm7 + 8-vertex cube on the rigid floor (K=1000, L=1e-4), MLCP/PGS max_iter=10; 1M envs over 8 GPUs = 131,072 per GPU",
                     world=lambda ch: ch.world_c5(base_z=0.45, solver="MLCP"), envs=131072, settle=500, states=_default_states,
                     alg_bytes=1054.0, alg_flop=106191.0, cpu=(256, 400), ref=(128, 100)),
@@ -166,6 +170,35 @@ class ClockSampler:
         if self.note:
             out["note"] = self.note
         return out
+
+
+DUMP_BYTES = 64 * 10**6      # --dump-outputs: all files together, .npy headers included
+
+
+def step_outputs(fd, world):
+    """What a caller of the step path reads back after a step, one row per environment: the state (rkFDBatchGetState),
+    the status word and, in worlds with contact slots, the contact state and forces."""
+    q, qd, qdd = fd.batch_get_state()
+    out = {"q": q, "qd": qd, "qdd": qdd, "status": fd.batch_get_status()}
+    if world.nslot:
+        out["contact_active"], out["contact_type"], out["contact_ref"], out["contact_force"] = fd.batch_get_contact()
+    return out
+
+
+def dump_outputs(path, arrays, seed=SEED):
+    """Writes `arrays` (first axis: environment) as <path>/<name>.npy in float64, with env_index.npy naming the environments
+    written.  Beyond DUMP_BYTES in all, every array keeps the same fixed sample of environments (drawn from `seed`)."""
+    B = len(next(iter(arrays.values())))
+    per_env = 8 * (1 + sum(a[0].size for a in arrays.values()))
+    room = DUMP_BYTES - 4096 * (len(arrays) + 1)
+    idx = np.arange(B)
+    if B * per_env > room:
+        idx = np.sort(np.random.default_rng(seed).choice(B, room // per_env, replace=False))
+    out = {name: np.asarray(a, np.float64)[idx] for name, a in arrays.items()}
+    out["env_index"] = idx.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def cpu_settled_state(world, ch, cfg, n_envs, seed=SEED):
@@ -326,14 +359,16 @@ def main():
     ap.add_argument("--e2e-upload-state", action="store_true", help="e2e leg: also re-send (q, q') host->device every step")
     ap.add_argument("--e2e-outputs", default="q,qd", help="e2e leg: what the caller reads back every step, of q,qd,qdd (default q,qd: what the "
                     "feedback loop of the reference's example/chain/arm_box_test.c:10-23 reads - rkJointGetDis/GetVel - before it sets the motor inputs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed (state, status, contacts of rank 0's "
+                    "environments; a fixed sample of them beyond 64 MB) as DIR/<name>.npy in float64")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA engine (--impl b200)")
     if args.impl == "reference":
         return run_reference(args, emit)
     if args.warmup < 3:
         args.warmup = 3
     cfg = CONFIGS[args.config]
-    if cfg.get("max_steps"):
-        args.steps = min(args.steps, cfg["max_steps"])      # 38 ms-class steps: keep the default run within minutes
 
     import torch
     import rokifd_b200  # noqa: F401
@@ -392,11 +427,12 @@ def main():
     resorts = fd.resort_count - r0
     resort_kernels = fd.resort_kernel_count - rk0
     sampler.mark_end()
+    outputs = step_outputs(fd, world) if args.dump_outputs and rank == 0 else None     # before any further step
     if sampler.loaded_samples() == 0:
         # nvidia-smi delivered nothing inside the timed region (slow start): keep the same load on the device until it does
         t_wait = time.time()
         while sampler.loaded_samples() == 0 and time.time() - t_wait < 5.0:
-            fd.update_n(100 if not cfg.get("max_steps") else 5); torch.cuda.synchronize()
+            fd.update_n(5 if cfg.get("slow") else 100); torch.cuda.synchronize()
         sampler.mark_end()
         sampler.note = "no nvidia-smi sample fell inside the loaded region (settle + warm-up + timed steps); sampled under the same load right after it"
     clocks = sampler.stop()
@@ -530,6 +566,8 @@ def main():
             pass
         assert host_threads() == affinity0
         out["cpu_baseline"] = cpu_baseline_leg(world, ch, cfg)
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     fd.destroy()
     if rank == 0:
         emit(out)

@@ -1,8 +1,8 @@
 """Writes tests/golden/flat_<world>.txt: what the C-ABI (rkFDChainRegFile / rkFDContactInfoScanFile + the flattening of
-rkFDUpdateInit) makes of the reference's own example/model/*.ztk files, as text (`RkFD.describe_model()`).  The GPU box has
-no /root/reference, so the `-m gpu` parity tests load these tables (`chains.world_from_flat`); tests/test_capi_host.py checks
-here, where the reference tree exists, that they are what the files flatten to.  Run from the repo root:
-    python tests/golden/make_flat_models.py"""
+rkFDUpdateInit) makes of the reference's own example/model/*.ztk files, as text (`RkFD.describe_model()`).  The repository
+does not contain the reference, so the tests load these tables (`chains.world_from_flat`); tests/test_capi_host.py checks,
+when ROKIFD_REFERENCE names a reference tree, that they are what its files flatten to.  Run from the repo root:
+    ROKIFD_REFERENCE=<path of a mi-lib/roki-fd checkout> python tests/golden/make_flat_models.py"""
 import os
 import sys
 

@@ -45,6 +45,55 @@ def test_reference_arm_uses_every_host_thread_under_torchrun():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+def test_dump_outputs_keeps_a_fixed_sample_within_64_mb(tmp_path):
+    """--dump-outputs beyond its budget: every array keeps the same seeded sample of environments, in float64, and two
+    dumps of the same outputs are identical file for file."""
+    import numpy as np
+    import bench
+    B = 400000
+    arrays = {"q": np.random.default_rng(1).normal(size=(B, 7)), "status": np.arange(B, dtype=np.int32),
+              "contact_force": np.random.default_rng(2).normal(size=(B, 8, 3))}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    files = sorted(f.name for f in (tmp_path / "a").iterdir())
+    assert files == ["contact_force.npy", "env_index.npy", "q.npy", "status.npy"]
+    assert sum((tmp_path / "a" / f).stat().st_size for f in files) <= 64 * 10**6
+    got = {f[:-4]: np.load(tmp_path / "a" / f) for f in files}
+    idx = got["env_index"].astype(np.int64)
+    assert 0 < len(idx) < B and (np.diff(idx) > 0).all()
+    for name, a in arrays.items():
+        assert got[name].dtype == np.float64 and np.array_equal(got[name], a[idx])
+    assert all(np.array_equal(np.load(tmp_path / "b" / f), got[f[:-4]]) for f in files)
+
+
+def test_dump_outputs_below_the_budget_keeps_every_environment(tmp_path):
+    import numpy as np
+    import bench
+    q = np.arange(12.0).reshape(4, 3)
+    bench.dump_outputs(str(tmp_path), {"q": q})
+    assert np.array_equal(np.load(tmp_path / "q.npy"), q) and np.array_equal(np.load(tmp_path / "env_index.npy"), np.arange(4.0))
+
+
+@pytest.mark.gpu
+def test_gpu_arm_dump_outputs_and_steps(tmp_path):
+    """With the same arguments two runs dump identical outputs of their last timed step; --steps sets the number of timed
+    steps, in the slow configurations too."""
+    import numpy as np
+    dumps = []
+    for k in range(2):
+        d = run("--steps", "12", "--warmup", "3", "--envs", "32768", "--no-cpu-baseline", "--dump-outputs", str(tmp_path / str(k)))
+        assert d["steps"] == 12 and d["gpu_launches_detail"]["rkfd_step_kernel"] == 12
+        dumps.append({f.name: np.load(f) for f in (tmp_path / str(k)).iterdir()})
+    assert set(dumps[0]) == {"q.npy", "qd.npy", "qdd.npy", "status.npy", "contact_active.npy", "contact_type.npy", "contact_ref.npy",
+                             "contact_force.npy", "env_index.npy"}
+    assert dumps[0]["q.npy"].shape == (32768, 7) and dumps[0]["contact_force.npy"].shape == (32768, 8, 3)
+    assert np.isfinite(dumps[0]["q.npy"]).all() and (dumps[0]["status.npy"] == 0).all()
+    for name, a in dumps[0].items():
+        assert a.dtype == np.float64 and np.array_equal(a, dumps[1][name]), name
+    d = run("--steps", "12", "--warmup", "3", "--config", "C4", "--envs", "4096", "--no-cpu-baseline")
+    assert d["steps"] == 12 and d["gpu_launches_detail"]["rkfd_step_kernel"] == 12
+
+
 @pytest.mark.gpu
 @pytest.mark.parametrize("config", ["C2", "C5-mlcp", "C5-vert", "C4"])
 def test_gpu_arm_other_configs(config):

@@ -59,21 +59,27 @@ def test_c_caller_matches_oracle(tmp_path, oracle, solver, contacts, z0, cube):
 
 
 # ---- the reference's own example programs, compiled UNMODIFIED ---------------------------------------------------------
-REF_EX = "/root/reference/example/chain"
-REF_BUILD = os.path.join(ROOT, "tests", "c_callers", "_ref_build")      # git-ignored; travels to the GPU box with the snapshot
+# they come from a source tree of the reference (mi-lib/roki-fd) that ROKIFD_REFERENCE names; the repository holds none of them
+REF = os.environ.get("ROKIFD_REFERENCE", "")
+REF_EX = os.path.join(REF, "example", "chain")
+needs_reference = pytest.mark.skipif(not REF or not os.path.isdir(REF_EX), reason="no reference tree (set ROKIFD_REFERENCE)")
 EXAMPLES = ["boxdrop_hardsoft_test", "boxdrop_test", "arm_box_test", "arm_box_trq_test", "arm_wall_test"]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_EX), reason="reference tree not present")
-@pytest.mark.parametrize("name", EXAMPLES)
-def test_reference_examples_compile_unmodified(name):
-    """example/chain/*.c of the reference, straight from /root/reference (nothing is copied into the repo), against
-    include/roki_fd/roki_fd.h and librokifd_b200.so: every type, macro and function they touch exists (rkFD by value,
-    rkFDSetSolver / rkFDODE2Assign* macros, rkChain / rkJoint accessors, zVec, zRandF, eprintf, zVecFPrint ...)."""
-    os.makedirs(REF_BUILD, exist_ok=True)
-    exe = os.path.join(REF_BUILD, name)
+def build_reference_example(name, outdir):
+    exe = os.path.join(str(outdir), name)
     subprocess.check_call(["gcc", "-std=gnu99", "-I" + os.path.join(ROOT, "include"), os.path.join(REF_EX, name + ".c"),
                            "-L" + LIBDIR, "-lrokifd_b200", "-Wl,-rpath," + LIBDIR, "-o", exe])
+    return exe
+
+
+@needs_reference
+@pytest.mark.parametrize("name", EXAMPLES)
+def test_reference_examples_compile_unmodified(tmp_path, name):
+    """example/chain/*.c of the reference, straight from its tree (nothing is copied into the repo), against
+    include/roki_fd/roki_fd.h and librokifd_b200.so: every type, macro and function they touch exists (rkFD by value,
+    rkFDSetSolver / rkFDODE2Assign* macros, rkChain / rkJoint accessors, zVec, zRandF, eprintf, zVecFPrint ...)."""
+    exe = build_reference_example(name, tmp_path)
     needed = subprocess.check_output(["readelf", "-d", exe], text=True)
     assert "librokifd_b200.so" in needed and "libcuda" not in needed
 
@@ -89,15 +95,17 @@ def _splitmix(seed):
 
 
 @pytest.mark.gpu
-def test_reference_boxdrop_hardsoft_runs_unmodified(oracle):
-    """The reference's example/chain/boxdrop_hardsoft_test.c (compiled unmodified in the container by the test above; the
-    binary travels with the snapshot) dropping ONE box (argv[1] = 1) on the hard/soft floor under the Volume solver: it opens
-    ../model/{contactinfo,box,floor_hardsoft}.ztk (builder-authored stand-ins with the reference's constants under
-    tests/c_callers/model), steps 5 s and prints the joint displacements every step; compared with the oracle."""
-    exe = os.path.join(REF_BUILD, "boxdrop_hardsoft_test")
-    if not os.path.exists(exe):
-        pytest.skip("built where the reference tree exists (tests/c_callers/_ref_build)")
-    cwd = os.path.join(ROOT, "tests", "c_callers", "chain")
+@needs_reference
+def test_reference_boxdrop_hardsoft_runs_unmodified(tmp_path, oracle):
+    """The reference's example/chain/boxdrop_hardsoft_test.c (compiled unmodified as in the test above) dropping ONE box
+    (argv[1] = 1) on the hard/soft floor under the Volume solver: it opens ../model/{contactinfo,box,floor_hardsoft}.ztk
+    (stand-ins with the reference's constants under tests/c_callers/model), steps 5 s and prints the joint displacements
+    every step; compared with the oracle."""
+    import shutil
+    exe = build_reference_example("boxdrop_hardsoft_test", tmp_path)
+    shutil.copytree(os.path.join(ROOT, "tests", "c_callers", "model"), tmp_path / "model")
+    cwd = tmp_path / "chain"
+    cwd.mkdir()
     seed = 12345
     subprocess.run([exe, "1"], cwd=cwd, env=dict(os.environ, ROKIFD_ZRAND_SEED=str(seed)), check=True,
                    stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL, timeout=600)

@@ -13,6 +13,10 @@ from rokifd_b200 import capi, chains as ch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 GOLD = os.path.join(ROOT, "tests", "golden")
+# a source tree of the reference (mi-lib/roki-fd), when ROKIFD_REFERENCE names one: the tests that read its own files run then
+REF = os.environ.get("ROKIFD_REFERENCE", "")
+REF_MODELS = os.path.join(REF, "example", "model")
+needs_reference = pytest.mark.skipif(not REF or not os.path.isdir(REF_MODELS), reason="no reference tree (set ROKIFD_REFERENCE)")
 
 
 def test_library_exports_every_declared_symbol():
@@ -106,10 +110,10 @@ def test_ztk_reader():
     fd.destroy()
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/example/model"), reason="reference tree not present")
+@needs_reference
 def test_ztk_reader_on_reference_models():
     """The reader accepts the reference's own model files unmodified (SURVEY.md section 8f.1)."""
-    d = "/root/reference/example/model"
+    d = REF_MODELS
     expect = {"box.ztk": (1, 6), "floor.ztk": (1, 0), "floor_hardsoft.ztk": (2, 0), "arm_2DoF.ztk": (3, 2),
               "arm_2DoF_trq.ztk": (3, 2), "puma.ztk": (7, 6), "mighty.ztk": (25, 26), "arm.ztk": (6, 12), "dualarm.ztk": (None, None),
               "wall.ztk": (4, 18), "crawler.ztk": (None, None), "box_small.ztk": (1, 6)}      # wall.ztk: three breakable float joints
@@ -166,7 +170,7 @@ REF_SLIDES = {"crawler_on_hardsoft": [(0, 1, 0, 0.3, (0.0, 1.0, 0.0)), (0, 2, 0,
 
 
 def reference_world_description(name):
-    d = "/root/reference/example/model"
+    d = REF_MODELS
     files, solver = REF_WORLDS[name]
     fa = capi.RkFD()
     assert fa.contact_info_scan_file(os.path.join(d, "contactinfo.ztk"))
@@ -187,7 +191,12 @@ def reference_world_description(name):
     return desc
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/example/model"), reason="reference tree not present")
+def flat_description(name):
+    """tests/golden/flat_<name>.txt: the device model the reference's own files of world `name` flatten to (written by
+    tests/golden/make_flat_models.py from a reference tree; checked against it by the test below when one is given)."""
+    return ch.load_flat(os.path.join(GOLD, "flat_%s.txt" % name))
+
+
 @pytest.mark.parametrize("name", list(REF_WORLDS))
 def test_reference_model_files_flatten_and_round_trip(name):
     """The reference's own model files, registered through rkFDChainRegFile / rkFDContactInfoScanFile, flatten to a device
@@ -196,25 +205,26 @@ def test_reference_model_files_flatten_and_round_trip(name):
     written by tests/golden/make_flat_models.py from these files) IS what the C-ABI makes of the reference's files."""
     if name == "arm2dof_on_floor":
         pytest.skip("152 contact slots: the rigid vertex solvers take 32")
-    desc = reference_world_description(name)
+    desc = flat_description(name)
+    if REF and os.path.isdir(REF_MODELS):
+        _same_model(reference_world_description(name), desc)
     fb, _ = capi.create_world(ch.world_from_flat(desc), B=1)
     _same_model(desc, _flattened(fb))
     fb.destroy()
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/example/model"), reason="reference tree not present")
 def test_reference_model_files_match_the_transcribed_worlds():
-    """rokifd_b200.chains transcribes box.ztk / floor*.ztk / arm_2DoF.ztk / contactinfo.ztk by hand (the GPU box has no
-    /root/reference): the transcriptions flatten to the same tables as the files (arm_2DoF: link tables; its collision
-    shapes are not transcribed)."""
-    _same_model(reference_world_description("boxdrop_hardsoft"), _flattened(capi.create_world(ch.world_c1_box(), B=1)[0]))
-    fa = capi.RkFD()
-    assert fa.chain_reg_file("/root/reference/example/model/arm_2DoF.ztk") is not None
-    ma, mb = _flattened(fa), _flattened(capi.create_world(ch.world_c1_serial(), B=1)[0])
+    """rokifd_b200.chains transcribes box.ztk / floor*.ztk / arm_2DoF.ztk / contactinfo.ztk by hand: the transcriptions
+    flatten to the same tables as the files (tests/golden/flat_*.txt; arm_2DoF: the link tables of the arm in
+    arm_box_floor, where it is registered first; its collision shapes are not transcribed)."""
+    _same_model(flat_description("boxdrop_hardsoft"), _flattened(capi.create_world(ch.world_c1_box(), B=1)[0]))
+    mb = _flattened(capi.create_world(ch.world_c1_serial(), B=1)[0])
+    ma = {k: v for k, v in flat_description("arm_box_floor").items() if k in mb}
     for m in (ma, mb):
         for k in m:
             if k.startswith("link.topo"):
                 m[k] = m[k][:5]            # parent, joint type, motor type, dofs, offset (not the cell range)
+    assert all("link.mass[%d]" % i in ma for i in range(3))
     _same_model(ma, mb, keys={"link.topo", "link.Ro", "link.po", "link.mass", "link.joint"})
 
 
@@ -279,11 +289,11 @@ def test_ztk_shape_sugar_and_automatic_mass_properties():
     assert np.allclose(Ic, tot, atol=1e-14)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/example/model"), reason="reference tree not present")
+@needs_reference
 def test_ztk_reader_fills_the_gaps_of_the_reference_models():
     """puma.ztk's loop/prism shapes give collision vertices, arm.ztk's `COM: auto` links get mass properties, no shape of
     the reference's model directory is dropped."""
-    d = "/root/reference/example/model"
+    d = REF_MODELS
     fd = capi.RkFD(); assert fd.chain_reg_file(os.path.join(d, "puma.ztk")) is not None
     m = _flattened(fd); fd.destroy()
     assert int(m["dims"][2]) == 7 and int(m["dims"][6]) > 300           # 7 cells: base, post, shoulder, upperarm, forearm, hand ...
@@ -301,9 +311,10 @@ def test_volume_kernel_keeps_its_warp_barriers():
     WARPSYNC) at the candidate loop and before the friction LPs.  Checked on the object file the build leaves in-tree."""
     import shutil, subprocess
     obj = os.path.join(os.path.dirname(capi.LIB_PATH), "csrc", "build", "rkfd_kernel_256_1_1_0_1.o")
-    if shutil.which("cuobjdump") is None or not os.path.exists(obj):
+    cuobjdump = shutil.which("cuobjdump") or shutil.which("cuobjdump", path=os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin"))
+    if cuobjdump is None or not os.path.exists(obj):
         pytest.skip("no cuobjdump / no object file of the Volume variant")
-    sass = subprocess.run(["cuobjdump", "-sass", obj], capture_output=True, text=True, timeout=300).stdout
+    sass = subprocess.run([cuobjdump, "-sass", obj], capture_output=True, text=True, timeout=300).stdout
     assert sass.count("BRA.DIV") >= 3 and "WARPSYNC.EXCLUSIVE" in sass
     src = open(os.path.join(os.path.dirname(capi.LIB_PATH), "csrc", "rkfd_volume.cuh")).read()
     assert src.count("c.hsync()") >= 2 and "c.hany(ci < ncand)" in src
