@@ -146,8 +146,11 @@ RKFD_HD S3 sym3_inverse(const S3 &d){
 template <int JT_, int CLS_, int ROOT_> struct LinkTag { static constexpr int jt = JT_, cls = CLS_, root = ROOT_; };
 using TagRT = LinkTag<-1, -1, -1>;
 
+/* FUSE = 1: pass 3 of a stage and pass 1 of the next walk the links together (Core::outward) - serial arms without rigid
+ * pairs, whose link i depends on link i-1 only; the generic kernel keeps the passes apart (tree worlds share branch slots
+ * between pass 1 and pass 3) */
 struct SpecGeneric {
-  static constexpr int ID = 0, NL = 0, UNROLL = 1, NSCRATCH = 0, ROLL = 0;
+  static constexpr int ID = 0, NL = 0, UNROLL = 1, NSCRATCH = 0, ROLL = 0, FUSE = 0;
   static RKFD_HD int nl(const ModelDev &m){ return m.nl; }
   static RKFD_HD int jtype(int, const LinkDev &L){ return L.jtype; }
   static RKFD_HD int parent(int, const LinkDev &L){ return L.parent; }
@@ -180,7 +183,7 @@ constexpr int SPEC_GENERIC_TM = 11, SPEC_GENERIC_TM_MAX_T = 128;
  * in warp-uniform code. */
 template <int ID_, int NL_, unsigned CLS_, int TM_>
 struct SpecSerialRev {
-  static constexpr int ID = ID_, NL = NL_, UNROLL = NL_, TM = TM_, ROLL = 0, SCS = 0, TCOLS = 128;
+  static constexpr int ID = ID_, NL = NL_, UNROLL = NL_, TM = TM_, ROLL = 0, SCS = 0, TCOLS = 128, FUSE = 1;
   static constexpr int WEXT = TM_ ? 6*NL_ : 6 + 10*(NL_-1);
   static constexpr int RK = TM_ ? 4*(NL_-1) : WEXT + 6;                 /* T space when TM_ */
   static constexpr int NSCRATCH = TM_ ? WEXT + 6 : RK + 4*(NL_-1);     /* shared-memory doubles per environment */
@@ -216,7 +219,7 @@ struct SpecSerialRev {
  * quarter-turn forms): every fixed-base serial revolute arm gets the rolled kernel, whatever its DH twists. */
 template <int ID_, int NL_, int RG_ = 0, int GEN_ = 0>
 struct SpecSerialRevRolled {
-  static constexpr int ID = ID_, NL = NL_, UNROLL = 1, TM = 1, ROLL = 1, RG = RG_, RCLS = GEN_ ? RO_GENERAL : RO_RXS;
+  static constexpr int ID = ID_, NL = NL_, UNROLL = 1, TM = 1, ROLL = 1, RG = RG_, RCLS = GEN_ ? RO_GENERAL : RO_RXS, FUSE = !RG_;
   /* RG: (sin, cos, 1/D, u) stay in the shared-memory column (SCS): the contact solve reads them for OTHER lanes'
    * environments (lane-parallel probes) and in divergent code, which tensor memory allows neither */
   static constexpr int SCS = RG_, TCOLS = 128;
@@ -343,8 +346,15 @@ struct Core {
   int bad;
   unsigned wk = 0;              /* work class of the last rigid solve (StateDev::work) */
   int rk0;                      /* first slot of the integrator stage state (QS, QDS, PQ, PQD) */
+  /* committed state (buffer `cur` of StateDev::q/qd) and the output buffer, where the running combination of a step becomes
+   * the next committed state; selected once, swapped when a step commits.  Indexing StateDev::q with the run-time `cur` at
+   * every access instead makes nvcc keep a copy of the whole StateDev on the stack and reload the pointers from there. */
+  double *qc, *qdc, *qn, *qdn;
 
-  RKFD_HD explicit Core(Ctx &ctx) : c(ctx), piv(0), cfl(0), cw(0), bad(0), rk0(0) {}
+  RKFD_HD explicit Core(Ctx &ctx) : c(ctx), piv(0), cfl(0), cw(0), bad(0), rk0(0),
+    qc(ctx.cur ? ctx.st.q[1] : ctx.st.q[0]), qdc(ctx.cur ? ctx.st.qd[1] : ctx.st.qd[0]),
+    qn(ctx.cur ? ctx.st.q[0] : ctx.st.q[1]), qdn(ctx.cur ? ctx.st.qd[0] : ctx.st.qd[1]) {}
+  RKFD_HD void commit_swap(){ double *t = qc; qc = qn; qn = t; t = qdc; qdc = qdn; qdn = t; }
 
   /* the flag word the following code works on (warp-uniform: decided by the model) */
   RKFD_HD void flag_select(int w){
@@ -714,100 +724,116 @@ struct Core {
    * not formed): no gravity direction to propagate outward, no gravity terms in the bias forces. */
   static RKFD_HD bool grav_acc(const ModelDev &m){ return Spec::NL != 0 ? true : !m.has_rigid; }
 
-  /* `fresh`: sin/cos of the revolute joints are computed from the stage angle (first stage of a step, single
-   * evaluations); otherwise pass 3 of the previous stage has already rotated them to the new stage angle */
-  RKFD_HD void pass1(const ModelDev &m, bool ref, bool fresh){
+  /* pass-1 values carried outward: world frame, linear velocity (link axes) and angular velocity of the parent link, gravity direction */
+  struct Kin { M3 Rw; V3 pw, vl, om, gd; };
+  static RKFD_HD void kin_init(Kin &k){ k.Rw = ident3(); k.pw = v3(0,0,0); k.vl = v3(0,0,0); k.om = v3(0,0,0); k.gd = v3(0,0,-GRAVITY); }
+  /* sin, cos and velocity of revolute joint i from the T space.  `fresh`: sin/cos are computed from the stage angle (first
+   * stage of a step, single evaluations) and stored for the passes that follow; otherwise pass 3 of the previous stage has
+   * already rotated them to the new stage angle */
+  RKFD_HD void revol_state(const ModelDev &m, int i, bool fresh, double &sn, double &co, double &wz){
+    const LinkDev &L = m.link[i]; const int qo = Spec::qofs(i,L);
+    if( fresh ){ sincos(T(rk0+qo), &sn, &co); Qw(Spec::sc(i,L), sn); Qw(Spec::sc(i,L)+1, co); }
+    else Q2(Spec::sc(i,L), sn, co);
+    wz = T(rk0 + Spec::nq(m) + qo);
+  }
+  /* pass 1 at link i.  A revolute joint's (sin, cos, q') are handed in by the caller (revol_state, or pass 3 of the previous
+   * stage in Core::outward).  `cont`: the contacts of the link's cells run here (false: the caller runs them after the loop) */
+  template <class Kt>
+  RKFD_HD void pass1_link(const ModelDev &m, int i, Kin &k, bool ref, double sn, double co, double wz, bool cont){
     const bool gacc = grav_acc(m);
-    M3 Rw = ident3(); V3 pw = v3(0,0,0), vl = v3(0,0,0), om = v3(0,0,0), gd = v3(0,0,-GRAVITY);
     const int qs = rk0, qds = rk0 + Spec::nq(m);
+    const LinkDev &L = m.link[i]; const int sl = Spec::slot(i,L), qo = Spec::qofs(i,L);
+    if( !SER<Kt>(i,L) ){
+      if( ROOT<Kt>(i,L) ) kin_init(k);
+      else {
+        const LinkDev &P = m.link[L.parent];
+        k.om = ld3(P.wslot); k.gd = ld3(P.wslot+3);
+        if( m.need_world ){ k.Rw = ldm(P.branch_slot); k.pw = ld3(P.branch_slot+9); k.vl = ld3(P.branch_slot+12); }
+      }
+    }
+    XF x; x.fast = 0; x.cls = CLS<Kt>(i,L); x.sg = ro_sign(x.cls, L.rsg); x.c = 1.0; x.s = 0.0;
+    x.pz = L.pz;      /* revolute / fixed joint with org position (0, 0, z): decided once on the host (rkfd_model.cpp) */
+    V3 vJ = v3(0,0,0), wJ = v3(0,0,0);
+    switch(JT<Kt>(i,L)){
+    case J_REVOL: {
+      x.s = sn; x.c = co; x.p = org_p(L);
+      if( CLS<Kt>(i,L) != RO_GENERAL ) x.fast = 1;
+      else { const M3 Ro = org_R(L); const V3 o0 = col0(Ro), o1 = col1(Ro);
+        x.R = from_cols(co*o0 + sn*o1, co*o1 - sn*o0, col2(Ro)); }
+      wJ.z = wz;
+    } break;
+    case J_PRISM: x.R = org_R(L); x.p = org_p(L) + T(qs+qo)*col2(x.R); vJ.z = T(qds+qo); break;
+    case J_SPHER: {
+      const M3 Ro = org_R(L);
+      x.R = mm(Ro, aa_to_mat(t3(qs+qo))); x.p = org_p(L);
+      stm(sl+27, x.R);
+      wJ = tmul(x.R, mul(Ro, t3(qds+qo)));
+    } break;
+    case J_FLOAT: {
+      const M3 Ro = org_R(L);
+      x.R = mm(Ro, aa_to_mat(t3(qs+qo+3))); x.p = org_p(L) + mul(Ro, t3(qs+qo));
+      stm(sl+6, x.R); st3(sl+15, x.p);
+      vJ = tmul(x.R, mul(Ro, t3(qds+qo))); wJ = tmul(x.R, mul(Ro, t3(qds+qo+3)));
+    } break;
+    case J_BRFLOAT: {
+      const M3 Ro = org_R(L); const bool brk = (piv >> qo) & 1u;
+      x.R = mm(Ro, aa_to_mat(t3(qs+qo+3))); x.p = org_p(L) + mul(Ro, t3(qs+qo));
+      stm(sl+6, x.R); st3(sl+15, x.p); c.S(sl+45) = brk ? 1.0 : 0.0;
+      const V3 v = t3(qds+qo), w = t3(qds+qo+3);
+      if( brk ){ vJ = tmul(x.R, mul(Ro, v)); wJ = tmul(x.R, mul(Ro, w)); }
+    } break;
+    case J_CYLIN: {
+      const M3 Ro = org_R(L); double s1, c1; sincos(T(qs+qo+1), &s1, &c1);
+      const V3 o0 = col0(Ro), o1 = col1(Ro);
+      x.R = from_cols(c1*o0 + s1*o1, c1*o1 - s1*o0, col2(Ro)); x.p = org_p(L) + T(qs+qo)*col2(Ro);
+      stm(sl+17, x.R); st3(sl+26, x.p);
+      vJ.z = T(qds+qo); wJ.z = T(qds+qo+1);
+    } break;
+    case J_HOOKE: {
+      const M3 Ro = org_R(L); double s0, c0, s1, c1; sincos(T(qs+qo), &s0, &c0); sincos(T(qs+qo+1), &s1, &c1);
+      M3 RJ; RJ.xx = c0*c1; RJ.xy = -s0; RJ.xz = c0*s1; RJ.yx = s0*c1; RJ.yy = c0; RJ.yz = s0*s1; RJ.zx = -s1; RJ.zy = 0.0; RJ.zz = c1;
+      x.R = mm(Ro, RJ); x.p = org_p(L);
+      stm(sl+17, x.R); st3(sl+26, x.p); c.S(sl+29) = s1; c.S(sl+30) = c1;
+      const double v0 = T(qds+qo), v1 = T(qds+qo+1); wJ = v3(-s1*v0, v1, c1*v0);
+    } break;
+    default: x.R = org_R(L); x.p = org_p(L); break;
+    }
+    V3 om_n = xf_tmul(x, k.om);
+    if( JT<Kt>(i,L) == J_REVOL ) om_n.z += wJ.z; else om_n = om_n + wJ;      /* additions of literal zeros are not folded away */
+    if( m.need_world ){
+      V3 vl_n = xf_tmul(x, cadd_p(k.vl, k.om, x.p, x.pz));
+      if( JT<Kt>(i,L) != J_REVOL ) vl_n = vl_n + vJ;
+      k.pw = madd_p(k.pw, k.Rw, x.p, x.pz); k.Rw = xf_world(x, k.Rw); k.vl = vl_n;
+    }
+    k.om = om_n;
+    st3(Spec::wslot(i,L), k.om);
+    if( !gacc ){ k.gd = xf_tmul(x, k.gd); st3(Spec::wslot(i,L)+3, k.gd); }
+    const int wx = Spec::wext_slot(i,L), fs = Spec::frame_slot(i,L), bs = Spec::branch_slot(i,L);
+    if( cont && wx >= 0 ){
+      const V6 w = contacts(m, L, k.Rw, k.pw, k.vl, k.om, ref);
+      st3(wx, w.l); st3(wx+3, w.a);
+      if( fs >= 0 ){ stm(fs, k.Rw); st3(fs+9, k.pw); st3(fs+12, k.vl); st3(fs+15, k.om); }
+    }
+    if( bs >= 0 && m.need_world ){ stm(bs, k.Rw); st3(bs+9, k.pw); st3(bs+12, k.vl); }
+  }
+  /* `fresh`: as in revol_state */
+  RKFD_HD void pass1(const ModelDev &m, bool ref, bool fresh){
+    Kin k; kin_init(k);
     auto body = [&](const int i, auto Ktag){
       using Kt = decltype(Ktag);
-      const LinkDev &L = m.link[i]; const int sl = Spec::slot(i,L), qo = Spec::qofs(i,L);
       if( !Ctx::RIGID ) c.phase_sync(3);
-      if( !SER<Kt>(i,L) ){
-        if( ROOT<Kt>(i,L) ){ Rw = ident3(); pw = v3(0,0,0); vl = v3(0,0,0); om = v3(0,0,0); gd = v3(0,0,-GRAVITY); }
-        else {
-          const LinkDev &P = m.link[L.parent];
-          om = ld3(P.wslot); gd = ld3(P.wslot+3);
-          if( m.need_world ){ Rw = ldm(P.branch_slot); pw = ld3(P.branch_slot+9); vl = ld3(P.branch_slot+12); }
-        }
-      }
-      XF x; x.fast = 0; x.cls = CLS<Kt>(i,L); x.sg = ro_sign(x.cls, L.rsg); x.c = 1.0; x.s = 0.0;
-      x.pz = L.pz;      /* revolute / fixed joint with org position (0, 0, z): decided once on the host (rkfd_model.cpp) */
-      V3 vJ = v3(0,0,0), wJ = v3(0,0,0);
-      switch(JT<Kt>(i,L)){
-      case J_REVOL: {
-        double sn, co;
-        if( fresh ){ sincos(T(qs+qo), &sn, &co); Qw(Spec::sc(i,L), sn); Qw(Spec::sc(i,L)+1, co); }
-        else Q2(Spec::sc(i,L), sn, co);
-        x.s = sn; x.c = co; x.p = org_p(L);
-        if( CLS<Kt>(i,L) != RO_GENERAL ) x.fast = 1;
-        else { const M3 Ro = org_R(L); const V3 o0 = col0(Ro), o1 = col1(Ro);
-          x.R = from_cols(co*o0 + sn*o1, co*o1 - sn*o0, col2(Ro)); }
-        wJ.z = T(qds+qo);
-      } break;
-      case J_PRISM: x.R = org_R(L); x.p = org_p(L) + T(qs+qo)*col2(x.R); vJ.z = T(qds+qo); break;
-      case J_SPHER: {
-        const M3 Ro = org_R(L);
-        x.R = mm(Ro, aa_to_mat(t3(qs+qo))); x.p = org_p(L);
-        stm(sl+27, x.R);
-        wJ = tmul(x.R, mul(Ro, t3(qds+qo)));
-      } break;
-      case J_FLOAT: {
-        const M3 Ro = org_R(L);
-        x.R = mm(Ro, aa_to_mat(t3(qs+qo+3))); x.p = org_p(L) + mul(Ro, t3(qs+qo));
-        stm(sl+6, x.R); st3(sl+15, x.p);
-        vJ = tmul(x.R, mul(Ro, t3(qds+qo))); wJ = tmul(x.R, mul(Ro, t3(qds+qo+3)));
-      } break;
-      case J_BRFLOAT: {
-        const M3 Ro = org_R(L); const bool brk = (piv >> qo) & 1u;
-        x.R = mm(Ro, aa_to_mat(t3(qs+qo+3))); x.p = org_p(L) + mul(Ro, t3(qs+qo));
-        stm(sl+6, x.R); st3(sl+15, x.p); c.S(sl+45) = brk ? 1.0 : 0.0;
-        const V3 v = t3(qds+qo), w = t3(qds+qo+3);
-        if( brk ){ vJ = tmul(x.R, mul(Ro, v)); wJ = tmul(x.R, mul(Ro, w)); }
-      } break;
-      case J_CYLIN: {
-        const M3 Ro = org_R(L); double sn, co; sincos(T(qs+qo+1), &sn, &co);
-        const V3 o0 = col0(Ro), o1 = col1(Ro);
-        x.R = from_cols(co*o0 + sn*o1, co*o1 - sn*o0, col2(Ro)); x.p = org_p(L) + T(qs+qo)*col2(Ro);
-        stm(sl+17, x.R); st3(sl+26, x.p);
-        vJ.z = T(qds+qo); wJ.z = T(qds+qo+1);
-      } break;
-      case J_HOOKE: {
-        const M3 Ro = org_R(L); double s0, c0, s1, c1; sincos(T(qs+qo), &s0, &c0); sincos(T(qs+qo+1), &s1, &c1);
-        M3 RJ; RJ.xx = c0*c1; RJ.xy = -s0; RJ.xz = c0*s1; RJ.yx = s0*c1; RJ.yy = c0; RJ.yz = s0*s1; RJ.zx = -s1; RJ.zy = 0.0; RJ.zz = c1;
-        x.R = mm(Ro, RJ); x.p = org_p(L);
-        stm(sl+17, x.R); st3(sl+26, x.p); c.S(sl+29) = s1; c.S(sl+30) = c1;
-        const double v0 = T(qds+qo), v1 = T(qds+qo+1); wJ = v3(-s1*v0, v1, c1*v0);
-      } break;
-      default: x.R = org_R(L); x.p = org_p(L); break;
-      }
-      V3 om_n = xf_tmul(x, om);
-      if( JT<Kt>(i,L) == J_REVOL ) om_n.z += wJ.z; else om_n = om_n + wJ;      /* additions of literal zeros are not folded away */
-      if( m.need_world ){
-        V3 vl_n = xf_tmul(x, cadd_p(vl, om, x.p, x.pz));
-        if( JT<Kt>(i,L) != J_REVOL ) vl_n = vl_n + vJ;
-        pw = madd_p(pw, Rw, x.p, x.pz); Rw = xf_world(x, Rw); vl = vl_n;
-      }
-      om = om_n;
-      st3(Spec::wslot(i,L), om);
-      if( !gacc ){ gd = xf_tmul(x, gd); st3(Spec::wslot(i,L)+3, gd); }
-      const int wx = Spec::wext_slot(i,L), fs = Spec::frame_slot(i,L), bs = Spec::branch_slot(i,L);
-      if( wx >= 0 ){
-        const V6 w = contacts(m, L, Rw, pw, vl, om, ref);
-        st3(wx, w.l); st3(wx+3, w.a);
-        if( fs >= 0 ){ stm(fs, Rw); st3(fs+9, pw); st3(fs+12, vl); st3(fs+15, om); }
-      }
-      if( bs >= 0 && m.need_world ){ stm(bs, Rw); st3(bs+9, pw); st3(bs+12, vl); }
+      double sn = 0.0, co = 1.0, wz = 0.0;
+      if( JT<Kt>(i, m.link[i]) == J_REVOL ) revol_state(m, i, fresh, sn, co, wz);
+      pass1_link<Kt>(m, i, k, ref, sn, co, wz, true);
     };
     links_fwd(m, body);
   }
 
   /* motor + joint friction of a 1-DoF joint: returns tau = driving torque + friction, jm = rotor inertia
    * (rkfd_util.c:330-364, [EXT A-6, A-7]); at the reference stage commits pivot type and prev_trq */
-  RKFD_HD double joint_torque(const ModelDev &m, const LinkDev &L, int i, bool ref, double &jm, double u_in, double prev_in){
+  /* v = the joint velocity (the caller has it from joint_xform) */
+  RKFD_HD double joint_torque(const ModelDev &m, const LinkDev &L, int i, bool ref, double &jm, double u_in, double prev_in, double v){
     const int j = Spec::qofs(i,L);
-    const double v = T(rk0 + Spec::nq(m) + j);
     const double qj = L.stiffness != 0.0 ? T(rk0 + j) : 0.0;      /* warp-uniform condition: T-space reads stay collective */
     double tdrive = 0.0, tf = 0.0; jm = 0.0;
     if( L.mtype != M_NONE ){
@@ -900,7 +926,7 @@ struct Core {
       }
       switch(JT<Kt>(i,L)){
       case J_REVOL: {
-        double jm; const double tau = joint_torque(m, L, i, ref, jm, pf_u, pf_prev);
+        double jm; const double tau = joint_torque(m, L, i, ref, jm, pf_u, pf_prev, wJ.z);
         const V3 Ul = col2(B), Ua = v3(C.xz, C.yz, C.zz);
         const double Dinv = 1.0/(C.zz + jm), u = tau - pn.z;
         st3(sl, Ul); st3(sl+3, Ua); Qw(Spec::sc(i,L)+2, Dinv); Qw(Spec::sc(i,L)+3, u);
@@ -911,7 +937,7 @@ struct Core {
         pf = vfma(u, Wl, pf); pn = vfma(u, Wa, pn);
       } break;
       case J_PRISM: {
-        double jm; const double tau = joint_torque(m, L, i, ref, jm, pf_u, pf_prev);
+        double jm; const double tau = joint_torque(m, L, i, ref, jm, pf_u, pf_prev, vJ.z);
         const V3 Ul = v3(A.xz, A.yz, A.zz), Ua = v3(B.zx, B.zy, B.zz);
         const double Dinv = 1.0/(A.zz + jm), u = tau - pf.z;
         st3(sl, Ul); st3(sl+3, Ua); Qw(Spec::sc(i,L)+2, Dinv); Qw(Spec::sc(i,L)+3, u);
@@ -1006,13 +1032,14 @@ struct Core {
   /* velocity-like (vector-space) component j */
   RKFD_HD void rk_lin(const ModelDev &m, const RK &k, int stage, int slotS, int slotP, double *gin, double *gout, int j, double slope){
     const double F = ( stage >= ST_K2 && stage <= ST_K4 ) ? c.gld(gout, j) : 0.0, x0 = stage == ST_K2 ? c.gld(gin, j) : 0.0;
-    rk_lin_pf(k, stage, slotS, slotP, gout, j, slope, F, x0);
+    rk_lin_pf(k, stage, slotS, slotP, gout, j, slope, F, x0, stage == ST_K1 ? T(slotS) : 0.0);
   }
-  /* F = running combination and x0 = committed value, fetched by the caller (possibly one link ahead) */
-  RKFD_HD double rk_lin_pf(const RK &k, int stage, int slotS, int slotP, double *gout, int j, double slope, double F, double x0g){
+  /* F = running combination and x0 = committed value, fetched by the caller (possibly one link ahead); xs = the stage value
+   * (T space slotS) at stage K1, which the caller has already loaded */
+  RKFD_HD double rk_lin_pf(const RK &k, int stage, int slotS, int slotP, double *gout, int j, double slope, double F, double x0g, double xs){
     double xn = 0.0;       /* the next stage value */
     switch(stage){
-    case ST_K1: { const double x0 = T(slotS); const double F = x0 + k.b1*slope; c.gst(gout, j, F); Tw(slotP, x0 + k.c31*slope); xn = k.ns == 1 ? F : x0 + k.c21*slope; Tw(slotS, xn); } break;
+    case ST_K1: { const double x0 = xs; const double F = x0 + k.b1*slope; c.gst(gout, j, F); Tw(slotP, x0 + k.c31*slope); xn = k.ns == 1 ? F : x0 + k.c21*slope; Tw(slotS, xn); } break;
     case ST_K2: { c.gst(gout, j, F + k.b2*slope); xn = T(slotP) + k.c32*slope; Tw(slotS, xn); Tw(slotP, x0g + k.c42*slope); } break;
     case ST_K3: { c.gst(gout, j, F + k.b3*slope); xn = T(slotP) + k.c43*slope; Tw(slotS, xn); } break;
     case ST_K4: { xn = F + k.b4*slope; c.gst(gout, j, xn); Tw(slotS, xn); } break;
@@ -1023,13 +1050,13 @@ struct Core {
   /* sin/cos of a revolute joint carried from the stage angle qold to qnew = qold + d: angle addition with the
    * Taylor series of (sin d, cos d) (|d| <= 1/16: truncation below 1e-18), a full sincos otherwise.  A step
    * computes sincos once per joint (first stage) instead of five times; four chained rotations add a few ulp. */
-  RKFD_HD void rot_sincos(const ModelDev &m, int sc, double s0, double c0, double qold, double qnew){
+  RKFD_HD void rot_sincos(const ModelDev &m, int sc, double s0, double c0, double qold, double qnew, double &sn, double &co){
     const double d = qnew - qold, d2 = d*d;
     /* the coefficients 1/9!, -1/7!, 1/5!, -1/3!, 1/8!, -1/6! come from the model table (same values: operands of the multiply-adds
      * instead of two moves each) */
     const double sd = d*fma(d2, fma(d2, fma(d2, fma(d2, m.tay[0], m.tay[1]), m.tay[2]), m.tay[3]), 1.0);
     const double cd = fma(d2, fma(d2, fma(d2, fma(d2, m.tay[4], m.tay[5]), 1.0/24.0), -0.5), 1.0);
-    double sn = fma(s0, cd, c0*sd), co = fma(c0, cd, -(s0*sd));
+    sn = fma(s0, cd, c0*sd); co = fma(c0, cd, -(s0*sd));
     if( !(fabs(d) <= 0.0625) ) sincos(qnew, &sn, &co);
     Qw(sc, sn); Qw(sc+1, co);
   }
@@ -1057,170 +1084,202 @@ struct Core {
     if( stage == ST_PROBE ) return;
     if( stage >= ST_REF ){ c.gst(c.st.qdd, j, acc); if( !(fabs(acc) < 1.0e300) ) bad = 1; return; }
     const double vel = T(qds);
-    rk_lin(m, k, stage, qs, pq, c.st.q[c.cur], c.st.q[c.cur^1], j, vel);
-    rk_lin(m, k, stage, qds, pqd, c.st.qd[c.cur], c.st.qd[c.cur^1], j, acc);
+    rk_lin(m, k, stage, qs, pq, qc, qn, j, vel);
+    rk_lin(m, k, stage, qds, pqd, qdc, qdn, j, acc);
   }
 
   /* ---- pass 3: outward acceleration pass + integrator bookkeeping */
-  RKFD_HD void pass3(const ModelDev &m, int stage){
+  /* pass-3 values carried outward: linear / angular acceleration and angular velocity of the parent link; the running
+   * combination (and, at stage 2, the committed state) of the next 1-DoF joint, requested one link ahead */
+  struct Acc { V3 al, aa, om; double nxq[4]; };
+  static RKFD_HD void acc_init(Acc &a){ a.al = v3(0,0,0); a.aa = v3(0,0,0); a.om = v3(0,0,0); a.nxq[0] = a.nxq[1] = a.nxq[2] = a.nxq[3] = 0; }
+  /* pass 3 at link i.  Stages K1-K4: a revolute joint returns its (sin, cos, q') of the next stage in (sn, co, wz), the
+   * values it also stores in the T space */
+  template <class Kt>
+  RKFD_HD void pass3_link(const ModelDev &m, int i, Acc &a, int stage, double &sn, double &co, double &wz){
     const RK &k = m.rk;
-    V3 al = v3(0,0,0), aa = v3(0,0,0), om = v3(0,0,0);
-    /* running combination (and, at stage 2, the committed state) of the next 1-DoF joint are requested one link ahead */
-    double nxq[4] = {0,0,0,0};
     const bool pfF = stage >= ST_K2 && stage <= ST_K4, pfX = stage == ST_K2;
     const int NLc = Spec::nl(m), NQc = Spec::nq(m);
+    const LinkDev &L = m.link[i]; const int sl = Spec::slot(i,L), qo = Spec::qofs(i,L);
+    if( i == 0 && Spec::ndof(i,L) == 1 ){
+      if( pfF ){ a.nxq[0] = c.gld(qn, qo); a.nxq[1] = c.gld(qdn, qo); }
+      if( pfX ){ a.nxq[2] = c.gld(qc, qo); a.nxq[3] = c.gld(qdc, qo); }
+    }
+    const double pfq[4] = { a.nxq[0], a.nxq[1], a.nxq[2], a.nxq[3] };
+    if( i+1 < NLc && Spec::ndof(i+1, m.link[i+1]) == 1 ){
+      const int jn = Spec::qofs(i+1, m.link[i+1]);
+      if( pfF ){ a.nxq[0] = c.gld(qn, jn); a.nxq[1] = c.gld(qdn, jn); }
+      if( pfX ){ a.nxq[2] = c.gld(qc, jn); a.nxq[3] = c.gld(qdc, jn); }
+    }
+    if( !SER<Kt>(i,L) ){
+      if( ROOT<Kt>(i,L) ){ a.al = v3(0,0, grav_acc(m) ? GRAVITY : 0.0); a.aa = v3(0,0,0); a.om = v3(0,0,0); }
+      else { const int b = m.link[L.parent].branch_slot; a.al = ld3(b); a.aa = ld3(b+3); a.om = ld3(b+6); }
+    }
+    V3 vJ, wJ;
+    const XF x = joint_xform<Kt>(m, L, i, vJ, wJ);
+    const V3 omp = xf_tmul(x, a.om);
+    V3 zl, za;
+    if( JT<Kt>(i,L) == J_REVOL ){ zl = cross(omp, cross(omp, x.ptl)); za = v3(omp.y*wJ.z, -omp.x*wJ.z, 0.0); }
+    else { zl = cross(omp, cross(omp, x.ptl)) + 2.0*cross(omp, vJ); za = cross(omp, wJ); }
+    const V3 xl = xf_tmul(x, cadd_p(a.al, a.aa, x.p, x.pz)), xa = xf_tmul(x, a.aa);
+    switch(JT<Kt>(i,L)){
+    case J_REVOL: case J_PRISM: {
+      const V3 Ul = ld3(sl), Ua = ld3(sl+3);
+      double Dinv, uu; Q2(Spec::sc(i,L)+2, Dinv, uu);
+      const double acc = Dinv*fma(-Ua.z,xa.z,fma(-Ua.y,xa.y,fma(-Ua.x,xa.x,fma(-Ul.z,xl.z,fma(-Ul.y,xl.y,fma(-Ul.x,xl.x,uu))))));
+      if( JT<Kt>(i,L) == J_REVOL ){
+        a.al = cadd(xl, omp, cross(omp, x.ptl));
+        a.aa = v3(fma(omp.y, wJ.z, xa.x), fma(-omp.x, wJ.z, xa.y), xa.z + acc);
+      } else { a.al = xl + zl; a.aa = xa + za; a.al.z += acc; }
+      if( stage == ST_PROBE ){}
+      else if( stage >= ST_REF ){ c.gst(c.st.qdd, qo, acc); if( !(fabs(acc) < 1.0e300) ) bad = 1; }
+      else {
+        const int j = qo, qs = rk0 + j, qds = qs + NQc, pq = qs + 2*NQc, pqd = qs + 3*NQc;
+        const double vel = JT<Kt>(i,L) == J_REVOL ? wJ.z : vJ.z;     /* T(qds), loaded by joint_xform */
+        const double qold = ( JT<Kt>(i,L) == J_REVOL || stage == ST_K1 ) ? T(qs) : 0.0;
+        const double qnew = rk_lin_pf(k, stage, qs,  pq,  qn,  j, vel, pfq[0], pfq[2], qold);
+        if( JT<Kt>(i,L) == J_REVOL ) rot_sincos(m, Spec::sc(i,L), x.s, x.c, qold, qnew, sn, co);
+        wz = rk_lin_pf(k, stage, qds, pqd, qdn, j, acc, pfq[1], pfq[3], vel);
+      }
+    } break;
+    case J_SPHER: {
+      const M3 Ul = ldm(sl), Ua = ldm(sl+9); const S3 Di = lds(sl+18); const V3 u = ld3(sl+24);
+      const V3 rhs = u - (tmul(Ul, xl) + tmul(Ua, xa));
+      const V3 acc = mul(Di, rhs);
+      const M3 E = tmm(x.R, org_R(L));
+      a.al = xl + zl; a.aa = xa + za + mul(E, acc);
+      if( stage == ST_PROBE ){}
+      else if( stage >= ST_REF ){ c.gst(c.st.qdd,L.qofs,acc.x); c.gst(c.st.qdd,L.qofs+1,acc.y); c.gst(c.st.qdd,L.qofs+2,acc.z);
+        if( !(fabs(acc.x)+fabs(acc.y)+fabs(acc.z) < 1.0e300) ) bad = 1; }
+      else {
+        const int qs = rk0 + L.qofs, qds = qs + m.nq, pq = qs + 2*m.nq, pqd = qs + 3*m.nq;
+        const V3 w = t3(qds);
+        rk_rot(m, k, stage, qs, pq, qc, qn, L.qofs, w);
+        rk_lin(m, k, stage, qds,   pqd,   qdc, qdn, L.qofs,   acc.x);
+        rk_lin(m, k, stage, qds+1, pqd+1, qdc, qdn, L.qofs+1, acc.y);
+        rk_lin(m, k, stage, qds+2, pqd+2, qdc, qdn, L.qofs+2, acc.z);
+      }
+    } break;
+    case J_CYLIN: case J_HOOKE: {
+      if( JT<Kt>(i,L) == J_HOOKE ){ const double qq = T(rk0 + NQc + qo)*T(rk0 + NQc + qo + 1); za.x -= c.S(sl+30)*qq; za.z -= c.S(sl+29)*qq; }
+      V3 l0, a0, l1, a1; axes2(JT<Kt>(i,L), sl, l0, a0, l1, a1);
+      const double r0 = c.S(sl+15) - (dot(ld3(sl),xl) + dot(ld3(sl+3),xa)), r1 = c.S(sl+16) - (dot(ld3(sl+6),xl) + dot(ld3(sl+9),xa));
+      const double acc0 = c.S(sl+12)*r0 + c.S(sl+13)*r1, acc1 = c.S(sl+13)*r0 + c.S(sl+14)*r1;
+      a.al = xl + zl + acc0*l0 + acc1*l1; a.aa = xa + za + acc0*a0 + acc1*a1;
+      if( stage == ST_PROBE ){}
+      else if( stage >= ST_REF ){ c.gst(c.st.qdd, qo, acc0); c.gst(c.st.qdd, qo+1, acc1); if( !(fabs(acc0)+fabs(acc1) < 1.0e300) ) bad = 1; }
+      else {
+        const int qs = rk0 + qo, qds = qs + m.nq, pq = qs + 2*m.nq, pqd = qs + 3*m.nq;
+        const double v0 = T(qds), v1 = T(qds+1);
+        rk_lin(m, k, stage, qs,   pq,   qc, qn, qo,   v0);
+        rk_lin(m, k, stage, qs+1, pq+1, qc, qn, qo+1, v1);
+        rk_lin(m, k, stage, qds,   pqd,   qdc, qdn, qo,   acc0);
+        rk_lin(m, k, stage, qds+1, pqd+1, qdc, qdn, qo+1, acc1);
+      }
+    } break;
+    case J_FLOAT: {
+      const V3 a0l = ld3(sl), a0a = ld3(sl+3);
+      const M3 RJ = mm(transpose(org_R(L)), x.R);     /* S^-1 = blockdiag(RJ, RJ) */
+      const V3 accl = mul(RJ, a0l - xl - zl), acca = mul(RJ, a0a - xa - za);
+      a.al = a0l; a.aa = a0a;
+      if( stage == ST_PROBE ){}
+      else if( stage >= ST_REF ){
+        c.gst(c.st.qdd,L.qofs,accl.x); c.gst(c.st.qdd,L.qofs+1,accl.y); c.gst(c.st.qdd,L.qofs+2,accl.z);
+        c.gst(c.st.qdd,L.qofs+3,acca.x); c.gst(c.st.qdd,L.qofs+4,acca.y); c.gst(c.st.qdd,L.qofs+5,acca.z);
+        if( !(fabs(accl.x)+fabs(accl.y)+fabs(accl.z)+fabs(acca.x)+fabs(acca.y)+fabs(acca.z) < 1.0e300) ) bad = 1;
+      } else {
+        const int qs = rk0 + L.qofs, qds = qs + m.nq, pq = qs + 2*m.nq, pqd = qs + 3*m.nq;
+        const V3 v = t3(qds), w = t3(qds+3);
+        rk_lin(m, k, stage, qs,   pq,   qc, qn, L.qofs,   v.x);
+        rk_lin(m, k, stage, qs+1, pq+1, qc, qn, L.qofs+1, v.y);
+        rk_lin(m, k, stage, qs+2, pq+2, qc, qn, L.qofs+2, v.z);
+        rk_rot(m, k, stage, qs+3, pq+3, qc, qn, L.qofs+3, w);
+        rk_lin(m, k, stage, qds,   pqd,   qdc, qdn, L.qofs,   accl.x);
+        rk_lin(m, k, stage, qds+1, pqd+1, qdc, qdn, L.qofs+1, accl.y);
+        rk_lin(m, k, stage, qds+2, pqd+2, qdc, qdn, L.qofs+2, accl.z);
+        rk_lin(m, k, stage, qds+3, pqd+3, qdc, qdn, L.qofs+3, acca.x);
+        rk_lin(m, k, stage, qds+4, pqd+4, qdc, qdn, L.qofs+4, acca.y);
+        rk_lin(m, k, stage, qds+5, pqd+5, qdc, qdn, L.qofs+5, acca.z);
+      }
+    } break;
+    case J_BRFLOAT: {
+      /* broken: the float joint; rigid: the fixed joint whose six dofs are held (zero slopes), and in the committing
+       * evaluation the wrench it transmits, IA (X a_parent) + p' at the link origin ([EXT A-17]; rkChainUpdateABIWrench,
+       * rkfd_sim.c:511-514), is compared with its thresholds.  One code path for both: the integrator bookkeeping touches
+       * the T space, which only warp-uniform code may do. */
+      const bool brk = c.S(sl+45) != 0.0;
+      V3 accl = v3(0,0,0), acca = v3(0,0,0);
+      if( brk ){ const V3 a0l = ld3(sl), a0a = ld3(sl+3); const M3 RJ = mm(transpose(org_R(L)), x.R);
+        accl = mul(RJ, a0l - xl - zl); acca = mul(RJ, a0a - xa - za); a.al = a0l; a.aa = a0a; }
+      else { a.al = xl + zl; a.aa = xa + za; }
+      if( stage == ST_PROBE ){}
+      else if( stage >= ST_REF ){
+        c.gst(c.st.qdd,L.qofs,accl.x); c.gst(c.st.qdd,L.qofs+1,accl.y); c.gst(c.st.qdd,L.qofs+2,accl.z);
+        c.gst(c.st.qdd,L.qofs+3,acca.x); c.gst(c.st.qdd,L.qofs+4,acca.y); c.gst(c.st.qdd,L.qofs+5,acca.z);
+        if( !(fabs(accl.x)+fabs(accl.y)+fabs(accl.z)+fabs(acca.x)+fabs(acca.y)+fabs(acca.z) < 1.0e300) ) bad = 1;
+        if( !brk && ( stage == ST_REF || stage == ST_EVAL_REF ) ){
+          S3 A, C; A.xx=c.S(sl+18); A.xy=c.S(sl+19); A.xz=c.S(sl+20); A.yy=c.S(sl+21); A.yz=c.S(sl+22); A.zz=c.S(sl+23);
+          const M3 B = ldm(sl+24);
+          C.xx=c.S(sl+33); C.xy=c.S(sl+34); C.xz=c.S(sl+35); C.yy=c.S(sl+36); C.yz=c.S(sl+37); C.zz=c.S(sl+38);
+          const V3 f = ld3(sl+39) + mul(A, xl) + mul(B, xa), n = ld3(sl+42) + tmul(B, xl) + mul(C, xa);
+          if( norm(f) > L.brk_f || norm(n) > L.brk_t ) piv |= 1u << L.qofs;
+        }
+      } else {
+        const int qs = rk0 + L.qofs, qds = qs + m.nq, pq = qs + 2*m.nq, pqd = qs + 3*m.nq;
+        V3 v = t3(qds), w = t3(qds+3);
+        if( !brk ){ v = v3(0,0,0); w = v; }
+        rk_lin(m, k, stage, qs,   pq,   qc, qn, L.qofs,   v.x);
+        rk_lin(m, k, stage, qs+1, pq+1, qc, qn, L.qofs+1, v.y);
+        rk_lin(m, k, stage, qs+2, pq+2, qc, qn, L.qofs+2, v.z);
+        rk_rot(m, k, stage, qs+3, pq+3, qc, qn, L.qofs+3, w);
+        rk_lin(m, k, stage, qds,   pqd,   qdc, qdn, L.qofs,   accl.x);
+        rk_lin(m, k, stage, qds+1, pqd+1, qdc, qdn, L.qofs+1, accl.y);
+        rk_lin(m, k, stage, qds+2, pqd+2, qdc, qdn, L.qofs+2, accl.z);
+        rk_lin(m, k, stage, qds+3, pqd+3, qdc, qdn, L.qofs+3, acca.x);
+        rk_lin(m, k, stage, qds+4, pqd+4, qdc, qdn, L.qofs+4, acca.y);
+        rk_lin(m, k, stage, qds+5, pqd+5, qdc, qdn, L.qofs+5, acca.z);
+      }
+    } break;
+    default: a.al = xl + zl; a.aa = xa + za; break;
+    }
+    if( JT<Kt>(i,L) == J_REVOL ) a.om = v3(omp.x, omp.y, omp.z + wJ.z); else a.om = omp + wJ;
+    if( Spec::frame_slot(i,L) >= 0 ){ st3(Spec::frame_slot(i,L)+18, a.al); st3(Spec::frame_slot(i,L)+21, a.aa); }
+    if( Spec::branch_slot(i,L) >= 0 ){ st3(L.branch_slot, a.al); st3(L.branch_slot+3, a.aa); st3(L.branch_slot+6, a.om); }
+  }
+  RKFD_HD void pass3(const ModelDev &m, int stage){
+    Acc a; acc_init(a);
     auto body = [&](const int i, auto Ktag){
       using Kt = decltype(Ktag);
-      const LinkDev &L = m.link[i]; const int sl = Spec::slot(i,L), qo = Spec::qofs(i,L);
       if( !Ctx::RIGID ) c.phase_sync(3);
-      if( i == 0 && Spec::ndof(i,L) == 1 ){
-        if( pfF ){ nxq[0] = c.gld(c.st.q[c.cur^1], qo); nxq[1] = c.gld(c.st.qd[c.cur^1], qo); }
-        if( pfX ){ nxq[2] = c.gld(c.st.q[c.cur], qo); nxq[3] = c.gld(c.st.qd[c.cur], qo); }
-      }
-      const double pfq[4] = { nxq[0], nxq[1], nxq[2], nxq[3] };
-      if( i+1 < NLc && Spec::ndof(i+1, m.link[i+1]) == 1 ){
-        const int jn = Spec::qofs(i+1, m.link[i+1]);
-        if( pfF ){ nxq[0] = c.gld(c.st.q[c.cur^1], jn); nxq[1] = c.gld(c.st.qd[c.cur^1], jn); }
-        if( pfX ){ nxq[2] = c.gld(c.st.q[c.cur], jn); nxq[3] = c.gld(c.st.qd[c.cur], jn); }
-      }
-      if( !SER<Kt>(i,L) ){
-        if( ROOT<Kt>(i,L) ){ al = v3(0,0, grav_acc(m) ? GRAVITY : 0.0); aa = v3(0,0,0); om = v3(0,0,0); }
-        else { const int b = m.link[L.parent].branch_slot; al = ld3(b); aa = ld3(b+3); om = ld3(b+6); }
-      }
-      V3 vJ, wJ;
-      const XF x = joint_xform<Kt>(m, L, i, vJ, wJ);
-      const V3 omp = xf_tmul(x, om);
-      V3 zl, za;
-      if( JT<Kt>(i,L) == J_REVOL ){ zl = cross(omp, cross(omp, x.ptl)); za = v3(omp.y*wJ.z, -omp.x*wJ.z, 0.0); }
-      else { zl = cross(omp, cross(omp, x.ptl)) + 2.0*cross(omp, vJ); za = cross(omp, wJ); }
-      const V3 xl = xf_tmul(x, cadd_p(al, aa, x.p, x.pz)), xa = xf_tmul(x, aa);
-      switch(JT<Kt>(i,L)){
-      case J_REVOL: case J_PRISM: {
-        const V3 Ul = ld3(sl), Ua = ld3(sl+3);
-        double Dinv, uu; Q2(Spec::sc(i,L)+2, Dinv, uu);
-        const double acc = Dinv*fma(-Ua.z,xa.z,fma(-Ua.y,xa.y,fma(-Ua.x,xa.x,fma(-Ul.z,xl.z,fma(-Ul.y,xl.y,fma(-Ul.x,xl.x,uu))))));
-        if( JT<Kt>(i,L) == J_REVOL ){
-          al = cadd(xl, omp, cross(omp, x.ptl));
-          aa = v3(fma(omp.y, wJ.z, xa.x), fma(-omp.x, wJ.z, xa.y), xa.z + acc);
-        } else { al = xl + zl; aa = xa + za; al.z += acc; }
-        if( stage == ST_PROBE ){}
-        else if( stage >= ST_REF ){ c.gst(c.st.qdd, qo, acc); if( !(fabs(acc) < 1.0e300) ) bad = 1; }
-        else {
-          const int j = qo, qs = rk0 + j, qds = qs + NQc, pq = qs + 2*NQc, pqd = qs + 3*NQc;
-          const double vel = T(qds);
-          if( JT<Kt>(i,L) == J_REVOL ){
-            const double qold = T(qs);
-            const double qnew = rk_lin_pf(k, stage, qs,  pq,  c.st.q[c.cur^1],  j, vel, pfq[0], pfq[2]);
-            rot_sincos(m, Spec::sc(i,L), x.s, x.c, qold, qnew);
-          } else rk_lin_pf(k, stage, qs,  pq,  c.st.q[c.cur^1],  j, vel, pfq[0], pfq[2]);
-          rk_lin_pf(k, stage, qds, pqd, c.st.qd[c.cur^1], j, acc, pfq[1], pfq[3]);
-        }
-      } break;
-      case J_SPHER: {
-        const M3 Ul = ldm(sl), Ua = ldm(sl+9); const S3 Di = lds(sl+18); const V3 u = ld3(sl+24);
-        const V3 rhs = u - (tmul(Ul, xl) + tmul(Ua, xa));
-        const V3 acc = mul(Di, rhs);
-        const M3 E = tmm(x.R, org_R(L));
-        al = xl + zl; aa = xa + za + mul(E, acc);
-        if( stage == ST_PROBE ){}
-        else if( stage >= ST_REF ){ c.gst(c.st.qdd,L.qofs,acc.x); c.gst(c.st.qdd,L.qofs+1,acc.y); c.gst(c.st.qdd,L.qofs+2,acc.z);
-          if( !(fabs(acc.x)+fabs(acc.y)+fabs(acc.z) < 1.0e300) ) bad = 1; }
-        else {
-          const int qs = rk0 + L.qofs, qds = qs + m.nq, pq = qs + 2*m.nq, pqd = qs + 3*m.nq;
-          const V3 w = t3(qds);
-          rk_rot(m, k, stage, qs, pq, c.st.q[c.cur], c.st.q[c.cur^1], L.qofs, w);
-          rk_lin(m, k, stage, qds,   pqd,   c.st.qd[c.cur], c.st.qd[c.cur^1], L.qofs,   acc.x);
-          rk_lin(m, k, stage, qds+1, pqd+1, c.st.qd[c.cur], c.st.qd[c.cur^1], L.qofs+1, acc.y);
-          rk_lin(m, k, stage, qds+2, pqd+2, c.st.qd[c.cur], c.st.qd[c.cur^1], L.qofs+2, acc.z);
-        }
-      } break;
-      case J_CYLIN: case J_HOOKE: {
-        if( JT<Kt>(i,L) == J_HOOKE ){ const double qq = T(rk0 + NQc + qo)*T(rk0 + NQc + qo + 1); za.x -= c.S(sl+30)*qq; za.z -= c.S(sl+29)*qq; }
-        V3 l0, a0, l1, a1; axes2(JT<Kt>(i,L), sl, l0, a0, l1, a1);
-        const double r0 = c.S(sl+15) - (dot(ld3(sl),xl) + dot(ld3(sl+3),xa)), r1 = c.S(sl+16) - (dot(ld3(sl+6),xl) + dot(ld3(sl+9),xa));
-        const double acc0 = c.S(sl+12)*r0 + c.S(sl+13)*r1, acc1 = c.S(sl+13)*r0 + c.S(sl+14)*r1;
-        al = xl + zl + acc0*l0 + acc1*l1; aa = xa + za + acc0*a0 + acc1*a1;
-        if( stage == ST_PROBE ){}
-        else if( stage >= ST_REF ){ c.gst(c.st.qdd, qo, acc0); c.gst(c.st.qdd, qo+1, acc1); if( !(fabs(acc0)+fabs(acc1) < 1.0e300) ) bad = 1; }
-        else {
-          const int qs = rk0 + qo, qds = qs + m.nq, pq = qs + 2*m.nq, pqd = qs + 3*m.nq;
-          const double v0 = T(qds), v1 = T(qds+1);
-          rk_lin(m, k, stage, qs,   pq,   c.st.q[c.cur], c.st.q[c.cur^1], qo,   v0);
-          rk_lin(m, k, stage, qs+1, pq+1, c.st.q[c.cur], c.st.q[c.cur^1], qo+1, v1);
-          rk_lin(m, k, stage, qds,   pqd,   c.st.qd[c.cur], c.st.qd[c.cur^1], qo,   acc0);
-          rk_lin(m, k, stage, qds+1, pqd+1, c.st.qd[c.cur], c.st.qd[c.cur^1], qo+1, acc1);
-        }
-      } break;
-      case J_FLOAT: {
-        const V3 a0l = ld3(sl), a0a = ld3(sl+3);
-        const M3 RJ = mm(transpose(org_R(L)), x.R);     /* S^-1 = blockdiag(RJ, RJ) */
-        const V3 accl = mul(RJ, a0l - xl - zl), acca = mul(RJ, a0a - xa - za);
-        al = a0l; aa = a0a;
-        if( stage == ST_PROBE ){}
-        else if( stage >= ST_REF ){
-          c.gst(c.st.qdd,L.qofs,accl.x); c.gst(c.st.qdd,L.qofs+1,accl.y); c.gst(c.st.qdd,L.qofs+2,accl.z);
-          c.gst(c.st.qdd,L.qofs+3,acca.x); c.gst(c.st.qdd,L.qofs+4,acca.y); c.gst(c.st.qdd,L.qofs+5,acca.z);
-          if( !(fabs(accl.x)+fabs(accl.y)+fabs(accl.z)+fabs(acca.x)+fabs(acca.y)+fabs(acca.z) < 1.0e300) ) bad = 1;
-        } else {
-          const int qs = rk0 + L.qofs, qds = qs + m.nq, pq = qs + 2*m.nq, pqd = qs + 3*m.nq;
-          const V3 v = t3(qds), w = t3(qds+3);
-          rk_lin(m, k, stage, qs,   pq,   c.st.q[c.cur], c.st.q[c.cur^1], L.qofs,   v.x);
-          rk_lin(m, k, stage, qs+1, pq+1, c.st.q[c.cur], c.st.q[c.cur^1], L.qofs+1, v.y);
-          rk_lin(m, k, stage, qs+2, pq+2, c.st.q[c.cur], c.st.q[c.cur^1], L.qofs+2, v.z);
-          rk_rot(m, k, stage, qs+3, pq+3, c.st.q[c.cur], c.st.q[c.cur^1], L.qofs+3, w);
-          rk_lin(m, k, stage, qds,   pqd,   c.st.qd[c.cur], c.st.qd[c.cur^1], L.qofs,   accl.x);
-          rk_lin(m, k, stage, qds+1, pqd+1, c.st.qd[c.cur], c.st.qd[c.cur^1], L.qofs+1, accl.y);
-          rk_lin(m, k, stage, qds+2, pqd+2, c.st.qd[c.cur], c.st.qd[c.cur^1], L.qofs+2, accl.z);
-          rk_lin(m, k, stage, qds+3, pqd+3, c.st.qd[c.cur], c.st.qd[c.cur^1], L.qofs+3, acca.x);
-          rk_lin(m, k, stage, qds+4, pqd+4, c.st.qd[c.cur], c.st.qd[c.cur^1], L.qofs+4, acca.y);
-          rk_lin(m, k, stage, qds+5, pqd+5, c.st.qd[c.cur], c.st.qd[c.cur^1], L.qofs+5, acca.z);
-        }
-      } break;
-      case J_BRFLOAT: {
-        /* broken: the float joint; rigid: the fixed joint whose six dofs are held (zero slopes), and in the committing
-         * evaluation the wrench it transmits, IA (X a_parent) + p' at the link origin ([EXT A-17]; rkChainUpdateABIWrench,
-         * rkfd_sim.c:511-514), is compared with its thresholds.  One code path for both: the integrator bookkeeping touches
-         * the T space, which only warp-uniform code may do. */
-        const bool brk = c.S(sl+45) != 0.0;
-        V3 accl = v3(0,0,0), acca = v3(0,0,0);
-        if( brk ){ const V3 a0l = ld3(sl), a0a = ld3(sl+3); const M3 RJ = mm(transpose(org_R(L)), x.R);
-          accl = mul(RJ, a0l - xl - zl); acca = mul(RJ, a0a - xa - za); al = a0l; aa = a0a; }
-        else { al = xl + zl; aa = xa + za; }
-        if( stage == ST_PROBE ){}
-        else if( stage >= ST_REF ){
-          c.gst(c.st.qdd,L.qofs,accl.x); c.gst(c.st.qdd,L.qofs+1,accl.y); c.gst(c.st.qdd,L.qofs+2,accl.z);
-          c.gst(c.st.qdd,L.qofs+3,acca.x); c.gst(c.st.qdd,L.qofs+4,acca.y); c.gst(c.st.qdd,L.qofs+5,acca.z);
-          if( !(fabs(accl.x)+fabs(accl.y)+fabs(accl.z)+fabs(acca.x)+fabs(acca.y)+fabs(acca.z) < 1.0e300) ) bad = 1;
-          if( !brk && ( stage == ST_REF || stage == ST_EVAL_REF ) ){
-            S3 A, C; A.xx=c.S(sl+18); A.xy=c.S(sl+19); A.xz=c.S(sl+20); A.yy=c.S(sl+21); A.yz=c.S(sl+22); A.zz=c.S(sl+23);
-            const M3 B = ldm(sl+24);
-            C.xx=c.S(sl+33); C.xy=c.S(sl+34); C.xz=c.S(sl+35); C.yy=c.S(sl+36); C.yz=c.S(sl+37); C.zz=c.S(sl+38);
-            const V3 f = ld3(sl+39) + mul(A, xl) + mul(B, xa), n = ld3(sl+42) + tmul(B, xl) + mul(C, xa);
-            if( norm(f) > L.brk_f || norm(n) > L.brk_t ) piv |= 1u << L.qofs;
-          }
-        } else {
-          const int qs = rk0 + L.qofs, qds = qs + m.nq, pq = qs + 2*m.nq, pqd = qs + 3*m.nq;
-          V3 v = t3(qds), w = t3(qds+3);
-          if( !brk ){ v = v3(0,0,0); w = v; }
-          rk_lin(m, k, stage, qs,   pq,   c.st.q[c.cur], c.st.q[c.cur^1], L.qofs,   v.x);
-          rk_lin(m, k, stage, qs+1, pq+1, c.st.q[c.cur], c.st.q[c.cur^1], L.qofs+1, v.y);
-          rk_lin(m, k, stage, qs+2, pq+2, c.st.q[c.cur], c.st.q[c.cur^1], L.qofs+2, v.z);
-          rk_rot(m, k, stage, qs+3, pq+3, c.st.q[c.cur], c.st.q[c.cur^1], L.qofs+3, w);
-          rk_lin(m, k, stage, qds,   pqd,   c.st.qd[c.cur], c.st.qd[c.cur^1], L.qofs,   accl.x);
-          rk_lin(m, k, stage, qds+1, pqd+1, c.st.qd[c.cur], c.st.qd[c.cur^1], L.qofs+1, accl.y);
-          rk_lin(m, k, stage, qds+2, pqd+2, c.st.qd[c.cur], c.st.qd[c.cur^1], L.qofs+2, accl.z);
-          rk_lin(m, k, stage, qds+3, pqd+3, c.st.qd[c.cur], c.st.qd[c.cur^1], L.qofs+3, acca.x);
-          rk_lin(m, k, stage, qds+4, pqd+4, c.st.qd[c.cur], c.st.qd[c.cur^1], L.qofs+4, acca.y);
-          rk_lin(m, k, stage, qds+5, pqd+5, c.st.qd[c.cur], c.st.qd[c.cur^1], L.qofs+5, acca.z);
-        }
-      } break;
-      default: al = xl + zl; aa = xa + za; break;
-      }
-      if( JT<Kt>(i,L) == J_REVOL ) om = v3(omp.x, omp.y, omp.z + wJ.z); else om = omp + wJ;
-      if( Spec::frame_slot(i,L) >= 0 ){ st3(Spec::frame_slot(i,L)+18, al); st3(Spec::frame_slot(i,L)+21, aa); }
-      if( Spec::branch_slot(i,L) >= 0 ){ st3(L.branch_slot, al); st3(L.branch_slot+3, aa); st3(L.branch_slot+6, om); }
+      double sn, co, wz;
+      pass3_link<Kt>(m, i, a, stage, sn, co, wz);
     };
     links_fwd(m, body);
+  }
+
+  /* ---- the outward pass of the FUSE specialisations: pass 3 of stage s3 and pass 1 of stage s1 in ONE walk over the links
+   * (-1: that half does not run).  A Runge-Kutta-Gill step is then
+   *   P1(K1) P2(K1) [P3(K1) P1(K2)] P2(K2) [P3(K2) P1(K3)] P2(K3) [P3(K3) P1(K4)] P2(K4) [P3(K4) P1(REF)] P2(REF) P3(REF):
+   * 11 passes and block barriers instead of 15, and pass 1 takes the new (sin, cos, q') of each joint from the registers
+   * pass 3 has just computed them in.  At link i pass 3 reads U before pass 1 writes the new angular velocity into the same
+   * slots; link i reads nothing of links > i.  Both halves sit in one function with one call site, selected by the
+   * warp-uniform stages, so that the link body and the contact code exist once in the kernel (instruction cache); the
+   * contacts of the tip run after the loop, when pass 3's carried values are dead. */
+  RKFD_HD void outward(const ModelDev &m, int s3, int s1){
+    const bool ref = s1 == ST_REF || s1 == ST_EVAL_REF;
+    Acc a; acc_init(a);
+    Kin kn; kin_init(kn);
+    auto body = [&](const int i, auto Ktag){
+      using Kt = decltype(Ktag);
+      if( !Ctx::RIGID ) c.phase_sync(3);
+      double sn = 0.0, co = 1.0, wz = 0.0;
+      if( s3 >= 0 ) pass3_link<Kt>(m, i, a, s3, sn, co, wz);
+      else if( JT<Kt>(i, m.link[i]) == J_REVOL ) revol_state(m, i, true, sn, co, wz);   /* first pass 1 of a step or evaluation */
+      if( s1 >= 0 ) pass1_link<Kt>(m, i, kn, ref, sn, co, wz, false);
+    };
+    links_fwd(m, body);
+    const int t = Spec::NL - 1; const LinkDev &L = m.link[t]; const int wx = Spec::wext_slot(t, L);
+    if( s1 >= 0 && wx >= 0 ){ const V6 w = contacts(m, L, kn.Rw, kn.pw, kn.vl, kn.om, ref); st3(wx, w.l); st3(wx+3, w.a); }
   }
 
 
@@ -2227,11 +2286,11 @@ struct Core {
   RKFD_HD void load_flags(){ piv = c.st.piv_type[c.e]; cw = 0; cfl = c.st.cflags[c.e]; }
   RKFD_HD void store_flags(){ c.st.piv_type[c.e] = piv; c.st.cflags[(size_t)(Spec::NL != 0 ? 0 : cw)*c.st.ld + c.e] = cfl; if( bad ) c.st.status[c.e] |= bad;
     if( Ctx::RIGID ){ if( c.st.work ) c.st.work[c.e] = (unsigned char)wk; } }
-  /* committed state (buffer `cur`) -> stage state */
+  /* committed state -> stage state */
   RKFD_HD void load_stage_state(const ModelDev &m){
     const int NQc = Spec::nq(m);
 #pragma unroll (Spec::UNROLL)
-    for(int j=0;j<NQc;j++){ Tw(rk0+j, c.gld(c.st.q[c.cur], j)); Tw(rk0+NQc+j, c.gld(c.st.qd[c.cur], j)); }
+    for(int j=0;j<NQc;j++){ Tw(rk0+j, c.gld(qc, j)); Tw(rk0+NQc+j, c.gld(qdc, j)); }
   }
   RKFD_HD void evaluate(const ModelDev &m, int stage){
     const bool ref = (stage == ST_REF) || (stage == ST_EVAL_REF);
@@ -2289,12 +2348,28 @@ struct Core {
     for(int s=0;s<nsteps;s++){
       load_stage_state(m);
       const int ns = m.rk.ns;
+      if constexpr ( Spec::FUSE != 0 ){
+        /* outward passes [P3(s3) P1(s1)] (Core::outward) and the inward pass of s1 in turn; one loop, one call site each */
 #pragma unroll 1
-      for(int stage=first;;){
-        if( stage == ST_REF ) c.cur ^= 1;   /* the output buffer now holds the committed state */
-        evaluate(m, stage);
-        if( stage == last ) break;
-        stage = rk_next_stage(stage, ns);
+        for(int s3 = -1, s1 = first;;){
+          c.phase_sync(1);          /* as in evaluate */
+          c.tfence();
+          outward(m, s3, s1);
+          if( s1 < 0 ) break;
+          if( s1 == ST_REF ) commit_swap();   /* pass 3 of the last stage has formed the new state in the output buffer */
+          c.phase_sync(2);
+          c.tfence();
+          pass2(m, s1 == ST_REF || s1 == ST_EVAL_REF);
+          s3 = s1; s1 = s1 == last ? -1 : rk_next_stage(s1, ns);
+        }
+      } else {
+#pragma unroll 1
+        for(int stage=first;;){
+          if( stage == ST_REF ) commit_swap();   /* the output buffer now holds the committed state */
+          evaluate(m, stage);
+          if( stage == last ) break;
+          stage = rk_next_stage(stage, ns);
+        }
       }
     }
     store_flags();
