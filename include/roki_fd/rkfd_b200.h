@@ -349,6 +349,25 @@ __ROKI_FD_EXPORT int rkFDBatchGetStateAsync(rkFD *fd, double *q, double *qd, dou
 __ROKI_FD_EXPORT int rkFDBatchJoin(rkFD *fd);
 __ROKI_FD_EXPORT void *rkFDBatchDevicePtr(rkFD *fd, int shard, int which, int *ld, int *B);  /* 0 q, 1 qd, 2 qdd, 3 u; SoA [k][ld] */
 __ROKI_FD_EXPORT long long rkFDBatchLaunchCount(rkFD *fd);
+/* Environment reset: restarts some environments of a running batch while the others go on.  After the call, environment
+ * envs[i] is bit for bit what environment i of a new simulator of the same world would be after an rkFDUpdateInit from
+ * (q[i], qd[i], u[i]): state, q'' of the committing evaluation at t=0, contact flags, anchors and forces, friction pivots,
+ * broken breakable-float joints (broken again only if the t=0 evaluation breaks them) and status word - right after the call
+ * and in every later step.  Environments not listed are unaffected.  fd->t does not change (nothing on the step path reads
+ * the time).  Both calls need rkFDUpdateInit; n = 0 does nothing.  Each call runs one step-kernel launch per shard touched and
+ * up to 65,536 environments (counted in rkFDBatchLaunchCount), with a few small kernels around it
+ * (rkFDBatchResetKernelCount).
+ * rkFDBatchResetEnvs: host arrays, env-major: q[n][size] (required), qd[n][size] (NULL: zero), u[n][links] (NULL: keep the
+ * current input); global environment indices.  Everything is checked before any device work (indices in [0, B), no
+ * duplicates, q given): a refused call changes nothing.  Synchronous, like rkFDBatchSetState.
+ * rkFDBatchResetEnvsDevice: the same arrays on the device of shard `shard` (envs[n], q[n][size], ...), indices local to
+ * that shard (slots do not matter: the engine maps them through its re-sort order).  Stream-ordered on the engine's stream
+ * without a host synchronisation, except for the first call and a call with a longer list than any before (it allocates the
+ * reset's buffers).  Indices outside [0, B) are skipped; a duplicate index is the caller's error (the environment ends up with
+ * one of its states). */
+__ROKI_FD_EXPORT int rkFDBatchResetEnvs(rkFD *fd, int n, const int *envs, const double *q, const double *qd, const double *u);
+__ROKI_FD_EXPORT int rkFDBatchResetEnvsDevice(rkFD *fd, int shard, int n, const int *envs, const double *q, const double *qd, const double *u);
+__ROKI_FD_EXPORT long long rkFDBatchResetKernelCount(rkFD *fd);       /* gather, zero fill and scatter launches of the resets so far */
 /* the flattened model of the last rkFDUpdateInit as text (host side; also after an rkFDUpdateInit that found no device):
  * returns the length needed */
 __ROKI_FD_EXPORT int rkFDB200DescribeModel(rkFD *fd, char *buf, int cap);

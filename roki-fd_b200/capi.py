@@ -82,6 +82,8 @@ def lib():
         "rkFDBatchSetResortInterval": (ci, [vp, ci]), "rkFDBatchSlotMap": (ci, [vp, ci, _ip]), "rkFDBatchResortCount": (C.c_longlong, [vp]), "rkFDBatchResortKernelCount": (C.c_longlong, [vp]),
         "rkFDBatchGetStatus": (ci, [vp, vp]), "rkFDBatchStats": (ci, [vp, C.POINTER(cd)]), "rkFDBatchEval": (ci, [vp, ci]), "rkFDBatchSync": (ci, [vp]),
         "rkFDBatchDevicePtr": (vp, [vp, ci, ci, _ip, _ip]), "rkFDBatchLaunchCount": (C.c_longlong, [vp]),
+        "rkFDBatchResetEnvs": (ci, [vp, ci, vp, vp, vp, vp]), "rkFDBatchResetEnvsDevice": (ci, [vp, ci, ci, vp, vp, vp, vp]),
+        "rkFDBatchResetKernelCount": (C.c_longlong, [vp]),
         "rkFDB200DescribeModel": (ci, [vp, C.c_char_p, ci]), "rkFDBatchLastError": (C.c_char_p, []), "rkFDBatchDeviceCount": (ci, []), "rkFDB200MeasureFp64": (ci, [_dp]),
     }
     for name, (res, args) in sig.items():
@@ -431,6 +433,28 @@ class RkFD:
     @property
     def launch_count(self):
         return lib().rkFDBatchLaunchCount(self.h)
+
+    def batch_reset_envs(self, envs, q, qd=None, u=None):
+        """rkFDBatchResetEnvs: environments envs[i] restart from (q[i], qd[i], u[i]) as after a new update_init; qd None: zero,
+        u None: the current motor input.  The other environments go on unchanged."""
+        e = np.ascontiguousarray(envs, np.int32).reshape(-1)
+        n = e.shape[0]
+        q = None if q is None else np.ascontiguousarray(q, np.float64)     # None: refused by the library (q is required)
+        qd = None if qd is None else np.ascontiguousarray(qd, np.float64)
+        u = None if u is None else np.ascontiguousarray(u, np.float64)
+        for a, w in ((q, self.size), (qd, self.size), (u, self.link_num)):
+            if a is not None and a.size != n * w:
+                raise ValueError("batch_reset_envs: expected %d x %d values, got shape %s" % (n, w, a.shape))
+        self._ck(lib().rkFDBatchResetEnvs(self.h, n, _ptr(e), _ptr(q), _ptr(qd), _ptr(u)))
+
+    def batch_reset_envs_device(self, shard, n, envs_ptr, q_ptr, qd_ptr=None, u_ptr=None):
+        """rkFDBatchResetEnvsDevice: raw device addresses (e.g. torch CUDA tensor .data_ptr()) of int32 envs[n] (indices local to
+        the shard), q[n][size], qd[n][size], u[n][links]; stream-ordered on the engine's stream."""
+        self._ck(lib().rkFDBatchResetEnvsDevice(self.h, shard, n, _ptr(envs_ptr), _ptr(q_ptr), _ptr(qd_ptr), _ptr(u_ptr)))
+
+    @property
+    def reset_kernel_count(self):
+        return lib().rkFDBatchResetKernelCount(self.h)
 
 
 def create_world(world: World, B=None, devices=None):

@@ -548,6 +548,35 @@ extern "C" int rkFDBatchJoin(rkFD *fd){ BATCH_GUARD(fd); NEED_ENGINE(); TRY(fi->
 extern "C" int rkFDBatchSync(rkFD *fd){ BATCH_GUARD(fd); NEED_ENGINE(); TRY(fi->engine->sync()); }
 extern "C" void *rkFDBatchDevicePtr(rkFD *fd, int shard, int which, int *ld, int *B){ FDImpl *fi = FI(fd); if( !fi || !fi->engine ) return NULL; return fi->engine->device_ptr(shard, which, ld, B); }
 extern "C" long long rkFDBatchLaunchCount(rkFD *fd){ FDImpl *fi = FI(fd); return ( fi && fi->engine ) ? fi->engine->launches() : 0; }
+/* environment reset (Engine::reset_envs): the listed environments restart as in a new rkFDUpdateInit, the others go on */
+extern "C" int rkFDBatchResetEnvs(rkFD *fd, int n, const int *envs, const double *q, const double *qd, const double *u)
+{
+  BATCH_GUARD(fd); NEED_ENGINE();
+  if( n < 0 ) return fail("rkFDBatchResetEnvs: n must be >= 0");
+  if( n == 0 ) return 0;
+  if( !envs || !q ) return fail("rkFDBatchResetEnvs: envs and q are needed");
+  std::vector<char> seen(fi->B, 0);
+  for(int i=0;i<n;i++){
+    const int e = envs[i];
+    if( e < 0 || e >= fi->B ) return fail("rkFDBatchResetEnvs: environment " + std::to_string(e) + " out of range [0, " + std::to_string(fi->B) + ")");
+    if( seen[e] ) return fail("rkFDBatchResetEnvs: environment " + std::to_string(e) + " listed twice");
+    seen[e] = 1;
+  }
+  try {
+    fi->engine->reset_envs_host(n, envs, q, qd, u);
+    if( !fi->batch ) mirror_env0(fd);
+  } catch(const std::exception &ex){ return fail(ex.what()); }
+  return 0;
+}
+extern "C" int rkFDBatchResetEnvsDevice(rkFD *fd, int shard, int n, const int *envs, const double *q, const double *qd, const double *u)
+{
+  BATCH_GUARD(fd); NEED_ENGINE();
+  if( shard < 0 || shard >= fi->engine->num_shards() ) return fail("rkFDBatchResetEnvsDevice: shard index out of range");
+  if( n < 0 ) return fail("rkFDBatchResetEnvsDevice: n must be >= 0");
+  if( n > 0 && ( !envs || !q ) ) return fail("rkFDBatchResetEnvsDevice: envs and q are needed");
+  TRY(fi->engine->reset_envs(shard, n, envs, q, qd, u));
+}
+extern "C" long long rkFDBatchResetKernelCount(rkFD *fd){ FDImpl *fi = FI(fd); return ( fi && fi->engine ) ? fi->engine->reset_kernels() : 0; }
 extern "C" const char *rkFDBatchLastError(void){ return g_err.c_str(); }
 extern "C" int rkFDBatchDeviceCount(void){ return device_count(); }
 extern "C" int rkFDB200MeasureFp64(double *tflops){ try { *tflops = measure_fp64_tflops(); } catch(const std::exception &ex){ return fail(ex.what()); } return 0; }

@@ -11,6 +11,7 @@
 
 #include <cuda_runtime.h>
 
+#include <cstdint>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -126,6 +127,53 @@ __global__ void __launch_bounds__(256) rkfd_perm_compose_kernel(const int * __re
   perm_new[d] = e; inv_new[e] = d;
 }
 
+/* ---- environment reset -------------------------------------------------------------------------------------------
+ * The committing evaluation of rkFDUpdateInit for a list of environments that sit in scattered slots: a launch covers whole
+ * blocks, so it cannot run in place without committing the neighbours as well.  The listed environments are gathered into
+ * a compact sub-state (slot i = list entry i), evaluated there by the shard's own kernel variant in mode 2, and the rows the
+ * re-sort permutes (plus the work class) are scattered back to their slots.  Results per environment do not depend on the
+ * slot or on the other environments of the launch, so an environment comes out exactly as a new engine started from the
+ * same state would have it.  The padding slots [n, ld) of the sub-state hold the zero state, like those of a shard. */
+constexpr int RESET_CHUNK = 65536;     /* sub-state capacity: longer lists run in chunks */
+constexpr int RESET_SEGS = 11, RESET_ROWS = 32;
+/* q, q' and u of the sub-state: the given rows, u from the environment's slot when none is given, zero on padding slots */
+__global__ void __launch_bounds__(256) rkfd_reset_gather_kernel(StateDev sub, const double * __restrict__ u_cur, int ld, int B, const int * __restrict__ inv,
+                                                                const int * __restrict__ envs, int n, const double * __restrict__ q, const double * __restrict__ qd,
+                                                                const double * __restrict__ u, int nq, int nl)
+{
+  const int i = blockIdx.x*blockDim.x + threadIdx.x;
+  if( i >= sub.ld ) return;
+  const int e = i < n ? envs[i] : -1;
+  const bool live = e >= 0 && e < B;
+  const int sl = live ? ( inv ? inv[e] : e ) : 0;
+  for(int k=0;k<nq;k++){
+    sub.q[0][(size_t)k*sub.ld + i] = live ? q[(size_t)i*nq + k] : 0.0;
+    sub.qd[0][(size_t)k*sub.ld + i] = live && qd ? qd[(size_t)i*nq + k] : 0.0;
+  }
+  for(int k=0;k<nl;k++) sub.u[(size_t)k*sub.ld + i] = !live ? 0.0 : ( u ? u[(size_t)i*nl + k] : u_cur[(size_t)k*ld + sl] );
+}
+/* row groups copied back from the sub-state (stride ld_sub, slot i) to the shard (stride ld, the environment's slot) */
+struct ResetRows { int nseg; int rows[RESET_SEGS], esz[RESET_SEGS]; const char *src[RESET_SEGS]; char *dst[RESET_SEGS]; };
+__global__ void __launch_bounds__(256) rkfd_reset_scatter_kernel(ResetRows rr, const int * __restrict__ envs, int n, int B, const int * __restrict__ inv, int ld_sub, int ld)
+{
+  const int i = blockIdx.x*blockDim.x + threadIdx.x;
+  if( i >= n ) return;
+  const int e = envs[i];
+  if( e < 0 || e >= B ) return;
+  const int sl = inv ? inv[e] : e;
+  /* blockIdx.y: rows [r0, r0 + RESET_ROWS) of the concatenated groups (mighty.ztk has 6,000 rows of anchors and forces) */
+  const int r0 = blockIdx.y*RESET_ROWS, r1 = r0 + RESET_ROWS;
+  for(int g=0, base=0; g<rr.nseg && base<r1; base+=rr.rows[g], g++){
+    const int a = max(r0, base) - base, b = min(r1, base + rr.rows[g]) - base;
+    for(int r=a; r<b; r++){
+      const size_t si = (size_t)r*ld_sub + i, di = (size_t)r*ld + sl;
+      if( rr.esz[g] == 8 ) ((unsigned long long*)rr.dst[g])[di] = ((const unsigned long long*)rr.src[g])[si];
+      else if( rr.esz[g] == 4 ) ((unsigned int*)rr.dst[g])[di] = ((const unsigned int*)rr.src[g])[si];
+      else rr.dst[g][di] = rr.src[g][si];
+    }
+  }
+}
+
 /* rows k0..k0+n-1 of an SoA array <- one value per row, every environment (rkFDChainSetDis/SetVel and
  * rkJointMotorSetInput on a running simulator: the reference's cell windows alias fd->dis/vel, rkfd_sim.c:277-287) */
 __global__ void rkfd_fill_rows_kernel(double * __restrict__ dst, int ld, int B, int n, const double * __restrict__ vals)
@@ -215,6 +263,8 @@ struct Shard {
   int *perm = nullptr, *inv = nullptr, *perm_buf[2] = {nullptr, nullptr}, *inv_buf = nullptr, *newpos = nullptr, *bins = nullptr; unsigned char *key = nullptr;
   void *ptmp = nullptr; size_t ptmp_bytes = 0; int perm_cur = 0, steps_since_sort = 0; long long sorts = 0;
   std::vector<int> h_perm; bool h_perm_valid = false;
+  /* environment reset (Engine::reset_envs): one buffer for the sub-state of up to rcap environments and the host path's staging */
+  char *rbuf = nullptr; int rcap = 0;
   std::vector<void*> allocs;
 };
 
@@ -363,6 +413,7 @@ Engine::~Engine()
       for(int i=0;i<Shard::NRING;i++){ cudaEventDestroy(s->ring_done[i]); cudaEventDestroy(s->ring_ready[i]); }
       cudaStreamDestroy(s->h2d_stream); cudaStreamDestroy(s->d2h_stream); }
     for(void *p : s->allocs) cudaFree(p);
+    cudaFree(s->rbuf);
     if( s->own_stream && s->stream ) cudaStreamDestroy(s->stream);
     delete s;
   }
@@ -379,14 +430,14 @@ void Engine::upload_model(Shard &s)
   owner = id_;
 }
 
-void Engine::launch(Shard &s, int mode, int nsteps)
+/* the shard's step kernel on `st`: the shard's own state, or the sub-state of a reset */
+void Engine::launch(Shard &s, const StateDev &st, int cur, int mode, int nsteps)
 {
   CK(cudaSetDevice(s.dev));
   upload_model(s);
-  s.kv->launch(s.st, s.cur, mode, nsteps, (s.ld + s.kv->block - 1)/s.kv->block, s.smem, s.stream);
+  s.kv->launch(st, cur, mode, nsteps, (st.ld + s.kv->block - 1)/s.kv->block, s.smem, s.stream);
   CK(cudaGetLastError());
   launches_++;
-  if( mode == 0 && (nsteps & 1) ) s.cur ^= 1;
 }
 
 static const std::vector<int> &host_perm(Shard &s)
@@ -437,6 +488,118 @@ void Engine::resort(Shard &s)
   s.perm = pn; s.inv = s.inv_buf; s.perm_cur ^= 1; s.h_perm_valid = false; s.steps_since_sort = 0; s.sorts++;
 }
 
+/* Shard::rbuf for a reset sub-state of leading dimension ld (a multiple of 512, <= cap): the host path's staging for cap
+ * environments (ids, q, q', u), then the rows a new engine holds zero (contiguous: one memset clears them), then q, q', u and
+ * the evaluation's workspaces.  With base = 0 it gives the size. */
+struct ResetLayout { StateDev st; size_t zero_ofs, zero_bytes, bytes; int *envs; double *q, *qd, *u; };
+static ResetLayout reset_layout(const Shard &s, const ModelDev &m, int ld, int cap, char *base)
+{
+  const size_t nq = m.nq > 0 ? m.nq : 1, nl = m.nl > 0 ? m.nl : 1, ns = m.nslot > 0 ? m.nslot : 1, nfw = m.nfw > 0 ? m.nfw : 1, L = ld, C = cap;
+  size_t off = 0;
+  auto take = [&](size_t bytes){ void *p = (void*)((uintptr_t)base + off); off += (bytes + 255) & ~(size_t)255; return p; };
+  ResetLayout r; std::memset(&r, 0, sizeof r);
+  r.envs = (int*)take(4*C); r.q = (double*)take(8*nq*C); r.qd = (double*)take(8*nq*C); r.u = (double*)take(8*nl*C);
+  StateDev &st = r.st;
+  st.B = ld; st.ld = ld;
+  r.zero_ofs = off;
+  st.qdd = (double*)take(8*nq*L); st.piv_prev = (double*)take(8*nq*L); st.cflags = (unsigned long long*)take(8*nfw*L);
+  st.cref = (double*)take(8*3*ns*L); st.cf = (double*)take(8*3*ns*L);
+  st.piv_type = (unsigned int*)take(4*L); st.status = (int*)take(4*L);
+  if( s.st.work ) st.work = (unsigned char*)take(L);
+  r.zero_bytes = off - r.zero_ofs;
+  for(int k=0;k<2;k++){ st.q[k] = (double*)take(8*nq*L); st.qd[k] = (double*)take(8*nq*L); }
+  st.u = (double*)take(8*nl*L);
+  if( s.st.scratch ) st.scratch = (double*)take(8*(size_t)m.nscratch*L);
+  if( s.st.ws ) st.ws = (double*)take(8*(L/32)*(size_t)m.ws_doubles);
+  if( s.st.ws1 ) st.ws1 = (double*)take(8*(size_t)m.ws1_doubles*L);
+  r.bytes = off;
+  return r;
+}
+/* the sub-state for lists of up to n environments (allocated on first use, grown when a longer list comes) */
+static int reset_reserve(Shard &s, const ModelDev &m, int n)
+{
+  const int ld = ((n < RESET_CHUNK ? n : RESET_CHUNK) + 511) & ~511;
+  if( ld > s.rcap ){
+    CK(cudaStreamSynchronize(s.stream));      /* earlier resets may still use the old buffer */
+    CK(cudaFree(s.rbuf)); s.rbuf = nullptr; s.rcap = 0;
+    const size_t bytes = reset_layout(s, m, ld, ld, nullptr).bytes;
+    CK(cudaMalloc(&s.rbuf, bytes)); CK(cudaMemset(s.rbuf, 0, bytes));
+    CK(cudaDeviceSynchronize());              /* the zero fill runs on the legacy stream */
+    s.rcap = ld;
+  }
+  return ld;
+}
+
+void Engine::reset_chunk(Shard &s, int n, const int *envs, const double *q, const double *qd, const double *u)
+{
+  const int nq = model_.nq, nl = model_.nl, ns = model_.nslot > 0 ? model_.nslot : 1, nfw = model_.nfw > 0 ? model_.nfw : 1;
+  const int ld = reset_reserve(s, model_, n);
+  const ResetLayout r = reset_layout(s, model_, ld, s.rcap, s.rbuf);
+  const StateDev &sub = r.st;
+  CK(cudaMemsetAsync(s.rbuf + r.zero_ofs, 0, r.zero_bytes, s.stream));
+  rkfd_reset_gather_kernel<<<ld/256, 256, 0, s.stream>>>(sub, s.st.u, s.ld, s.B, s.inv, envs, n, q, qd, u, nq, nl);
+  CK(cudaGetLastError());
+  launch(s, sub, 0, 2, 0);                    /* rkFDUpdateInit's committing evaluation, on the sub-state */
+  ResetRows rr; std::memset(&rr, 0, sizeof rr);
+  auto seg = [&](const void *src, void *dst, int rows, int esz){ rr.src[rr.nseg] = (const char*)src; rr.dst[rr.nseg] = (char*)dst; rr.rows[rr.nseg] = rows; rr.esz[rr.nseg] = esz; rr.nseg++; };
+  seg(sub.q[0], s.st.q[s.cur], nq, 8); seg(sub.qd[0], s.st.qd[s.cur], nq, 8); seg(sub.qdd, s.st.qdd, nq, 8); seg(sub.u, s.st.u, nl, 8);
+  seg(sub.piv_prev, s.st.piv_prev, nq, 8); seg(sub.cflags, s.st.cflags, nfw, 8); seg(sub.cref, s.st.cref, 3*ns, 8); seg(sub.cf, s.st.cf, 3*ns, 8);
+  seg(sub.piv_type, s.st.piv_type, 1, 4); seg(sub.status, s.st.status, 1, 4);
+  if( s.st.work ) seg(sub.work, s.st.work, 1, 1);
+  int rows = 0; for(int g=0; g<rr.nseg; g++) rows += rr.rows[g];
+  rkfd_reset_scatter_kernel<<<dim3((n + 255)/256, (rows + RESET_ROWS - 1)/RESET_ROWS), 256, 0, s.stream>>>(rr, envs, n, s.B, s.inv, ld, s.ld);
+  CK(cudaGetLastError());
+  reset_kernels_ += 3;                        /* zero fill, gather, scatter */
+}
+
+void Engine::reset_envs(int si, int n, const int *envs, const double *q, const double *qd, const double *u)
+{
+  if( si < 0 || si >= (int)shards_.size() ) throw std::runtime_error("rokifd_b200: reset: shard index out of range");
+  if( n <= 0 ) return;
+  Shard &s = *shards_[si];
+  const int nq = model_.nq, nl = model_.nl;
+  int prev = 0; CK(cudaGetDevice(&prev)); CK(cudaSetDevice(s.dev));
+  for(int c0=0; c0<n; c0+=RESET_CHUNK){
+    const int nc = n - c0 < RESET_CHUNK ? n - c0 : RESET_CHUNK;
+    reset_chunk(s, nc, envs + c0, q + (size_t)c0*nq, qd ? qd + (size_t)c0*nq : nullptr, u ? u + (size_t)c0*nl : nullptr);
+  }
+  CK(cudaSetDevice(prev));
+}
+
+void Engine::reset_envs_host(int n, const int *envs, const double *q, const double *qd, const double *u)
+{
+  if( n <= 0 ) return;
+  const int nq = model_.nq, nl = model_.nl;
+  int prev = 0; CK(cudaGetDevice(&prev));
+  for(Shard *s : shards_){
+    /* this shard's part of the list, with local indices, and its rows */
+    std::vector<int> ids; std::vector<double> hq, hqd, hu;
+    for(int i=0;i<n;i++){
+      const int e = envs[i] - s->e0;
+      if( e < 0 || e >= s->B ) continue;
+      ids.push_back(e);
+      hq.insert(hq.end(), q + (size_t)i*nq, q + (size_t)(i+1)*nq);
+      if( qd ) hqd.insert(hqd.end(), qd + (size_t)i*nq, qd + (size_t)(i+1)*nq);
+      if( u ) hu.insert(hu.end(), u + (size_t)i*nl, u + (size_t)(i+1)*nl);
+    }
+    CK(cudaSetDevice(s->dev));
+    for(int c0=0; c0<(int)ids.size(); c0+=RESET_CHUNK){
+      const int nc = (int)ids.size() - c0 < RESET_CHUNK ? (int)ids.size() - c0 : RESET_CHUNK;
+      const int ld = reset_reserve(*s, model_, nc);
+      const ResetLayout r = reset_layout(*s, model_, ld, s->rcap, s->rbuf);
+      /* the staging is reused by the next chunk only after this chunk's kernels (same stream) */
+      CK(cudaMemcpyAsync(r.envs, ids.data() + c0, (size_t)nc*sizeof(int), cudaMemcpyHostToDevice, s->stream));
+      CK(cudaMemcpyAsync(r.q, hq.data() + (size_t)c0*nq, (size_t)nc*nq*sizeof(double), cudaMemcpyHostToDevice, s->stream));
+      if( qd ) CK(cudaMemcpyAsync(r.qd, hqd.data() + (size_t)c0*nq, (size_t)nc*nq*sizeof(double), cudaMemcpyHostToDevice, s->stream));
+      if( u ) CK(cudaMemcpyAsync(r.u, hu.data() + (size_t)c0*nl, (size_t)nc*nl*sizeof(double), cudaMemcpyHostToDevice, s->stream));
+      reset_chunk(*s, nc, r.envs, r.q, qd ? r.qd : nullptr, u ? r.u : nullptr);
+    }
+    /* the host vectors are read by the copies: finish before they go out of scope */
+    CK(cudaStreamSynchronize(s->stream));
+  }
+  CK(cudaSetDevice(prev));
+}
+
 void Engine::step(int nsteps)
 {
   if( nsteps <= 0 ) return;
@@ -444,14 +607,15 @@ void Engine::step(int nsteps)
   for(Shard *s : shards_){
     if( resort_interval_ > 0 && s->B > 32 && s->steps_since_sort >= resort_interval_ ){      /* one warp: nothing to group */ CK(cudaSetDevice(s->dev)); resort(*s); }
     s->steps_since_sort += nsteps;
-    launch(*s, 0, nsteps);
+    launch(*s, s->st, s->cur, 0, nsteps);
+    if( nsteps & 1 ) s->cur ^= 1;
   }
   CK(cudaSetDevice(prev));
 }
 void Engine::eval(bool ref)
 {
   int prev = 0; CK(cudaGetDevice(&prev));
-  for(Shard *s : shards_) launch(*s, ref ? 2 : 1, 0);
+  for(Shard *s : shards_) launch(*s, s->st, s->cur, ref ? 2 : 1, 0);
   CK(cudaSetDevice(prev));
 }
 void Engine::sync()

@@ -61,15 +61,26 @@ class Engine {
   long long launches() const { return launches_; }
   long long resort_kernels() const { return resort_kernels_; }      /* kernels launched by the re-sorts (key, offsets, assign, row permutations, order) */
 
+  /* environment reset: environments envs[0..n) of shard `shard` (local indices) restart from (q, q', u) - device arrays,
+   * env-major [n][nq] / [n][nl] - with every other per-environment row as a new engine holds it, and the committing
+   * evaluation of rkFDUpdateInit runs for them alone.  qd null: zero, u null: the current input.  Entries outside [0, B) are
+   * skipped; duplicates leave the environment with one of their states.  Stream-ordered on the shard's stream (the first
+   * call, and a call with a longer list than any before, allocates and synchronises the device) */
+  void reset_envs(int shard, int n, const int *envs, const double *q, const double *qd, const double *u);
+  /* the same from host arrays, global environment indices (in range, no duplicates: the caller checks); synchronous */
+  void reset_envs_host(int n, const int *envs, const double *q, const double *qd, const double *u);
+  long long reset_kernels() const { return reset_kernels_; }        /* gather, zero fill and scatter launches of the resets */
+
  private:
   void upload_model(Shard &s);
-  void launch(Shard &s, int mode, int nsteps);
+  void launch(Shard &s, const StateDev &st, int cur, int mode, int nsteps);
   void resort(Shard &s);
+  void reset_chunk(Shard &s, int n, const int *envs, const double *q, const double *qd, const double *u);
   int resort_interval_ = 0;
   ModelDev model_, model_tm_;     /* model_tm_: the same table with the tensor-memory scratch map (generic TM kernel) */
   int B_;
   std::vector<Shard*> shards_;
-  long long launches_ = 0, resort_kernels_ = 0;
+  long long launches_ = 0, resort_kernels_ = 0, reset_kernels_ = 0;
   int id_;
 };
 
