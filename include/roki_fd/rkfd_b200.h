@@ -368,6 +368,25 @@ __ROKI_FD_EXPORT long long rkFDBatchLaunchCount(rkFD *fd);
 __ROKI_FD_EXPORT int rkFDBatchResetEnvs(rkFD *fd, int n, const int *envs, const double *q, const double *qd, const double *u);
 __ROKI_FD_EXPORT int rkFDBatchResetEnvsDevice(rkFD *fd, int shard, int n, const int *envs, const double *q, const double *qd, const double *u);
 __ROKI_FD_EXPORT long long rkFDBatchResetKernelCount(rkFD *fd);       /* gather, zero fill and scatter launches of the resets so far */
+/* Link kinematics: world frames and velocities of selected links of every environment, from the committed state (what
+ * rkFDBatchGetState returns: q and q' of the current buffer, and for breakable-float joints the broken bit of rkFDBatchGetPivot).
+ * The frames are computed from the committed q with the joint model of the step kernel's pass 1 (revolute sin/cos from
+ * sincos(q)): they agree with the step kernel's internal frames to rounding.  Nothing of the engine's state is written.
+ * links: host array of nlink link indices in [0, rkFDBatchLinkNum) - moving chains in registration order, links in chain order
+ * (the order of the motor input u); duplicates are allowed; NULL: all links, then nlink must be rkFDBatchLinkNum.  nlink = 0
+ * does nothing.  nlink < 0, nlink > 32 (MAX_LINKS) or an index out of range is refused, and nothing is written.
+ * frame[env][k][12]: the world-from-link rotation R of links[k], row-major, then the world position p of the link origin.
+ * vel[env][k][6]: the linear velocity of the link origin, then the angular velocity, both in world axes.
+ * Either pointer may be NULL: that output is neither computed nor written.  An unbroken breakable-float joint contributes no
+ * joint velocity (it is rigid).
+ * rkFDBatchGetLinkFrames: host arrays, global environment index, every shard; synchronous, like rkFDBatchGetState.
+ * rkFDBatchGetLinkFramesDevice: device buffers on the device of shard `shard`, [Bs][nlink][12] and [Bs][nlink][6], indexed by
+ * the environment local to the shard (the engine maps its re-sorted slots itself).  Stream-ordered on the engine's stream,
+ * without a host synchronisation or an allocation.
+ * Both need rkFDUpdateInit; each launches one kernel per shard it covers (rkFDBatchLinkFrameKernelCount). */
+__ROKI_FD_EXPORT int rkFDBatchGetLinkFrames(rkFD *fd, int nlink, const int *links, double *frame, double *vel);
+__ROKI_FD_EXPORT int rkFDBatchGetLinkFramesDevice(rkFD *fd, int shard, int nlink, const int *links, double *frame, double *vel);
+__ROKI_FD_EXPORT long long rkFDBatchLinkFrameKernelCount(rkFD *fd);   /* kinematics launches of the calls so far */
 /* the flattened model of the last rkFDUpdateInit as text (host side; also after an rkFDUpdateInit that found no device):
  * returns the length needed */
 __ROKI_FD_EXPORT int rkFDB200DescribeModel(rkFD *fd, char *buf, int cap);

@@ -84,6 +84,8 @@ def lib():
         "rkFDBatchDevicePtr": (vp, [vp, ci, ci, _ip, _ip]), "rkFDBatchLaunchCount": (C.c_longlong, [vp]),
         "rkFDBatchResetEnvs": (ci, [vp, ci, vp, vp, vp, vp]), "rkFDBatchResetEnvsDevice": (ci, [vp, ci, ci, vp, vp, vp, vp]),
         "rkFDBatchResetKernelCount": (C.c_longlong, [vp]),
+        "rkFDBatchGetLinkFrames": (ci, [vp, ci, vp, vp, vp]), "rkFDBatchGetLinkFramesDevice": (ci, [vp, ci, ci, vp, vp, vp]),
+        "rkFDBatchLinkFrameKernelCount": (C.c_longlong, [vp]),
         "rkFDB200DescribeModel": (ci, [vp, C.c_char_p, ci]), "rkFDBatchLastError": (C.c_char_p, []), "rkFDBatchDeviceCount": (ci, []), "rkFDB200MeasureFp64": (ci, [_dp]),
     }
     for name, (res, args) in sig.items():
@@ -455,6 +457,36 @@ class RkFD:
     @property
     def reset_kernel_count(self):
         return lib().rkFDBatchResetKernelCount(self.h)
+
+    def batch_get_link_frames(self, links=None, frames=True, vel=True):
+        """rkFDBatchGetLinkFrames: world frames (B, n, 12) - R row-major, then p - and velocities (B, n, 6) - linear, angular,
+        world axes - of links (indices in flat_links() order; None: all links), from the committed state.  An output not
+        requested is returned as None."""
+        if links is None:
+            n, pl = self.link_num, None
+        else:
+            pl = np.ascontiguousarray(links, np.int32).reshape(-1)
+            n = pl.shape[0]
+        B = self.env_num
+        fr = np.zeros((B, n, 12)) if frames else None
+        v = np.zeros((B, n, 6)) if vel else None
+        self._ck(lib().rkFDBatchGetLinkFrames(self.h, n, _ptr(pl), _ptr(fr), _ptr(v)))
+        return fr, v
+
+    def batch_get_link_frames_device(self, shard, links, frame_ptr, vel_ptr):
+        """rkFDBatchGetLinkFramesDevice: raw device addresses (e.g. torch CUDA tensor .data_ptr(), or None) of float64
+        frame[Bs][n][12] and vel[Bs][n][6] of shard `shard`, indexed by the shard's local environment; stream-ordered on the
+        engine's stream.  links: a host list of link indices (None: all links)."""
+        if links is None:
+            n, pl = self.link_num, None
+        else:
+            pl = np.ascontiguousarray(links, np.int32).reshape(-1)
+            n = pl.shape[0]
+        self._ck(lib().rkFDBatchGetLinkFramesDevice(self.h, shard, n, _ptr(pl), _ptr(frame_ptr), _ptr(vel_ptr)))
+
+    @property
+    def link_frame_kernel_count(self):
+        return lib().rkFDBatchLinkFrameKernelCount(self.h)
 
 
 def create_world(world: World, B=None, devices=None):

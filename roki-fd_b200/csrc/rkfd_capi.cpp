@@ -577,6 +577,23 @@ extern "C" int rkFDBatchResetEnvsDevice(rkFD *fd, int shard, int n, const int *e
   TRY(fi->engine->reset_envs(shard, n, envs, q, qd, u));
 }
 extern "C" long long rkFDBatchResetKernelCount(rkFD *fd){ FDImpl *fi = FI(fd); return ( fi && fi->engine ) ? fi->engine->reset_kernels() : 0; }
+/* link kinematics (Engine::link_frames): world frames and velocities of selected links from the committed state */
+extern "C" int rkFDBatchGetLinkFrames(rkFD *fd, int nlink, const int *links, double *frame, double *vel)
+{
+  BATCH_GUARD(fd); NEED_ENGINE();
+  KinDev t; std::string err;
+  if( !kin_table(fi->engine->model(), nlink, links, t, err) ) return fail("rkFDBatchGetLinkFrames: " + err);
+  TRY(fi->engine->link_frames_host(t, frame, vel));
+}
+extern "C" int rkFDBatchGetLinkFramesDevice(rkFD *fd, int shard, int nlink, const int *links, double *frame, double *vel)
+{
+  BATCH_GUARD(fd); NEED_ENGINE();
+  if( shard < 0 || shard >= fi->engine->num_shards() ) return fail("rkFDBatchGetLinkFramesDevice: shard index out of range");
+  KinDev t; std::string err;
+  if( !kin_table(fi->engine->model(), nlink, links, t, err) ) return fail("rkFDBatchGetLinkFramesDevice: " + err);
+  TRY(fi->engine->link_frames(shard, t, frame, vel));
+}
+extern "C" long long rkFDBatchLinkFrameKernelCount(rkFD *fd){ FDImpl *fi = FI(fd); return ( fi && fi->engine ) ? fi->engine->link_frame_kernels() : 0; }
 extern "C" const char *rkFDBatchLastError(void){ return g_err.c_str(); }
 extern "C" int rkFDBatchDeviceCount(void){ return device_count(); }
 extern "C" int rkFDB200MeasureFp64(double *tflops){ try { *tflops = measure_fp64_tflops(); } catch(const std::exception &ex){ return fail(ex.what()); } return 0; }

@@ -18,6 +18,7 @@
 #include <stdexcept>
 
 #include "rkfd_kernel.cuh"
+#include "rkfd_kin.cuh"
 #include "rkfd_model.h"
 
 namespace rkfd {
@@ -174,6 +175,51 @@ __global__ void __launch_bounds__(256) rkfd_reset_scatter_kernel(ResetRows rr, c
   }
 }
 
+/* ---- link kinematics (rkFDBatchGetLinkFrames) ---------------------------------------------------------------------
+ * One thread per slot walks the links of the table outward (rkfd_kin.cuh) on the committed q, q' (SoA rows: coalesced
+ * loads) and keeps the frames that later children need in a shared-memory column per thread.  The outputs are env-major
+ * (frame[env][k][12], vel[env][k][6]): every thread puts its rows into a shared-memory tile, and the block then writes the
+ * tile environment by environment through perm, as the second half of rkfd_gather_kernel does - each output double is
+ * written once, by contiguous warp stores.  The table is a __grid_constant__ parameter: the __constant__ banks belong to the
+ * step-kernel variants and to whichever engine uploaded its model last. */
+constexpr int KIN_MAX_THREADS = 128;
+constexpr size_t KIN_TILE_BYTES = 64*1024;     /* blocks shrink (down to one warp) until tile and keep slots fit in this */
+struct KinSrcDev {
+  const double *qp, *qdp; const unsigned int *pv; int ld, sl;
+  __device__ double q(int k) const { return __ldg(qp + (size_t)k*ld + sl); }
+  __device__ double qd(int k) const { return __ldg(qdp + (size_t)k*ld + sl); }
+  __device__ unsigned piv() const { return __ldg(pv + sl); }
+};
+struct KinKeepDev {
+  double *col; int nb;
+  __device__ double ld(int s, int c) const { return col[(s*KIN_KEEP + c)*nb]; }
+  __device__ void st(int s, int c, double v){ col[(s*KIN_KEEP + c)*nb] = v; }
+};
+struct KinOutDev {
+  double *tf, *tv;
+  __device__ void frame(int k, int c, double v){ tf[12*k + c] = v; }
+  __device__ void vel(int k, int c, double v){ tv[6*k + c] = v; }
+};
+__global__ void __launch_bounds__(KIN_MAX_THREADS) rkfd_link_frames_kernel(const __grid_constant__ KinDev t, const double * __restrict__ q,
+                                                                           const double * __restrict__ qd, const unsigned int * __restrict__ piv,
+                                                                           const int * __restrict__ perm, int B, int ld,
+                                                                           double * __restrict__ frame, double * __restrict__ vel)
+{
+  extern __shared__ double kin_smem[];
+  const int nb = blockDim.x, tid = threadIdx.x, e0 = blockIdx.x*nb, sl = e0 + tid;
+  /* tile rows padded to an odd number of doubles: the lanes of a warp hit different banks */
+  const int fw = frame ? 12*t.nsel : 0, vw = vel ? 6*t.nsel : 0, fs = fw ? (fw | 1) : 0, vs = vw ? (vw | 1) : 0;
+  double *tf = kin_smem, *tv = tf + (size_t)nb*fs, *keep = tv + (size_t)nb*vs;
+  if( sl < B ){
+    const KinSrcDev S{q, qd, piv, ld, sl}; KinKeepDev K{keep + tid, nb}; KinOutDev O{tf + (size_t)tid*fs, tv + (size_t)tid*vs};
+    kin_walk(t, S, K, O, frame != nullptr, vel != nullptr);
+  }
+  __syncthreads();
+  const int ne = min(nb, B - e0);
+  for(int i=tid; i<ne*fw; i+=nb){ const int e = i/fw, c = i - e*fw; frame[(size_t)(perm ? perm[e0 + e] : e0 + e)*fw + c] = tf[e*fs + c]; }
+  for(int i=tid; i<ne*vw; i+=nb){ const int e = i/vw, c = i - e*vw; vel[(size_t)(perm ? perm[e0 + e] : e0 + e)*vw + c] = tv[e*vs + c]; }
+}
+
 /* rows k0..k0+n-1 of an SoA array <- one value per row, every environment (rkFDChainSetDis/SetVel and
  * rkJointMotorSetInput on a running simulator: the reference's cell windows alias fd->dis/vel, rkfd_sim.c:277-287) */
 __global__ void rkfd_fill_rows_kernel(double * __restrict__ dst, int ld, int B, int n, const double * __restrict__ vals)
@@ -265,6 +311,8 @@ struct Shard {
   std::vector<int> h_perm; bool h_perm_valid = false;
   /* environment reset (Engine::reset_envs): one buffer for the sub-state of up to rcap environments and the host path's staging */
   char *rbuf = nullptr; int rcap = 0;
+  /* link kinematics: the host path's device outputs (allocated on first use, grown when a call needs more) */
+  double *kbuf = nullptr; size_t kcap = 0; bool kin_smem_attr = false;
   std::vector<void*> allocs;
 };
 
@@ -413,7 +461,7 @@ Engine::~Engine()
       for(int i=0;i<Shard::NRING;i++){ cudaEventDestroy(s->ring_done[i]); cudaEventDestroy(s->ring_ready[i]); }
       cudaStreamDestroy(s->h2d_stream); cudaStreamDestroy(s->d2h_stream); }
     for(void *p : s->allocs) cudaFree(p);
-    cudaFree(s->rbuf);
+    cudaFree(s->rbuf); cudaFree(s->kbuf);
     if( s->own_stream && s->stream ) cudaStreamDestroy(s->stream);
     delete s;
   }
@@ -597,6 +645,52 @@ void Engine::reset_envs_host(int n, const int *envs, const double *q, const doub
     /* the host vectors are read by the copies: finish before they go out of scope */
     CK(cudaStreamSynchronize(s->stream));
   }
+  CK(cudaSetDevice(prev));
+}
+
+void Engine::kin_launch(Shard &s, const KinDev &t, double *frame, double *vel)
+{
+  const size_t fw = 12*(size_t)t.nsel, vw = 6*(size_t)t.nsel;
+  const size_t per_env = sizeof(double)*((frame ? (fw | 1) : 0) + (vel ? (vw | 1) : 0) + (size_t)KIN_KEEP*t.nkeep);
+  int nb = KIN_MAX_THREADS;
+  while( nb > 32 && nb*per_env > KIN_TILE_BYTES ) nb >>= 1;
+  const size_t smem = nb*per_env;
+  if( smem > 227*1024 ) throw std::runtime_error("rokifd_b200: link frames: the output tile does not fit in shared memory");
+  if( smem > 48*1024 && !s.kin_smem_attr ){
+    CK(cudaFuncSetAttribute(rkfd_link_frames_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227*1024)); s.kin_smem_attr = true; }
+  rkfd_link_frames_kernel<<<(s.B + nb - 1)/nb, nb, smem, s.stream>>>(t, s.st.q[s.cur], s.st.qd[s.cur], s.st.piv_type, s.perm, s.B, s.ld, frame, vel);
+  CK(cudaGetLastError());
+  kin_kernels_++;
+}
+
+void Engine::link_frames(int si, const KinDev &t, double *frame, double *vel)
+{
+  if( si < 0 || si >= (int)shards_.size() ) throw std::runtime_error("rokifd_b200: link frames: shard index out of range");
+  if( t.nsel == 0 || ( !frame && !vel ) ) return;
+  int prev = 0; CK(cudaGetDevice(&prev)); CK(cudaSetDevice(shards_[si]->dev));
+  kin_launch(*shards_[si], t, frame, vel);
+  CK(cudaSetDevice(prev));
+}
+
+void Engine::link_frames_host(const KinDev &t, double *frame, double *vel)
+{
+  if( t.nsel == 0 || ( !frame && !vel ) ) return;
+  const size_t fw = 12*(size_t)t.nsel, vw = 6*(size_t)t.nsel;
+  int prev = 0; CK(cudaGetDevice(&prev));
+  for(Shard *s : shards_){
+    CK(cudaSetDevice(s->dev));
+    const size_t need = (size_t)s->B*((frame ? fw : 0) + (vel ? vw : 0));
+    if( need > s->kcap ){
+      CK(cudaStreamSynchronize(s->stream));      /* an earlier call's copies may still read the old buffer */
+      CK(cudaFree(s->kbuf)); s->kbuf = nullptr; s->kcap = 0;
+      CK(cudaMalloc(&s->kbuf, need*sizeof(double))); s->kcap = need;
+    }
+    double *df = frame ? s->kbuf : nullptr, *dv = vel ? s->kbuf + ( frame ? (size_t)s->B*fw : 0 ) : nullptr;
+    kin_launch(*s, t, df, dv);
+    if( frame ) CK(cudaMemcpyAsync(frame + (size_t)s->e0*fw, df, (size_t)s->B*fw*sizeof(double), cudaMemcpyDeviceToHost, s->stream));
+    if( vel ) CK(cudaMemcpyAsync(vel + (size_t)s->e0*vw, dv, (size_t)s->B*vw*sizeof(double), cudaMemcpyDeviceToHost, s->stream));
+  }
+  for(Shard *s : shards_){ CK(cudaSetDevice(s->dev)); CK(cudaStreamSynchronize(s->stream)); }
   CK(cudaSetDevice(prev));
 }
 

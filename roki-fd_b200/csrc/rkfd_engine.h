@@ -71,16 +71,26 @@ class Engine {
   void reset_envs_host(int n, const int *envs, const double *q, const double *qd, const double *u);
   long long reset_kernels() const { return reset_kernels_; }        /* gather, zero fill and scatter launches of the resets */
 
+  /* link kinematics (rkfd_kin.cuh): world frames [B][nsel][12] (R row-major, p) and velocities [B][nsel][6] (linear, angular;
+   * world axes) of the output columns of table `t`, from the committed state; a null output is neither computed nor written.
+   * Nothing of the engine's state is written.  link_frames: device buffers of shard `shard`, indexed by the environment local
+   * to the shard; stream-ordered on the shard's stream, no allocation.  link_frames_host: host arrays, global environment
+   * index, every shard; synchronous */
+  void link_frames(int shard, const KinDev &t, double *frame, double *vel);
+  void link_frames_host(const KinDev &t, double *frame, double *vel);
+  long long link_frame_kernels() const { return kin_kernels_; }     /* kinematics launches (one per shard and call) */
+
  private:
   void upload_model(Shard &s);
   void launch(Shard &s, const StateDev &st, int cur, int mode, int nsteps);
   void resort(Shard &s);
   void reset_chunk(Shard &s, int n, const int *envs, const double *q, const double *qd, const double *u);
+  void kin_launch(Shard &s, const KinDev &t, double *frame, double *vel);
   int resort_interval_ = 0;
   ModelDev model_, model_tm_;     /* model_tm_: the same table with the tensor-memory scratch map (generic TM kernel) */
   int B_;
   std::vector<Shard*> shards_;
-  long long launches_ = 0, resort_kernels_ = 0, reset_kernels_ = 0;
+  long long launches_ = 0, resort_kernels_ = 0, reset_kernels_ = 0, kin_kernels_ = 0;
   int id_;
 };
 

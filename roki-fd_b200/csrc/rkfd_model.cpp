@@ -319,4 +319,45 @@ bool build_model(const WorldHost &w, ModelDev &m, std::string &err)
   return true;
 }
 
+bool kin_table(const ModelDev &m, int nlink, const int *links, KinDev &t, std::string &err)
+{
+  std::memset(&t, 0, sizeof t);
+  if( nlink < 0 ){ err = "the number of links must be >= 0"; return false; }
+  if( nlink > MAX_LINKS ){ err = "at most " + std::to_string(MAX_LINKS) + " links per call (MAX_LINKS)"; return false; }
+  if( !links && nlink != m.nl ){ err = "links == NULL (all links) needs nlink == " + std::to_string(m.nl); return false; }
+  for(int k=0;k<nlink;k++){ const int i = links ? links[k] : k;
+    if( i < 0 || i >= m.nl ){ err = "link index " + std::to_string(i) + " out of range [0, " + std::to_string(m.nl) + ")"; return false; } }
+  /* links to visit: the requested ones and their ancestors (parents precede children in the model) */
+  bool need[MAX_LINKS] = {false};
+  for(int k=0;k<nlink;k++) for(int i = links ? links[k] : k; i >= 0 && !need[i]; i = m.link[i].parent) need[i] = true;
+  int pos[MAX_LINKS];
+  for(int i=0;i<m.nl;i++){
+    const LinkDev &d = m.link[i]; KinLinkDev &l = t.link[i];
+    std::memcpy(l.Ro, d.Ro, sizeof l.Ro); std::memcpy(l.po, d.po, sizeof l.po);
+    l.cls = d.rcls; l.sg = d.rcls == RO_RXP ? 1.0 : ( d.rcls == RO_RXM ? -1.0 : 0.0 ); l.pz = d.pz;
+    l.parent = d.parent; l.jtype = d.jtype; l.qofs = d.qofs; l.keep = -1; l.omask = 0u;
+    if( d.jtype == J_BRFLOAT ) t.brk = 1;
+    pos[i] = -1;
+    if( need[i] ){ pos[i] = t.nwalk; t.walk[t.nwalk++] = i; }
+  }
+  for(int k=0;k<nlink;k++) t.link[links ? links[k] : k].omask |= 1u << k;
+  t.nsel = nlink;
+  /* a parent that is not the link visited just before its child is read back from a keep slot; slots are reused once their
+   * last reader has loaded them */
+  int last[MAX_LINKS];
+  for(int i=0;i<MAX_LINKS;i++) last[i] = -1;
+  for(int w=0; w<t.nwalk; w++){ const int i = t.walk[w], p = m.link[i].parent;
+    if( p >= 0 && ( w == 0 || t.walk[w-1] != p ) ) last[p] = w; }
+  int owner[MAX_LINKS];      /* slot -> link kept there, -1 free */
+  for(int s=0;s<MAX_LINKS;s++) owner[s] = -1;
+  for(int w=0; w<t.nwalk; w++){
+    for(int s=0;s<t.nkeep;s++) if( owner[s] >= 0 && last[owner[s]] <= w ) owner[s] = -1;
+    const int i = t.walk[w];
+    if( last[i] < 0 ) continue;
+    int s = 0; while( owner[s] >= 0 ) s++;
+    owner[s] = i; t.link[i].keep = s; if( s + 1 > t.nkeep ) t.nkeep = s + 1;
+  }
+  return true;
+}
+
 }  // namespace rkfd

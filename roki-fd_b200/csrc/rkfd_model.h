@@ -79,5 +79,11 @@ bool build_model(const WorldHost &w, ModelDev &out, std::string &err);
  * memory), the column keeps the rest.  Rewrites slot/sc/wslot/branch/accum/wext/frame slots, rk_slot, nscratch, ntspace. */
 void model_layout(ModelDev &m, bool tm);
 
+/* Table of the kinematics pass (rkfd_kin.cuh) for output columns links[0..nlink) (link indices of the model; null: all links,
+ * then nlink must be m.nl): the links to visit (the requested ones and their ancestors, parents first), the output columns of
+ * each, and the keep slots of frames that a later child needs.  Returns false and fills `err` for a list it refuses
+ * (nlink < 0 or > MAX_LINKS, an index out of range). */
+bool kin_table(const ModelDev &m, int nlink, const int *links, KinDev &t, std::string &err);
+
 }  // namespace rkfd
 #endif

@@ -126,6 +126,28 @@ struct ModelDev {
   double vert[3 * MAX_VERTS];
 };
 
+/* Link table of the kinematics pass (rkfd_kin.cuh, rkFDBatchGetLinkFrames).  It is a __grid_constant__ kernel parameter, not
+ * the __constant__ bank of the step kernels (engines share those banks, g_model_owner), and holds what the walk needs: the
+ * joint model of every link and which links to visit and report.  ~4.5 KB at MAX_LINKS: within the 32 KB parameter limit. */
+struct KinLinkDev {
+  double Ro[9], po[3];  /* org frame w.r.t. the parent (LinkDev::Ro, po) */
+  double sg;            /* sign of the quarter turn (cls RO_RXP / RO_RXM) */
+  int cls, pz, parent, jtype, qofs;
+  int keep;             /* >= 0: shared-memory slot where the walk keeps this link's frame for a later child that is not the next
+                           link visited; -1: the next visited link continues from registers or nothing needs it */
+  unsigned omask;       /* bit k: output column k reports this link (duplicates in the list set several bits) */
+  int pad_;
+};
+struct KinDev {
+  int nwalk;            /* links visited: the requested links and their ancestors, parents first */
+  int nsel;             /* output columns (requested links, duplicates included) */
+  int nkeep;            /* shared-memory slots of kept frames (KIN_KEEP doubles each) */
+  int brk;              /* the world has breakable-float joints: the kernel reads piv_type */
+  int walk[MAX_LINKS];
+  KinLinkDev link[MAX_LINKS];   /* indexed by the model's link index */
+};
+constexpr int KIN_KEEP = 18;    /* Rw (9), pw (3), linear and angular velocity in link axes (3 + 3) */
+
 /* Per-environment state in HBM, structure-of-arrays with the environment index fastest:
  * element (k, e) of an array lives at base[k*ld + e].  Thread e of a warp therefore reads
  * consecutive 8-byte words: every load/store is one fully coalesced 256-byte request. */
