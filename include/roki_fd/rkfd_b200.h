@@ -387,6 +387,12 @@ __ROKI_FD_EXPORT long long rkFDBatchResetKernelCount(rkFD *fd);       /* gather,
 __ROKI_FD_EXPORT int rkFDBatchGetLinkFrames(rkFD *fd, int nlink, const int *links, double *frame, double *vel);
 __ROKI_FD_EXPORT int rkFDBatchGetLinkFramesDevice(rkFD *fd, int shard, int nlink, const int *links, double *frame, double *vel);
 __ROKI_FD_EXPORT long long rkFDBatchLinkFrameKernelCount(rkFD *fd);   /* kinematics launches of the calls so far */
+/* The compiled step-kernel variant that shard `shard` launches, as chosen by rkFDUpdateInit from the model and the tuning
+ * variables RKFD_SPEC, RKFD_FORCE_BLOCK, RKFD_FORCE_MINB, RKFD_FORCE_GSCR and RKFD_FORCE_SMEM: v[0] threads per block, v[1] 1
+ * when the scratch column lives in device memory (0: shared memory), v[2] 1 for the rigid-contact kernels, v[3] the model
+ * specialisation id (0: the generic table-driven kernel), v[4] the minimum resident blocks per SM it was compiled for.
+ * Needs rkFDUpdateInit; a bad shard index is refused. */
+__ROKI_FD_EXPORT int rkFDBatchKernelVariant(rkFD *fd, int shard, int v[5]);
 /* the flattened model of the last rkFDUpdateInit as text (host side; also after an rkFDUpdateInit that found no device):
  * returns the length needed */
 __ROKI_FD_EXPORT int rkFDB200DescribeModel(rkFD *fd, char *buf, int cap);

@@ -85,7 +85,7 @@ def lib():
         "rkFDBatchResetEnvs": (ci, [vp, ci, vp, vp, vp, vp]), "rkFDBatchResetEnvsDevice": (ci, [vp, ci, ci, vp, vp, vp, vp]),
         "rkFDBatchResetKernelCount": (C.c_longlong, [vp]),
         "rkFDBatchGetLinkFrames": (ci, [vp, ci, vp, vp, vp]), "rkFDBatchGetLinkFramesDevice": (ci, [vp, ci, ci, vp, vp, vp]),
-        "rkFDBatchLinkFrameKernelCount": (C.c_longlong, [vp]),
+        "rkFDBatchLinkFrameKernelCount": (C.c_longlong, [vp]), "rkFDBatchKernelVariant": (ci, [vp, ci, _ip]),
         "rkFDB200DescribeModel": (ci, [vp, C.c_char_p, ci]), "rkFDBatchLastError": (C.c_char_p, []), "rkFDBatchDeviceCount": (ci, []), "rkFDB200MeasureFp64": (ci, [_dp]),
     }
     for name, (res, args) in sig.items():
@@ -487,6 +487,12 @@ class RkFD:
     @property
     def link_frame_kernel_count(self):
         return lib().rkFDBatchLinkFrameKernelCount(self.h)
+
+    def kernel_variant(self, shard=0):
+        """rkFDBatchKernelVariant: (block, gscr, rigid, spec, minb) of the step-kernel variant shard `shard` launches."""
+        v = (C.c_int * 5)()
+        self._ck(lib().rkFDBatchKernelVariant(self.h, shard, v))
+        return tuple(v)
 
 
 def create_world(world: World, B=None, devices=None):

@@ -594,6 +594,13 @@ extern "C" int rkFDBatchGetLinkFramesDevice(rkFD *fd, int shard, int nlink, cons
   TRY(fi->engine->link_frames(shard, t, frame, vel));
 }
 extern "C" long long rkFDBatchLinkFrameKernelCount(rkFD *fd){ FDImpl *fi = FI(fd); return ( fi && fi->engine ) ? fi->engine->link_frame_kernels() : 0; }
+/* the step-kernel variant a shard launches (Engine::Engine's choice from the model and the RKFD_* tuning variables) */
+extern "C" int rkFDBatchKernelVariant(rkFD *fd, int shard, int v[5])
+{
+  BATCH_GUARD(fd); NEED_ENGINE();
+  if( !v ) return fail("rkFDBatchKernelVariant: v is needed");
+  TRY(fi->engine->kernel_variant(shard, v));
+}
 extern "C" const char *rkFDBatchLastError(void){ return g_err.c_str(); }
 extern "C" int rkFDBatchDeviceCount(void){ return device_count(); }
 extern "C" int rkFDB200MeasureFp64(double *tflops){ try { *tflops = measure_fp64_tflops(); } catch(const std::exception &ex){ return fail(ex.what()); } return 0; }

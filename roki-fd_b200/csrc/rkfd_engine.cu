@@ -737,6 +737,12 @@ void Engine::slot_map(int si, int *perm)
   CK(cudaSetDevice(prev));
 }
 long long Engine::resorts() const { long long n = 0; for(const Shard *s : shards_) n += s->sorts; return n; }
+void Engine::kernel_variant(int si, int v[5]) const
+{
+  if( si < 0 || si >= (int)shards_.size() ) throw std::runtime_error("rokifd_b200: kernel variant: shard index out of range");
+  const KernelVariant *kv = shards_[si]->kv;
+  v[0] = kv->block; v[1] = kv->gscr; v[2] = kv->rigid; v[3] = kv->spec; v[4] = kv->minb;
+}
 void *Engine::device_ptr(int si, int which, int *ld, int *B)
 {
   if( si < 0 || si >= (int)shards_.size() ) return nullptr;

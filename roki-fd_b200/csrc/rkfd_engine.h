@@ -80,6 +80,9 @@ class Engine {
   void link_frames_host(const KinDev &t, double *frame, double *vel);
   long long link_frame_kernels() const { return kin_kernels_; }     /* kinematics launches (one per shard and call) */
 
+  /* the step-kernel variant shard `shard` launches: v = (block, gscr, rigid, spec, minb); throws on a bad shard index */
+  void kernel_variant(int shard, int v[5]) const;
+
  private:
   void upload_model(Shard &s);
   void launch(Shard &s, const StateDev &st, int cur, int mode, int nsteps);

@@ -111,11 +111,14 @@ int hostsim_finalize(HostSim *h, int B)
 const char *hostsim_error(HostSim *h){ return h->err.c_str(); }
 int hostsim_nq(HostSim *h){ return h->model.nq; }
 int hostsim_nl(HostSim *h){ return h->model.nl; }
-/* model specialisation the kernel would pick (0: generic); hostsim_use_spec makes hostsim_run use it */
+/* model specialisation the kernel would pick (0: generic); hostsim_use_spec makes hostsim_run use it and returns the id
+ * it took (0 when the model does not match `id`) */
 int hostsim_spec_match(HostSim *h, int tm){ return tm == 2 ? spec_match_rolled(h->model) : spec_match(h->model, tm); }   /* 2: rolled */
-void hostsim_use_spec(HostSim *h, int id){
-  if( id == SPEC_GENERIC_TM ){ h->spec = h->model.has_rigid ? 0 : id; return; }
-  h->spec = ( id > 0 && (spec_match_mask(h->model) >> id & 1u) ) ? id : 0; }
+unsigned hostsim_spec_mask(HostSim *h){ return spec_match_mask(h->model); }
+int hostsim_use_spec(HostSim *h, int id){
+  if( id == SPEC_GENERIC_TM ) h->spec = h->model.has_rigid ? 0 : id;
+  else h->spec = ( id > 0 && (spec_match_mask(h->model) >> id & 1u) ) ? id : 0;
+  return h->spec; }
 int hostsim_nslot(HostSim *h){ return h->model.nslot; }
 int hostsim_nscratch(HostSim *h){ return h->model.nscratch; }
 void hostsim_free(HostSim *h){ for(void *p : h->allocs) std::free(p); for(auto *c : h->chains) delete c; delete h; }

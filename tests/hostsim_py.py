@@ -36,6 +36,8 @@ def lib():
         L.hostsim_error.argtypes = [C.c_void_p]
         L.hostsim_use_spec.argtypes = [C.c_void_p, C.c_int]
         L.hostsim_spec_match.argtypes = [C.c_void_p, C.c_int]
+        L.hostsim_spec_mask.restype = C.c_uint
+        L.hostsim_spec_mask.argtypes = [C.c_void_p]
         for f in ("hostsim_nq", "hostsim_nl", "hostsim_nslot", "hostsim_nscratch", "hostsim_free"):
             getattr(L, f).argtypes = [C.c_void_p]
         L.hostsim_set_state.argtypes = [C.c_void_p, _dp, _dp, _dp]
@@ -90,10 +92,12 @@ class HostSim:
         self.nscratch = L.hostsim_nscratch(self.h)
         # model specialisations the kernel could pick (0: generic): scratch in shared memory / in tensor memory
         self.spec, self.spec_tm, self.spec_rolled = (L.hostsim_spec_match(self.h, k) for k in (0, 1, 2))
-        if spec:                                   # "smem" | "tmem" | "rolled": run that specialisation's code path
-            sid = {"smem": self.spec, "tmem": self.spec_tm, "rolled": self.spec_rolled, "generic_tm": 11}[spec]
+        self.spec_mask = L.hostsim_spec_mask(self.h)    # bit id: every specialisation the model is eligible for
+        if spec:      # "smem" | "tmem" | "rolled" | "generic_tm", or a specialisation id: run that specialisation's code path
+            sid = spec if isinstance(spec, int) else {"smem": self.spec, "tmem": self.spec_tm, "rolled": self.spec_rolled, "generic_tm": 11}[spec]
             assert sid > 0, "model matches no compiled specialisation"
-            L.hostsim_use_spec(self.h, sid)
+            used = L.hostsim_use_spec(self.h, sid)
+            assert used == sid, "model does not match specialisation %d" % sid
 
     def __del__(self):
         if getattr(self, "h", None):

@@ -398,13 +398,15 @@ def test_kernel_variants_agree(capi, oracle, monkeypatch, variant):
         for k, v in env.items():
             monkeypatch.setenv(k, str(v))
         fd = gpu_world(capi, w, q, qd, u)
+        kv = fd.kernel_variant()
         fd.update_n(25)
-        out = fd.batch_get_state(), fd.batch_get_contact(), fd.batch_get_status()
+        out = fd.batch_get_state(), fd.batch_get_contact(), fd.batch_get_status(), kv
         fd.destroy()
         return out
 
-    (gq, gqd, gqdd), (ga, gt, gr, gf), status = run({"RKFD_SPEC": spec, "RKFD_FORCE_BLOCK": block, "RKFD_FORCE_MINB": minb})
-    (rq, rqd, rqdd), (ra, rt, rr, rf), _ = run({"RKFD_SPEC": 0})
+    (gq, gqd, gqdd), (ga, gt, gr, gf), status, kv = run({"RKFD_SPEC": spec, "RKFD_FORCE_BLOCK": block, "RKFD_FORCE_MINB": minb})
+    (rq, rqd, rqdd), (ra, rt, rr, rf), _, rkv = run({"RKFD_SPEC": 0})
+    assert kv == (block, 0, 0, spec, minb) and rkv[3] == 0 and (spec == 0 or rkv != kv)       # the engine runs what was forced
     assert (status == 0).all()
     assert relerr(gq, rq) < 1e-11 and relerr(gqd, rqd) < 1e-10 and relerr(gqdd, rqdd) < 1e-8
     assert (ga == ra).mean() > 0.9999 and ga.sum() > 0
@@ -431,16 +433,19 @@ def test_rigid_mlcp_kernel_variants_agree(capi, oracle, monkeypatch, variant):
             monkeypatch.setenv(k, str(v))
         fd = gpu_world(capi, w, q, qd, u)
         first = fd.batch_get_state()[2].copy(), fd.batch_get_contact()
+        kv = fd.kernel_variant()
         fd.update_n(nsteps)
-        out = first, fd.batch_get_state()
+        out = first, fd.batch_get_state(), kv
         fd.destroy()
         return out
 
     env = {"RKFD_SPEC": spec, "RKFD_FORCE_BLOCK": block, "RKFD_FORCE_MINB": minb}
     if smem:
         env["RKFD_FORCE_SMEM"] = 1
-    (a1, c1), (q1, qd1, _) = run(env, 8)
-    (a0, c0), (q0, qd0, _) = run({"RKFD_SPEC": 0}, 8)
+    (a1, c1), (q1, qd1, _), kv = run(env, 8)
+    (a0, c0), (q0, qd0, _), rkv = run({"RKFD_SPEC": 0}, 8)
+    # the rolled rigid kernel keeps its scratch column in device memory unless RKFD_FORCE_SMEM
+    assert kv == (block, int(spec == 7 and not smem), 1, spec, minb) and rkv[2:4] == (1, 0) and (spec == 0 or rkv != kv)
     assert c0[0].sum() > 1000 and (c0[0] == c1[0]).all()
     assert relerr(a1, a0) < 1e-9
     fin = np.isfinite(q0).all(1) & (np.abs(q0).max(1) < 1e3)      # envs that start deep inside the floor blow up
@@ -487,6 +492,7 @@ def test_divergent_slow_paths_keep_tensor_memory_accesses_converged(capi, monkey
     for spec in (0, 5, 3):
         monkeypatch.setenv("RKFD_SPEC", str(spec))
         fd = gpu_world(capi, w, q, qd, u)
+        assert fd.kernel_variant()[3] == spec
         fd.update_n(3)
         out.append(fd.batch_get_state())
         fd.destroy()
@@ -508,6 +514,7 @@ def test_generic_kernel_with_tensor_memory_scratch(capi, monkeypatch, name):
     for spec in (0, 11):
         monkeypatch.setenv("RKFD_SPEC", str(spec))
         fd = gpu_world(capi, w, q, qd, u)
+        assert fd.kernel_variant()[3] == spec
         fd.update_n(12)
         out.append(fd.batch_get_state())
         fd.destroy()
@@ -529,6 +536,7 @@ def test_general_frame_arm_specialisations(capi, oracle, monkeypatch, nlinks, sp
     for sid in (0, spec):
         monkeypatch.setenv("RKFD_SPEC", str(sid))
         fd = gpu_world(capi, w, q, qd, u)
+        assert fd.kernel_variant()[3] == sid
         fd.update_n(15)
         out.append(fd.batch_get_state())
         fd.destroy()
