@@ -387,6 +387,29 @@ __ROKI_FD_EXPORT long long rkFDBatchResetKernelCount(rkFD *fd);       /* gather,
 __ROKI_FD_EXPORT int rkFDBatchGetLinkFrames(rkFD *fd, int nlink, const int *links, double *frame, double *vel);
 __ROKI_FD_EXPORT int rkFDBatchGetLinkFramesDevice(rkFD *fd, int shard, int nlink, const int *links, double *frame, double *vel);
 __ROKI_FD_EXPORT long long rkFDBatchLinkFrameKernelCount(rkFD *fd);   /* kinematics launches of the calls so far */
+/* External wrenches: a force and a torque applied to links of every environment, for pushes, disturbances, tethers, drag or
+ * forces from another model.  The reference has no such input (it clears every link's wrench list at each evaluation).
+ * rkFDBatchSetExtWrenchLinks declares which links take one, before rkFDUpdateInit: links[0..n) are link indices in
+ * [0, rkFDBatchLinkNum), in the order of the motor input, without duplicates, 0 <= n <= 32; n = 0 clears the declaration.  A
+ * refused call (after rkFDUpdateInit, an index out of range, a duplicate, n out of range) changes nothing.  A new declaration
+ * drops a wrench held as pending.  Without a declaration nothing of the model, of the kernel choice or of the step changes.
+ * A declared world runs the generic kernels: the serial-arm specialisations take no external wrench.
+ * rkFDBatchSetExtWrench: host memory, env-major w[B][n][6] = (force, torque) of declared link k in row k.  The force acts at the
+ * link's centre of mass and the torque is about the centre of mass, both in world axes.  A push f at another world point p
+ * adds (p - c) x f to the torque, c being the world position of the centre of mass.  Before rkFDUpdateInit the wrench is held
+ * as pending, so the committing evaluation at t = 0 sees it; afterwards it is synchronous, like rkFDBatchSetMotorInput.
+ * rkFDBatchSetExtWrenchDevice: a device buffer [Bs][n][6] on the device of shard `shard`, indexed by the environment local to the
+ * shard (the engine maps it to its re-sorted slot); stream-ordered on the engine's stream, without a host synchronisation or an
+ * allocation.  It needs rkFDUpdateInit.
+ * Like the motor input, the wrench is an input held until it is changed; it is zero until set.  It is constant over the
+ * evaluations of a step (the stage evaluations and the committing one) and enters rkFDBatchEval as well.  It enters every
+ * contact solver (penalty, MLCP, Vert, Volume), through the bias of the articulated-body pass, and the transmitted-wrench test of
+ * breakable-float joints.  rkFDBatchResetEnvs* keeps it: a reset environment restarts as a new simulator given its current
+ * wrench before rkFDUpdateInit.  A non-finite wrench ends up in the status word (bit 0) like any other non-finite acceleration.
+ * Both setters need a declaration. */
+__ROKI_FD_EXPORT int rkFDBatchSetExtWrenchLinks(rkFD *fd, int n, const int *links);
+__ROKI_FD_EXPORT int rkFDBatchSetExtWrench(rkFD *fd, const double *w);
+__ROKI_FD_EXPORT int rkFDBatchSetExtWrenchDevice(rkFD *fd, int shard, const double *w);
 /* The compiled step-kernel variant that shard `shard` launches, as chosen by rkFDUpdateInit from the model and the tuning
  * variables RKFD_SPEC, RKFD_FORCE_BLOCK, RKFD_FORCE_MINB, RKFD_FORCE_GSCR and RKFD_FORCE_SMEM: v[0] threads per block, v[1] 1
  * when the scratch column lives in device memory (0: shared memory), v[2] 1 for the rigid-contact kernels, v[3] the model

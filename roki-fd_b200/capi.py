@@ -86,6 +86,7 @@ def lib():
         "rkFDBatchResetKernelCount": (C.c_longlong, [vp]),
         "rkFDBatchGetLinkFrames": (ci, [vp, ci, vp, vp, vp]), "rkFDBatchGetLinkFramesDevice": (ci, [vp, ci, ci, vp, vp, vp]),
         "rkFDBatchLinkFrameKernelCount": (C.c_longlong, [vp]), "rkFDBatchKernelVariant": (ci, [vp, ci, _ip]),
+        "rkFDBatchSetExtWrenchLinks": (ci, [vp, ci, vp]), "rkFDBatchSetExtWrench": (ci, [vp, vp]), "rkFDBatchSetExtWrenchDevice": (ci, [vp, ci, vp]),
         "rkFDB200DescribeModel": (ci, [vp, C.c_char_p, ci]), "rkFDBatchLastError": (C.c_char_p, []), "rkFDBatchDeviceCount": (ci, []), "rkFDB200MeasureFp64": (ci, [_dp]),
     }
     for name, (res, args) in sig.items():
@@ -487,6 +488,24 @@ class RkFD:
     @property
     def link_frame_kernel_count(self):
         return lib().rkFDBatchLinkFrameKernelCount(self.h)
+
+    def batch_set_ext_wrench_links(self, links):
+        """rkFDBatchSetExtWrenchLinks (before update_init): the links (indices in flat_links() order) that take an external
+        wrench, in the order of its rows; an empty list clears the declaration."""
+        pl = np.ascontiguousarray(links, np.int32).reshape(-1)
+        self._ck(lib().rkFDBatchSetExtWrenchLinks(self.h, pl.shape[0], _ptr(pl)))
+
+    def batch_set_ext_wrench(self, w):
+        """rkFDBatchSetExtWrench: (B, n, 6) float64 host array, (force, torque about the centre of mass) in world axes per declared
+        link; held as pending before update_init."""
+        if isinstance(w, np.ndarray):
+            w = np.ascontiguousarray(w, np.float64)
+        self._ck(lib().rkFDBatchSetExtWrench(self.h, _ptr(w)))
+
+    def batch_set_ext_wrench_device(self, shard, w_ptr):
+        """rkFDBatchSetExtWrenchDevice: raw device address (e.g. torch CUDA tensor .data_ptr()) of float64 w[Bs][n][6] of shard
+        `shard`, indexed by the shard's local environment; stream-ordered on the engine's stream."""
+        self._ck(lib().rkFDBatchSetExtWrenchDevice(self.h, shard, _ptr(w_ptr)))
 
     def kernel_variant(self, shard=0):
         """rkFDBatchKernelVariant: (block, gscr, rigid, spec, minb) of the step-kernel variant shard `shard` launches."""

@@ -48,6 +48,8 @@ struct FDImpl {
   Engine *engine = nullptr;
   ModelDev model;
   std::vector<double> pend_q, pend_qd, pend_u;   /* batched initial state given before rkFDUpdateInit */
+  std::vector<int> fext_links;                   /* links declared for an external wrench (rkFDBatchSetExtWrenchLinks) */
+  std::vector<double> pend_w;                    /* external wrench given before rkFDUpdateInit */
   bool warned = false;
 };
 
@@ -422,6 +424,7 @@ extern "C" void rkFDUpdateInit(rkFD *fd)
     if( fd->ode.form != RKFD_ODE2_Regular || fd->ode.integrator < RKFD_ODE_RKG || fd->ode.integrator > RKFD_ODE_Heun )
       throw std::runtime_error("integrators: Regular form with RKG, RK4, Euler or Heun");
     w.integrator = fd->ode.integrator;
+    w.fext_links = fi->fext_links;
     std::string err;
     if( !build_model(w, fi->model, err) ) throw std::runtime_error(err);
     /* static chains carry no joint state, so the device rows are the host offsets of relayout() */
@@ -438,6 +441,7 @@ extern "C" void rkFDUpdateInit(rkFD *fd)
       for(int e=0;e<B;e++) for(size_t k=0;k<ci->links.size();k++) u[(size_t)e*nl + ci->link_base + k] = ci->motor_in[k]; }
     if( n > 0 ) fi->engine->set_state(q.data(), qd.data());
     if( nl > 0 ) fi->engine->set_motor_input(u.data());
+    if( fi->model.nfext > 0 && fi->pend_w.size() == (size_t)B*6*fi->model.nfext ) fi->engine->set_ext_wrench(fi->pend_w.data());
     fi->engine->eval(true);            /* the committing evaluation at t=0 (reference rkfd_sim.c:556) */
     if( !fi->batch ){ fi->engine->sync(); mirror_env0(fd); }
   } catch(const std::exception &ex){ complain("rkFDUpdateInit", ex.what()); destroy_engine(fi); }
@@ -594,6 +598,41 @@ extern "C" int rkFDBatchGetLinkFramesDevice(rkFD *fd, int shard, int nlink, cons
   TRY(fi->engine->link_frames(shard, t, frame, vel));
 }
 extern "C" long long rkFDBatchLinkFrameKernelCount(rkFD *fd){ FDImpl *fi = FI(fd); return ( fi && fi->engine ) ? fi->engine->link_frame_kernels() : 0; }
+/* external wrenches on declared links (Engine::set_ext_wrench): an input held like the motor input */
+extern "C" int rkFDBatchSetExtWrenchLinks(rkFD *fd, int n, const int *links)
+{
+  BATCH_GUARD(fd);
+  if( fi->engine ) return fail("rkFDBatchSetExtWrenchLinks: declare the links before rkFDUpdateInit");
+  if( n < 0 || n > MAX_LINKS ) return fail("rkFDBatchSetExtWrenchLinks: n must be in [0, " + std::to_string(MAX_LINKS) + "]");
+  if( n > 0 && !links ) return fail("rkFDBatchSetExtWrenchLinks: links is needed");
+  const int nl = rkFDBatchLinkNum(fd);
+  std::vector<char> seen(nl > 0 ? nl : 1, 0);
+  for(int k=0;k<n;k++){
+    const int i = links[k];
+    if( i < 0 || i >= nl ) return fail("rkFDBatchSetExtWrenchLinks: link " + std::to_string(i) + " out of range [0, " + std::to_string(nl) + ")");
+    if( seen[i] ) return fail("rkFDBatchSetExtWrenchLinks: link " + std::to_string(i) + " listed twice");
+    seen[i] = 1;
+  }
+  fi->fext_links.assign(links, links + n);
+  fi->pend_w.clear();                 /* a wrench held for an earlier declaration has another row count */
+  return 0;
+}
+extern "C" int rkFDBatchSetExtWrench(rkFD *fd, const double *w)
+{
+  BATCH_GUARD(fd);
+  if( fi->fext_links.empty() ) return fail("rkFDBatchSetExtWrench: no link is declared (rkFDBatchSetExtWrenchLinks)");
+  if( !w ) return fail("rkFDBatchSetExtWrench: w is needed");
+  if( !fi->engine ){ fi->pend_w.assign(w, w + (size_t)fi->B*6*fi->fext_links.size()); return 0; }
+  TRY(fi->engine->set_ext_wrench(w));
+}
+extern "C" int rkFDBatchSetExtWrenchDevice(rkFD *fd, int shard, const double *w)
+{
+  BATCH_GUARD(fd); NEED_ENGINE();
+  if( fi->engine->model().nfext <= 0 ) return fail("rkFDBatchSetExtWrenchDevice: no link is declared (rkFDBatchSetExtWrenchLinks)");
+  if( shard < 0 || shard >= fi->engine->num_shards() ) return fail("rkFDBatchSetExtWrenchDevice: shard index out of range");
+  if( !w ) return fail("rkFDBatchSetExtWrenchDevice: w is needed");
+  TRY(fi->engine->set_ext_wrench_device(shard, w));
+}
 /* the step-kernel variant a shard launches (Engine::Engine's choice from the model and the RKFD_* tuning variables) */
 extern "C" int rkFDBatchKernelVariant(rkFD *fd, int shard, int v[5])
 {
@@ -632,7 +671,9 @@ extern "C" int rkFDB200DescribeModel(rkFD *fd, char *buf, int cap)
   for(int i=0;i<m.nslide;i++){ const SlideDev &d = m.slide[i]; double v[16] = { d.vel, d.axis[0], d.axis[1], d.axis[2] };
     for(int k=0;k<9;k++) v[4+k] = d.lR[k]; for(int k=0;k<3;k++) v[13+k] = d.lp[k]; arr("slide", i, v, 16); }
   for(int i=0;i<m.npair;i++) if( m.pair[i].slinfo & 0xffff ){ const int si = m.pair[i].slinfo; const double v[3] = { (double)(si & 255), (double)((si >> 8) & 255), (double)((si >> 16) & 1) }; arr("pair.slide", i, v, 3); }
-  if( fd->dis && fd->size > 0 ) arr("init.q", 0, fd->dis->buf, fd->size);      /* the registered initial displacements ([roki::chain::init]) */
+  /* links declared for an external wrench, in the order of its rows (rkFDBatchSetExtWrenchLinks) */
+  if( m.nfext > 0 ){ double v[MAX_LINKS]; for(int i=0;i<m.nl;i++) if( m.link[i].fext_row >= 0 ) v[m.link[i].fext_row] = i; arr("ext.links", 0, v, m.nfext); }
+  if( fd->dis && fd->size > 0 ) arr("init.q", 0, fd->dis->buf, fd->size);     /* the registered initial displacements ([roki::chain::init]) */
   if( buf && cap > 0 ){ std::snprintf(buf, cap, "%s", s.c_str()); }
   return (int)s.size();
 }

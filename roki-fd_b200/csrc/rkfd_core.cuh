@@ -164,6 +164,7 @@ struct SpecGeneric {
   static RKFD_HD int accum_slot(int, const LinkDev &L){ return L.accum_slot; }
   static RKFD_HD int wext_slot(int, const LinkDev &L){ return L.wext_slot; }
   static RKFD_HD int frame_slot(int, const LinkDev &L){ return L.frame_slot; }
+  static RKFD_HD int fext_row(int, const LinkDev &L){ return L.fext_row; }
   static RKFD_HD int rk_slot(const ModelDev &m){ return m.rk_slot; }
   static RKFD_HD int nq(const ModelDev &m){ return m.nq; }
   /* 1-DoF joints: slots of (sin, cos, 1/D, u) in the "T space" (Ctx::TL/TS) - the scratch column itself here */
@@ -202,6 +203,7 @@ struct SpecSerialRev {
   static RKFD_HD int accum_slot(int, const LinkDev &){ return -1; }
   static RKFD_HD int wext_slot(int i, const LinkDev &L){ return ( i == NL_-1 && L.cell_end > L.cell_begin ) ? WEXT : -1; }
   static RKFD_HD int frame_slot(int, const LinkDev &){ return -1; }
+  static constexpr RKFD_HD int fext_row(int, const LinkDev &){ return -1; }     /* external wrenches: generic kernels only */
   static RKFD_HD int rk_slot(const ModelDev &){ return RK; }
   static RKFD_HD int nq(const ModelDev &){ return NL_ - 1; }
 };
@@ -238,12 +240,13 @@ struct SpecSerialRevRolled {
   static RKFD_HD int accum_slot(int, const LinkDev &){ return -1; }
   static RKFD_HD int wext_slot(int i, const LinkDev &L){ return ( i == NL_-1 && L.cell_end > L.cell_begin ) ? WEXT : -1; }
   static RKFD_HD int frame_slot(int i, const LinkDev &L){ return ( RG_ && i == NL_-1 && L.cell_end > L.cell_begin ) ? FRAME : -1; }
+  static constexpr RKFD_HD int fext_row(int, const LinkDev &){ return -1; }     /* external wrenches: generic kernels only */
   static RKFD_HD int rk_slot(const ModelDev &){ return RK; }
   static RKFD_HD int nq(const ModelDev &){ return NL_ - 1; }
   static RKFD_HD int sc(int i, const LinkDev &){ return RG_ ? PER*i + 9 : 4*(i-1); }
 };
 inline bool spec_serial_rev_rolled_match(const ModelDev &m, int NL, int RG = 0, int GEN = 0){
-  if( m.nfw > 1 || m.npair > m.npair_static || m.nslide > 0 ) return false;       /* slide mode: generic kernel only */
+  if( m.nfw > 1 || m.npair > m.npair_static || m.nslide > 0 || m.nfext > 0 ) return false;   /* slide mode, external wrenches: generic kernel only */
   if( RG ? !( m.has_rigid && m.nrg == 1 && m.rigid_link == NL-1 ) : m.has_rigid ) return false;
   if( m.nl != NL || NL < 2 ) return false;
   for(int i=0;i<NL;i++){
@@ -258,7 +261,7 @@ inline bool spec_serial_rev_rolled_match(const ModelDev &m, int NL, int RG = 0, 
 
 /* does the flattened model have the shape SpecSerialRev<.,NL,CLS> assumes? (host side) */
 inline bool spec_serial_rev_match(const ModelDev &m, int NL, unsigned CLS){
-  if( m.has_rigid || m.nl != NL || NL < 2 || m.nfw > 1 || m.npair > m.npair_static || m.nslide > 0 ) return false;
+  if( m.has_rigid || m.nl != NL || NL < 2 || m.nfw > 1 || m.npair > m.npair_static || m.nslide > 0 || m.nfext > 0 ) return false;
   for(int i=0;i<NL;i++){
     const LinkDev &L = m.link[i];
     if( i == 0 ){ if( L.parent >= 0 || L.jtype != J_FIXED || L.cell_end > L.cell_begin ) return false; continue; }
@@ -808,9 +811,19 @@ struct Core {
     k.om = om_n;
     st3(Spec::wslot(i,L), k.om);
     if( !gacc ){ k.gd = xf_tmul(x, k.gd); st3(Spec::wslot(i,L)+3, k.gd); }
-    const int wx = Spec::wext_slot(i,L), fs = Spec::frame_slot(i,L), bs = Spec::branch_slot(i,L);
+    const int wx = Spec::wext_slot(i,L), fs = Spec::frame_slot(i,L), bs = Spec::branch_slot(i,L), fr = Spec::fext_row(i,L);
     if( cont && wx >= 0 ){
-      const V6 w = contacts(m, L, k.Rw, k.pw, k.vl, k.om, ref);
+      /* contacts() holds warp votes: a link that only takes an external wrench does not enter it (fr is a compile-time -1 in the
+       * specialisations, where this stays the unconditional call) */
+      V6 w; w.l = v3(0,0,0); w.a = v3(0,0,0);
+      if( fr < 0 || L.cell_end > L.cell_begin ) w = contacts(m, L, k.Rw, k.pw, k.vl, k.om, ref);
+      if( fr >= 0 ){
+        /* external wrench (force at the centre of mass, torque about it, world axes) -> link axes, about the link origin */
+        const V3 f = v3(c.gld(c.st.fext, 6*fr), c.gld(c.st.fext, 6*fr+1), c.gld(c.st.fext, 6*fr+2));
+        const V3 n = v3(c.gld(c.st.fext, 6*fr+3), c.gld(c.st.fext, 6*fr+4), c.gld(c.st.fext, 6*fr+5));
+        const V3 fl = tmul(k.Rw, f);
+        w.l = w.l + fl; w.a = w.a + ( tmul(k.Rw, n) + cross(v3(L.com[0], L.com[1], L.com[2]), fl) );
+      }
       st3(wx, w.l); st3(wx+3, w.a);
       if( fs >= 0 ){ stm(fs, k.Rw); st3(fs+9, k.pw); st3(fs+12, k.vl); st3(fs+15, k.om); }
     }

@@ -71,6 +71,14 @@ class Engine {
   void reset_envs_host(int n, const int *envs, const double *q, const double *qd, const double *u);
   long long reset_kernels() const { return reset_kernels_; }        /* gather, zero fill and scatter launches of the resets */
 
+  /* external wrench of the declared links (ModelDev::nfext), env-major [B][nfext][6]: (force, torque about the centre of mass),
+   * world axes.  set_ext_wrench: host array, global environment index, every shard; synchronous.  set_ext_wrench_device: a
+   * device buffer [Bs][nfext][6] of shard `shard`, indexed by the environment local to the shard, read through the slot
+   * permutation by the transposing scatter; stream-ordered on the shard's stream, no allocation.  Both throw without a
+   * declared link */
+  void set_ext_wrench(const double *w);
+  void set_ext_wrench_device(int shard, const double *w);
+
   /* link kinematics (rkfd_kin.cuh): world frames [B][nsel][12] (R row-major, p) and velocities [B][nsel][6] (linear, angular;
    * world axes) of the output columns of table `t`, from the committed state; a null output is neither computed nor written.
    * Nothing of the engine's state is written.  link_frames: device buffers of shard `shard`, indexed by the environment local

@@ -39,8 +39,9 @@ void model_layout(ModelDev &m, bool tm)
       LinkDev &p = m.link[d.parent];
       if( p.branch_slot < 0 ){ p.branch_slot = slot; slot += BRANCH_SLOTS; p.accum_slot = slot; slot += ACCUM_SLOTS; }
     }
-    if( d.cell_end > d.cell_begin || d.mcol ){ d.wext_slot = slot; slot += WEXT_SLOTS;
-      if( m.has_rigid || d.mcol ){ d.frame_slot = slot; slot += FRAME_SLOTS; } }
+    if( d.cell_end > d.cell_begin || d.mcol || d.fext_row >= 0 ){ d.wext_slot = slot; slot += WEXT_SLOTS;
+      /* a link that only takes an external wrench gets no frame slot: the contact paths read frames of links with cells */
+      if( ( m.has_rigid && d.cell_end > d.cell_begin ) || d.mcol ){ d.frame_slot = slot; slot += FRAME_SLOTS; } }
   }
   if( tm ){ m.rk_slot = t; t += 4*nq; m.ntspace = t; }
   else { m.rk_slot = slot; slot += 4*nq; m.ntspace = 0; }
@@ -130,6 +131,7 @@ bool build_model(const WorldHost &w, ModelDev &m, std::string &err)
       if( nl >= MAX_LINKS ){ err = "too many links (MAX_LINKS)"; return false; }
       if( l.parent >= (int)i ){ err = "link order: parent must precede child"; return false; }
       LinkDev &d = m.link[nl];
+      d.fext_row = -1;
       std::memcpy(d.Ro, l.Ro, sizeof d.Ro); std::memcpy(d.po, l.po, sizeof d.po);
       d.mass = l.mass;
       for(int k=0;k<3;k++){ d.com[k] = l.com[k]; d.mc[k] = l.mass*l.com[k]; }
@@ -247,7 +249,17 @@ bool build_model(const WorldHost &w, ModelDev &m, std::string &err)
   else { int fo = 0; for(int p=0;p<m.npair;p++){ m.pair[p].fofs = fo; fo += (m.cell[m.pair[p].cell].nvert + 31) & ~31; } m.nfw = fo/32; }
   if( m.nfw > MAX_FWORDS ){ err = "too many contact flag words (MAX_FWORDS)"; return false; }
   if( m.nfw < 1 ) m.nfw = 1;
-  m.need_world = m.npair > 0;
+  /* links that take an external wrench (rkFDBatchSetExtWrenchLinks): row k of the input is link fext_links[k].  The wrench
+   * comes in world axes, so such a world propagates the world frames */
+  if( (int)w.fext_links.size() > MAX_LINKS ){ err = "at most " + std::to_string(MAX_LINKS) + " links take an external wrench (MAX_LINKS)"; return false; }
+  for(size_t k=0;k<w.fext_links.size();k++){
+    const int i = w.fext_links[k];
+    if( i < 0 || i >= nl ){ err = "external wrench: link index " + std::to_string(i) + " out of range [0, " + std::to_string(nl) + ")"; return false; }
+    if( m.link[i].fext_row >= 0 ){ err = "external wrench: link " + std::to_string(i) + " listed twice"; return false; }
+    m.link[i].fext_row = (int)k;
+  }
+  m.nfext = (int)w.fext_links.size();
+  m.need_world = m.npair > 0 || m.nfext > 0;
 
   /* ---- topology flags and the scratch slot map */
   for(int i=0;i<nl;i++) if( m.link[i].parent >= 0 ) m.link[m.link[i].parent].nchild++;

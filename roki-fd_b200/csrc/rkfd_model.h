@@ -68,6 +68,7 @@ struct WorldHost {
   ContactInfoHost cidef;
   double dt = 0.001, friction_weight = 100.0;
   int pyramid = 8, max_iter = 10, solver = S_VERT, integrator = 0;
+  std::vector<int> fext_links;              /* links that take an external wrench, in the order of its input rows */
 };
 
 /* Flattens the world into `out`.  Returns false and fills `err` when a limit of the fused kernel is

@@ -48,6 +48,8 @@ struct LinkDev {
   double po[3];        /* org frame position */
   double pol[3];       /* Ro^T po */
   int rcls;            /* RoClass of Ro (rkfd_math.cuh): 0 general, 1 identity, 2/3 quarter turn about x */
+  int fext_row;        /* >=0: row of this link's external wrench in StateDev::fext (rkFDBatchSetExtWrenchLinks), else -1.  It
+                          fills the alignment gap before rsg, so no other entry of the table moves */
   double rsg;          /* +1 for Rx(+90), -1 for Rx(-90), 0 otherwise (sign read at run time by the rolled specialisation) */
   double mass;
   double com[3];
@@ -68,7 +70,7 @@ struct LinkDev {
   int nchild;          /* number of children */
   int branch_slot;     /* >=0: slots where this link publishes frame/velocity/acceleration for non-serial children */
   int accum_slot;      /* >=0: slots where non-serial children accumulate articulated inertia/bias (27) */
-  int wext_slot;       /* >=0: slots of the external wrench (6) (links that carry collision cells) */
+  int wext_slot;       /* >=0: slots of the external wrench (6) (links that carry collision cells or take a wrench, fext_row) */
   int frame_slot;      /* >=0 (worlds with rigid pairs, links with cells): Rw(9) pw(3) vl(3) w(3) a(6) = 24 slots */
   int cell_begin, cell_end;
   double brk_f, brk_t; /* breakable float: force / torque thresholds */
@@ -100,6 +102,7 @@ struct ModelDev {
   int rigid_moving;    /* a rigid pair of two moving links exists: the dense rigid path (A couples the two links / chains) */
   int solver, pyramid, max_iter;
   int integrator;      /* 0 Runge-Kutta-Gill, 1 classical Runge-Kutta, 2 Euler, 3 Heun ([EXT] zODE2AssignRegular) */
+  int nfext;           /* links declared for an external wrench (LinkDev::fext_row); in the alignment gap before rk */
   /* stage coefficients of the integrator times dt, folded on the host (constant-bank operands in the kernel) */
   struct RK { double c21, c31, c32, c42, c43, b1, b2, b3, b4; int ns; } rk;
   int nscratch;        /* scratch slots (doubles) per env */
@@ -151,7 +154,7 @@ constexpr int KIN_KEEP = 18;    /* Rw (9), pw (3), linear and angular velocity i
 /* Per-environment state in HBM, structure-of-arrays with the environment index fastest:
  * element (k, e) of an array lives at base[k*ld + e].  Thread e of a warp therefore reads
  * consecutive 8-byte words: every load/store is one fully coalesced 256-byte request. */
-struct StateDev {
+struct StateDevHead {
   int B;               /* environments on this device */
   int ld;              /* leading dimension (B rounded up to 32) */
   double *q[2], *qd[2];   /* double-buffered committed state [nq][ld] */
@@ -168,6 +171,12 @@ struct StateDev {
   int *status;            /* [ld] per-env status word (bit0: non-finite acceleration) */
   unsigned char *work;    /* [ld] or null: work class of the environment's last rigid solve (Vert / Volume: pairs or contacts and
                            * active-set iterations), 0 = no solve; the engine's re-sort groups equal classes into warps */
+};
+/* The step kernel takes the head as its first parameter and fext as its last one (rkfd_kernel.cuh): its other parameters keep
+ * their places in the parameter space, and kernels that never read fext compile to the code they had without it */
+struct StateDev : StateDevHead {
+  double *fext;           /* [6*nfext][ld] or null: external wrench per declared link, (force, torque about the centre of mass),
+                           * world axes (row 6*LinkDev::fext_row + k) */
 };
 
 }  // namespace rkfd
