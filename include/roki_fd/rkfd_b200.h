@@ -410,6 +410,32 @@ __ROKI_FD_EXPORT long long rkFDBatchLinkFrameKernelCount(rkFD *fd);   /* kinemat
 __ROKI_FD_EXPORT int rkFDBatchSetExtWrenchLinks(rkFD *fd, int n, const int *links);
 __ROKI_FD_EXPORT int rkFDBatchSetExtWrench(rkFD *fd, const double *w);
 __ROKI_FD_EXPORT int rkFDBatchSetExtWrenchDevice(rkFD *fd, int shard, const double *w);
+/* Per-environment mass properties: the mass, centre of mass and inertia of links may differ from environment to environment,
+ * for domain randomisation of payloads and links, system identification (B hypotheses of a payload stepped against one
+ * recording) or robots that carry different tools.  Environment e then steps exactly like a simulator of the world whose
+ * declared links carry environment e's values.
+ * rkFDBatchSetMassPropLinks declares which links take them, before rkFDUpdateInit: links[0..n) are link indices in
+ * [0, rkFDBatchLinkNum), in the order of the motor input, without duplicates, 0 <= n <= 32; n = 0 clears the declaration.  A
+ * refused call (after rkFDUpdateInit, an index out of range, a duplicate, n out of range, links NULL with n > 0) changes
+ * nothing.  A new declaration drops values held as pending.
+ * rkFDBatchSetMassProp: host memory, env-major mp[B][n][10]; row k = (mass, com_x, com_y, com_z, I_xx, I_xy, I_xz, I_yy, I_yz,
+ * I_zz) of declared link k: the centre of mass in the link frame, the inertia about the centre of mass in link axes (the
+ * convention of ZTK mass: / COM: / inertia: and of rkChainB200AddLink).  The whole array is checked before any device work:
+ * every entry finite, every mass > 0, every inertia positive definite; a refused call changes nothing and its message
+ * (rkFDBatchLastError) names the environment and the link.  Before rkFDUpdateInit the values are held as pending, so the
+ * committing evaluation at t = 0 sees them; afterwards the call is synchronous.
+ * rkFDBatchSetMassPropDevice: a device buffer [Bs][n][10] on the device of shard `shard`, indexed by the environment local to
+ * the shard; stream-ordered on the engine's stream, without a host synchronisation or an allocation.  It needs
+ * rkFDUpdateInit.  It checks no value: a non-physical row gives a non-finite acceleration, reported in the status word (bit 0).
+ * Until set, every environment holds the model's own values, so a declaration alone changes no result.  The values are held
+ * until changed and are constant over the evaluations of a step.  They enter every contact solver, rkFDBatchEval and the
+ * transmitted-wrench test of breakable-float joints; an external wrench on a declared link acts at the environment's centre
+ * of mass.  rkFDBatchResetEnvs* keeps them: a reset environment restarts like a new simulator of its own world.  A declared
+ * world runs the generic kernels: the serial-arm specialisations take no per-environment mass properties.  Both setters need a
+ * declaration. */
+__ROKI_FD_EXPORT int rkFDBatchSetMassPropLinks(rkFD *fd, int n, const int *links);
+__ROKI_FD_EXPORT int rkFDBatchSetMassProp(rkFD *fd, const double *mp);
+__ROKI_FD_EXPORT int rkFDBatchSetMassPropDevice(rkFD *fd, int shard, const double *mp);
 /* The compiled step-kernel variant that shard `shard` launches, as chosen by rkFDUpdateInit from the model and the tuning
  * variables RKFD_SPEC, RKFD_FORCE_BLOCK, RKFD_FORCE_MINB, RKFD_FORCE_GSCR and RKFD_FORCE_SMEM: v[0] threads per block, v[1] 1
  * when the scratch column lives in device memory (0: shared memory), v[2] 1 for the rigid-contact kernels, v[3] the model

@@ -87,6 +87,7 @@ def lib():
         "rkFDBatchGetLinkFrames": (ci, [vp, ci, vp, vp, vp]), "rkFDBatchGetLinkFramesDevice": (ci, [vp, ci, ci, vp, vp, vp]),
         "rkFDBatchLinkFrameKernelCount": (C.c_longlong, [vp]), "rkFDBatchKernelVariant": (ci, [vp, ci, _ip]),
         "rkFDBatchSetExtWrenchLinks": (ci, [vp, ci, vp]), "rkFDBatchSetExtWrench": (ci, [vp, vp]), "rkFDBatchSetExtWrenchDevice": (ci, [vp, ci, vp]),
+        "rkFDBatchSetMassPropLinks": (ci, [vp, ci, vp]), "rkFDBatchSetMassProp": (ci, [vp, vp]), "rkFDBatchSetMassPropDevice": (ci, [vp, ci, vp]),
         "rkFDB200DescribeModel": (ci, [vp, C.c_char_p, ci]), "rkFDBatchLastError": (C.c_char_p, []), "rkFDBatchDeviceCount": (ci, []), "rkFDB200MeasureFp64": (ci, [_dp]),
     }
     for name, (res, args) in sig.items():
@@ -506,6 +507,25 @@ class RkFD:
         """rkFDBatchSetExtWrenchDevice: raw device address (e.g. torch CUDA tensor .data_ptr()) of float64 w[Bs][n][6] of shard
         `shard`, indexed by the shard's local environment; stream-ordered on the engine's stream."""
         self._ck(lib().rkFDBatchSetExtWrenchDevice(self.h, shard, _ptr(w_ptr)))
+
+    def batch_set_mass_prop_links(self, links):
+        """rkFDBatchSetMassPropLinks (before update_init): the links (indices in flat_links() order) that take per-environment
+        mass properties, in the order of their rows; an empty list clears the declaration."""
+        pl = np.ascontiguousarray(links, np.int32).reshape(-1)
+        self._ck(lib().rkFDBatchSetMassPropLinks(self.h, pl.shape[0], _ptr(pl)))
+
+    def batch_set_mass_prop(self, mp):
+        """rkFDBatchSetMassProp: (B, n, 10) float64 host array, (mass, centre of mass, inertia about the centre of mass xx xy xz
+        yy yz zz) in link axes per declared link; checked (finite, mass > 0, inertia positive definite); held as pending before
+        update_init."""
+        if isinstance(mp, np.ndarray):
+            mp = np.ascontiguousarray(mp, np.float64)
+        self._ck(lib().rkFDBatchSetMassProp(self.h, _ptr(mp)))
+
+    def batch_set_mass_prop_device(self, shard, mp_ptr):
+        """rkFDBatchSetMassPropDevice: raw device address (e.g. torch CUDA tensor .data_ptr()) of float64 mp[Bs][n][10] of shard
+        `shard`, indexed by the shard's local environment; stream-ordered on the engine's stream, values unchecked."""
+        self._ck(lib().rkFDBatchSetMassPropDevice(self.h, shard, _ptr(mp_ptr)))
 
     def kernel_variant(self, shard=0):
         """rkFDBatchKernelVariant: (block, gscr, rigid, spec, minb) of the step-kernel variant shard `shard` launches."""

@@ -50,6 +50,8 @@ struct FDImpl {
   std::vector<double> pend_q, pend_qd, pend_u;   /* batched initial state given before rkFDUpdateInit */
   std::vector<int> fext_links;                   /* links declared for an external wrench (rkFDBatchSetExtWrenchLinks) */
   std::vector<double> pend_w;                    /* external wrench given before rkFDUpdateInit */
+  std::vector<int> mp_links;                     /* links declared for per-environment mass properties (rkFDBatchSetMassPropLinks) */
+  std::vector<double> pend_mp;                   /* mass properties given before rkFDUpdateInit */
   bool warned = false;
 };
 
@@ -425,11 +427,12 @@ extern "C" void rkFDUpdateInit(rkFD *fd)
       throw std::runtime_error("integrators: Regular form with RKG, RK4, Euler or Heun");
     w.integrator = fd->ode.integrator;
     w.fext_links = fi->fext_links;
-    std::string err;
-    if( !build_model(w, fi->model, err) ) throw std::runtime_error(err);
+    w.mp_links = fi->mp_links;
+    std::string err; std::vector<double> mp_default;
+    if( !build_model(w, fi->model, err, &mp_default) ) throw std::runtime_error(err);
     /* static chains carry no joint state, so the device rows are the host offsets of relayout() */
     if( fi->model.nq != fd->size ) throw std::runtime_error("joint state layout mismatch between the host mirror and the device model");
-    fi->engine = new Engine(fi->model, fi->B, fi->devices);
+    fi->engine = new Engine(fi->model, fi->B, fi->devices, mp_default.data());
     if( fi->resort >= 0 ) fi->engine->set_resort_interval(fi->resort);
     const int n = fd->size, nl = fi->model.nl, B = fi->B;
     /* initial state: the batched arrays when given, else the scalar state replicated over the envs */
@@ -442,6 +445,7 @@ extern "C" void rkFDUpdateInit(rkFD *fd)
     if( n > 0 ) fi->engine->set_state(q.data(), qd.data());
     if( nl > 0 ) fi->engine->set_motor_input(u.data());
     if( fi->model.nfext > 0 && fi->pend_w.size() == (size_t)B*6*fi->model.nfext ) fi->engine->set_ext_wrench(fi->pend_w.data());
+    if( fi->model.nmp > 0 && fi->pend_mp.size() == (size_t)B*10*fi->model.nmp ) fi->engine->set_mass_prop(fi->pend_mp.data());
     fi->engine->eval(true);            /* the committing evaluation at t=0 (reference rkfd_sim.c:556) */
     if( !fi->batch ){ fi->engine->sync(); mirror_env0(fd); }
   } catch(const std::exception &ex){ complain("rkFDUpdateInit", ex.what()); destroy_engine(fi); }
@@ -633,6 +637,59 @@ extern "C" int rkFDBatchSetExtWrenchDevice(rkFD *fd, int shard, const double *w)
   if( !w ) return fail("rkFDBatchSetExtWrenchDevice: w is needed");
   TRY(fi->engine->set_ext_wrench_device(shard, w));
 }
+/* per-environment mass properties of declared links (Engine::set_mass_prop): an input held like the external wrench */
+extern "C" int rkFDBatchSetMassPropLinks(rkFD *fd, int n, const int *links)
+{
+  BATCH_GUARD(fd);
+  if( fi->engine ) return fail("rkFDBatchSetMassPropLinks: declare the links before rkFDUpdateInit");
+  if( n < 0 || n > MAX_LINKS ) return fail("rkFDBatchSetMassPropLinks: n must be in [0, " + std::to_string(MAX_LINKS) + "]");
+  if( n > 0 && !links ) return fail("rkFDBatchSetMassPropLinks: links is needed");
+  const int nl = rkFDBatchLinkNum(fd);
+  std::vector<char> seen(nl > 0 ? nl : 1, 0);
+  for(int k=0;k<n;k++){
+    const int i = links[k];
+    if( i < 0 || i >= nl ) return fail("rkFDBatchSetMassPropLinks: link " + std::to_string(i) + " out of range [0, " + std::to_string(nl) + ")");
+    if( seen[i] ) return fail("rkFDBatchSetMassPropLinks: link " + std::to_string(i) + " listed twice");
+    seen[i] = 1;
+  }
+  fi->mp_links.assign(links, links + n);
+  fi->pend_mp.clear();                /* values held for an earlier declaration have another row count */
+  return 0;
+}
+/* "" when row r = (mass, c, Ic xx xy xz yy yz zz) is physical: finite, mass > 0, Ic positive definite (Cholesky) */
+static std::string mass_prop_problem(const double *r)
+{
+  for(int k=0;k<10;k++) if( !std::isfinite(r[k]) ) return "a non-finite entry";
+  if( !( r[0] > 0.0 ) ) return "mass " + std::to_string(r[0]) + " is not positive";
+  const double xx = r[4], xy = r[5], xz = r[6], yy = r[7], yz = r[8], zz = r[9];
+  if( !( xx > 0.0 ) ) return "the inertia is not positive definite";
+  const double l11 = std::sqrt(xx), l21 = xy/l11, l31 = xz/l11, d2 = yy - l21*l21;
+  if( !( d2 > 0.0 ) ) return "the inertia is not positive definite";
+  const double l22 = std::sqrt(d2), l32 = (yz - l31*l21)/l22, d3 = zz - l31*l31 - l32*l32;
+  if( !( d3 > 0.0 ) ) return "the inertia is not positive definite";
+  return "";
+}
+extern "C" int rkFDBatchSetMassProp(rkFD *fd, const double *mp)
+{
+  BATCH_GUARD(fd);
+  if( fi->mp_links.empty() ) return fail("rkFDBatchSetMassProp: no link is declared (rkFDBatchSetMassPropLinks)");
+  if( !mp ) return fail("rkFDBatchSetMassProp: mp is needed");
+  const size_t n = fi->mp_links.size();
+  for(int e=0;e<fi->B;e++) for(size_t k=0;k<n;k++){
+    const std::string why = mass_prop_problem(mp + ((size_t)e*n + k)*10);
+    if( !why.empty() ) return fail("rkFDBatchSetMassProp: environment " + std::to_string(e) + ", link " + std::to_string(fi->mp_links[k]) + ": " + why);
+  }
+  if( !fi->engine ){ fi->pend_mp.assign(mp, mp + (size_t)fi->B*10*n); return 0; }
+  TRY(fi->engine->set_mass_prop(mp));
+}
+extern "C" int rkFDBatchSetMassPropDevice(rkFD *fd, int shard, const double *mp)
+{
+  BATCH_GUARD(fd); NEED_ENGINE();
+  if( fi->engine->model().nmp <= 0 ) return fail("rkFDBatchSetMassPropDevice: no link is declared (rkFDBatchSetMassPropLinks)");
+  if( shard < 0 || shard >= fi->engine->num_shards() ) return fail("rkFDBatchSetMassPropDevice: shard index out of range");
+  if( !mp ) return fail("rkFDBatchSetMassPropDevice: mp is needed");
+  TRY(fi->engine->set_mass_prop_device(shard, mp));
+}
 /* the step-kernel variant a shard launches (Engine::Engine's choice from the model and the RKFD_* tuning variables) */
 extern "C" int rkFDBatchKernelVariant(rkFD *fd, int shard, int v[5])
 {
@@ -673,6 +730,8 @@ extern "C" int rkFDB200DescribeModel(rkFD *fd, char *buf, int cap)
   for(int i=0;i<m.npair;i++) if( m.pair[i].slinfo & 0xffff ){ const int si = m.pair[i].slinfo; const double v[3] = { (double)(si & 255), (double)((si >> 8) & 255), (double)((si >> 16) & 1) }; arr("pair.slide", i, v, 3); }
   /* links declared for an external wrench, in the order of its rows (rkFDBatchSetExtWrenchLinks) */
   if( m.nfext > 0 ){ double v[MAX_LINKS]; for(int i=0;i<m.nl;i++) if( m.link[i].fext_row >= 0 ) v[m.link[i].fext_row] = i; arr("ext.links", 0, v, m.nfext); }
+  /* links declared for per-environment mass properties, in the order of their rows (rkFDBatchSetMassPropLinks) */
+  if( m.nmp > 0 ){ double v[MAX_LINKS]; for(int i=0;i<m.nl;i++) if( m.mp_row[i] >= 0 ) v[m.mp_row[i]] = i; arr("mp.links", 0, v, m.nmp); }
   if( fd->dis && fd->size > 0 ) arr("init.q", 0, fd->dis->buf, fd->size);     /* the registered initial displacements ([roki::chain::init]) */
   if( buf && cap > 0 ){ std::snprintf(buf, cap, "%s", s.c_str()); }
   return (int)s.size();

@@ -165,6 +165,7 @@ struct SpecGeneric {
   static RKFD_HD int wext_slot(int, const LinkDev &L){ return L.wext_slot; }
   static RKFD_HD int frame_slot(int, const LinkDev &L){ return L.frame_slot; }
   static RKFD_HD int fext_row(int, const LinkDev &L){ return L.fext_row; }
+  static RKFD_HD int mp_row(const ModelDev &m, int i){ return m.mp_row[i]; }
   static RKFD_HD int rk_slot(const ModelDev &m){ return m.rk_slot; }
   static RKFD_HD int nq(const ModelDev &m){ return m.nq; }
   /* 1-DoF joints: slots of (sin, cos, 1/D, u) in the "T space" (Ctx::TL/TS) - the scratch column itself here */
@@ -204,6 +205,7 @@ struct SpecSerialRev {
   static RKFD_HD int wext_slot(int i, const LinkDev &L){ return ( i == NL_-1 && L.cell_end > L.cell_begin ) ? WEXT : -1; }
   static RKFD_HD int frame_slot(int, const LinkDev &){ return -1; }
   static constexpr RKFD_HD int fext_row(int, const LinkDev &){ return -1; }     /* external wrenches: generic kernels only */
+  static constexpr RKFD_HD int mp_row(const ModelDev &, int){ return -1; }      /* per-environment mass properties: generic kernels only */
   static RKFD_HD int rk_slot(const ModelDev &){ return RK; }
   static RKFD_HD int nq(const ModelDev &){ return NL_ - 1; }
 };
@@ -241,12 +243,14 @@ struct SpecSerialRevRolled {
   static RKFD_HD int wext_slot(int i, const LinkDev &L){ return ( i == NL_-1 && L.cell_end > L.cell_begin ) ? WEXT : -1; }
   static RKFD_HD int frame_slot(int i, const LinkDev &L){ return ( RG_ && i == NL_-1 && L.cell_end > L.cell_begin ) ? FRAME : -1; }
   static constexpr RKFD_HD int fext_row(int, const LinkDev &){ return -1; }     /* external wrenches: generic kernels only */
+  static constexpr RKFD_HD int mp_row(const ModelDev &, int){ return -1; }      /* per-environment mass properties: generic kernels only */
   static RKFD_HD int rk_slot(const ModelDev &){ return RK; }
   static RKFD_HD int nq(const ModelDev &){ return NL_ - 1; }
   static RKFD_HD int sc(int i, const LinkDev &){ return RG_ ? PER*i + 9 : 4*(i-1); }
 };
 inline bool spec_serial_rev_rolled_match(const ModelDev &m, int NL, int RG = 0, int GEN = 0){
-  if( m.nfw > 1 || m.npair > m.npair_static || m.nslide > 0 || m.nfext > 0 ) return false;   /* slide mode, external wrenches: generic kernel only */
+  if( m.nfw > 1 || m.npair > m.npair_static || m.nslide > 0 || m.nfext > 0 || m.nmp > 0 ) return false;   /* slide mode, external wrenches, mass
+                                                                                                          * properties: generic kernel only */
   if( RG ? !( m.has_rigid && m.nrg == 1 && m.rigid_link == NL-1 ) : m.has_rigid ) return false;
   if( m.nl != NL || NL < 2 ) return false;
   for(int i=0;i<NL;i++){
@@ -261,7 +265,7 @@ inline bool spec_serial_rev_rolled_match(const ModelDev &m, int NL, int RG = 0, 
 
 /* does the flattened model have the shape SpecSerialRev<.,NL,CLS> assumes? (host side) */
 inline bool spec_serial_rev_match(const ModelDev &m, int NL, unsigned CLS){
-  if( m.has_rigid || m.nl != NL || NL < 2 || m.nfw > 1 || m.npair > m.npair_static || m.nslide > 0 || m.nfext > 0 ) return false;
+  if( m.has_rigid || m.nl != NL || NL < 2 || m.nfw > 1 || m.npair > m.npair_static || m.nslide > 0 || m.nfext > 0 || m.nmp > 0 ) return false;
   for(int i=0;i<NL;i++){
     const LinkDev &L = m.link[i];
     if( i == 0 ){ if( L.parent >= 0 || L.jtype != J_FIXED || L.cell_end > L.cell_begin ) return false; continue; }
@@ -822,7 +826,9 @@ struct Core {
         const V3 f = v3(c.gld(c.st.fext, 6*fr), c.gld(c.st.fext, 6*fr+1), c.gld(c.st.fext, 6*fr+2));
         const V3 n = v3(c.gld(c.st.fext, 6*fr+3), c.gld(c.st.fext, 6*fr+4), c.gld(c.st.fext, 6*fr+5));
         const V3 fl = tmul(k.Rw, f);
-        w.l = w.l + fl; w.a = w.a + ( tmul(k.Rw, n) + cross(v3(L.com[0], L.com[1], L.com[2]), fl) );
+        const int mr = Spec::mp_row(m, i);     /* the centre of mass of the environment when the link takes mass properties */
+        const V3 com = mr >= 0 ? v3(c.gld(c.st.mp, 10*mr+1), c.gld(c.st.mp, 10*mr+2), c.gld(c.st.mp, 10*mr+3)) : v3(L.com[0], L.com[1], L.com[2]);
+        w.l = w.l + fl; w.a = w.a + ( tmul(k.Rw, n) + cross(com, fl) );
       }
       st3(wx, w.l); st3(wx+3, w.a);
       if( fs >= 0 ){ stm(fs, k.Rw); st3(fs+9, k.pw); st3(fs+12, k.vl); st3(fs+15, k.om); }
@@ -890,15 +896,25 @@ struct Core {
       const double pf_u = nx_u, pf_prev = nx_prev;
       if( i > 0 && m.link[i-1].mtype != M_NONE ){ nx_u = c.gld(c.st.u, i-1); nx_prev = c.gld(c.st.piv_prev, Spec::qofs(i-1, m.link[i-1])); }
       const V3 om = ld3(Spec::wslot(i,L));
-      const V3 mc = v3(L.mc[0],L.mc[1],L.mc[2]);
+      V3 mc = v3(L.mc[0],L.mc[1],L.mc[2]);
+      double mass = L.mass;
       S3 A, C; M3 B;
-      A.xx = L.mass; A.xy = 0; A.xz = 0; A.yy = L.mass; A.yz = 0; A.zz = L.mass;
-      B.xx = 0; B.xy = mc.z; B.xz = -mc.y; B.yx = -mc.z; B.yy = 0; B.yz = mc.x; B.zx = mc.y; B.zy = -mc.x; B.zz = 0;
       C.xx = L.Io[0]; C.xy = L.Io[1]; C.xz = L.Io[2]; C.yy = L.Io[3]; C.yz = L.Io[4]; C.zz = L.Io[5];
+      /* per-environment mass properties (a compile-time -1 in the specialisations): the row's (m, c, Ic) about the origin */
+      const int mr = Spec::mp_row(m, i);
+      if( mr >= 0 ){
+        S3 Ic; mass = c.gld(c.st.mp, 10*mr);
+        const V3 com = v3(c.gld(c.st.mp, 10*mr+1), c.gld(c.st.mp, 10*mr+2), c.gld(c.st.mp, 10*mr+3));
+        Ic.xx = c.gld(c.st.mp, 10*mr+4); Ic.xy = c.gld(c.st.mp, 10*mr+5); Ic.xz = c.gld(c.st.mp, 10*mr+6);
+        Ic.yy = c.gld(c.st.mp, 10*mr+7); Ic.yz = c.gld(c.st.mp, 10*mr+8); Ic.zz = c.gld(c.st.mp, 10*mr+9);
+        mass_prop_origin(mass, com, Ic, mc, C);
+      }
+      A.xx = mass; A.xy = 0; A.xz = 0; A.yy = mass; A.yz = 0; A.zz = mass;
+      B.xx = 0; B.xy = mc.z; B.xz = -mc.y; B.yx = -mc.z; B.yy = 0; B.yz = mc.x; B.zx = mc.y; B.zy = -mc.x; B.zz = 0;
       /* bias ( w x (w x mc) ; w x (Io w) ) minus gravity (m gd ; mc x gd) minus external wrench */
       V3 pf = cross(om, cross(om, mc));
       V3 pn = cross(om, mul(C, om));
-      if( !gacc ){ const V3 gd = ld3(Spec::wslot(i,L)+3); pf = pf - L.mass*gd; pn = pn - cross(mc, gd); }
+      if( !gacc ){ const V3 gd = ld3(Spec::wslot(i,L)+3); pf = pf - mass*gd; pn = pn - cross(mc, gd); }
       if( Spec::wext_slot(i,L) >= 0 ){ pf = pf - ld3(Spec::wext_slot(i,L)); pn = pn - ld3(Spec::wext_slot(i,L)+3); }
       if( Spec::accum_slot(i,L) >= 0 ){
         const int a = L.accum_slot; const S3 aA = lds(a), aC = lds(a+15); const M3 aB = ldm(a+6);

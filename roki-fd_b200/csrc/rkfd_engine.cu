@@ -138,10 +138,12 @@ __global__ void __launch_bounds__(256) rkfd_perm_compose_kernel(const int * __re
 constexpr int RESET_CHUNK = 65536;     /* sub-state capacity: longer lists run in chunks */
 constexpr int RESET_SEGS = 11, RESET_ROWS = 32;
 /* q, q' and u of the sub-state: the given rows, u from the environment's slot when none is given, zero on padding slots; the
- * external wrench (nfx rows) always from the environment's slot: a reset does not change the input */
+ * external wrench (nfx rows) always from the environment's slot: a reset does not change the input.  So do the mass properties
+ * (nmr rows), and padding slots take slot 0's: valid values, a padding thread runs the articulated-body pass too */
 __global__ void __launch_bounds__(256) rkfd_reset_gather_kernel(StateDev sub, const double * __restrict__ u_cur, int ld, int B, const int * __restrict__ inv,
                                                                 const int * __restrict__ envs, int n, const double * __restrict__ q, const double * __restrict__ qd,
-                                                                const double * __restrict__ u, int nq, int nl, const double * __restrict__ fext_cur, int nfx)
+                                                                const double * __restrict__ u, int nq, int nl, const double * __restrict__ fext_cur, int nfx,
+                                                                const double * __restrict__ mp_cur, int nmr)
 {
   const int i = blockIdx.x*blockDim.x + threadIdx.x;
   if( i >= sub.ld ) return;
@@ -154,6 +156,7 @@ __global__ void __launch_bounds__(256) rkfd_reset_gather_kernel(StateDev sub, co
   }
   for(int k=0;k<nl;k++) sub.u[(size_t)k*sub.ld + i] = !live ? 0.0 : ( u ? u[(size_t)i*nl + k] : u_cur[(size_t)k*ld + sl] );
   for(int k=0;k<nfx;k++) sub.fext[(size_t)k*sub.ld + i] = live ? fext_cur[(size_t)k*ld + sl] : 0.0;
+  for(int k=0;k<nmr;k++) sub.mp[(size_t)k*sub.ld + i] = mp_cur[(size_t)k*ld + sl];
 }
 /* row groups copied back from the sub-state (stride ld_sub, slot i) to the shard (stride ld, the environment's slot) */
 struct ResetRows { int nseg; int rows[RESET_SEGS], esz[RESET_SEGS]; const char *src[RESET_SEGS]; char *dst[RESET_SEGS]; };
@@ -349,11 +352,12 @@ static int g_model_owner[64][NVARIANTS] = {{0}};   /* [device][variant]: engine 
 
 static int variant_index(const KernelVariant *kv){ for(int i=0;i<NVARIANTS;i++) if( g_variants[i] == kv ) return i; return 0; }
 
-Engine::Engine(const ModelDev &model, int B, const std::vector<int> &devices) : model_(model), model_tm_(model), B_(B), id_(g_next_engine_id++)
+Engine::Engine(const ModelDev &model, int B, const std::vector<int> &devices, const double *mp_default) : model_(model), model_tm_(model), B_(B), id_(g_next_engine_id++)
 {
   /* the same table with the tensor-memory scratch map, for the generic kernel variant that keeps its T space in TMEM */
   if( !model.has_rigid ) model_layout(model_tm_, true);
   if( B <= 0 ) throw std::runtime_error("rokifd_b200: environment count must be positive");
+  if( model.nmp > 0 && !mp_default ) throw std::runtime_error("rokifd_b200: mass properties: the model's own values are needed");
   /* environment re-sort by contact count: every 16 steps when the world has contact pairs (RKFD_RESORT=<steps>, 0: never).
    * Measured on one B200 over 256 settled steps, sorts included (tools/exp_resort.py): C3 0.538 ms per step without, 0.484 /
    * 0.481 / 0.489 / 0.503 ms at 8 / 16 / 32 / 64; C5 MLCP 1.88 -> 1.42, C5 Vert 6.97 -> 5.09 at 16 */
@@ -389,15 +393,22 @@ Engine::Engine(const ModelDev &model, int B, const std::vector<int> &devices) : 
     st.cf = dalloc<double>(*s, (size_t)3*ns*s->ld);
     st.status = dalloc<int>(*s, s->ld);
     st.fext = model.nfext > 0 ? dalloc<double>(*s, (size_t)6*model.nfext*s->ld) : nullptr;     /* zero: the initial wrench */
+    st.mp = model.nmp > 0 ? dalloc<double>(*s, (size_t)10*model.nmp*s->ld) : nullptr;          /* filled below */
     st.work = ( std::getenv("RKFD_NO_WORK_SORT") == nullptr && model.has_rigid && model.solver != S_MLCP ) ? dalloc<unsigned char>(*s, s->ld) : nullptr;
     /* per-warp workspace of the dense warp-cooperative contact solve; the single-link paths use ws1 only */
     st.ws = ( model.ws_doubles > 0 && model.rigid_link < 0 ) ? dalloc<double>(*s, (size_t)(s->ld/32)*model.ws_doubles) : nullptr;
     st.ws1 = model.ws1_doubles > 0 ? dalloc<double>(*s, (size_t)model.ws1_doubles*s->ld) : nullptr;
     int nmax = nq; if( nl > nmax ) nmax = nl; if( 3*ns > nmax ) nmax = 3*ns; if( 6*model.nfext > nmax ) nmax = 6*model.nfext;
+    if( 10*model.nmp > nmax ) nmax = 10*model.nmp;
     /* the kernels index the per-environment arrays with 32-bit element offsets (row * ld + e) */
     if( (unsigned long long)nmax*(unsigned long long)s->ld >= (1ull << 32) )
       throw std::runtime_error("rokifd_b200: rows x environments per device exceed 2^32 elements - spread the batch over more devices (rkFDBatchSetDevices)");
     s->nstage = (size_t)nmax*s->B; if( s->nstage < 256 ) s->nstage = 256; s->dstage = dalloc<double>(*s, s->nstage);
+    if( st.mp ){    /* every slot, the padding [B, ld) too, starts with the model's own mass properties */
+      CK(cudaMemcpy(s->dstage, mp_default, (size_t)10*model.nmp*sizeof(double), cudaMemcpyHostToDevice));
+      rkfd_fill_rows_kernel<<<s->ld/256, 256>>>(st.mp, s->ld, s->ld, 10*model.nmp, s->dstage);
+      CK(cudaGetLastError());
+    }
     /* launch configuration: the block size that keeps most environments resident per SM; scratch in HBM
      * (gscr) only when no shared-memory variant fits */
     int best = 0; const bool rigid = model.has_rigid;
@@ -510,6 +521,7 @@ void Engine::resort(Shard &s)
     s.perm_buf[0] = dalloc<int>(s, s.ld); s.perm_buf[1] = dalloc<int>(s, s.ld); s.inv_buf = dalloc<int>(s, s.ld);
     size_t rows = (size_t)3*ns; if( (size_t)nq > rows ) rows = nq; if( (size_t)nl > rows ) rows = nl; if( (size_t)nfw > rows ) rows = nfw;
     if( (size_t)6*model_.nfext > rows ) rows = (size_t)6*model_.nfext;
+    if( (size_t)10*model_.nmp > rows ) rows = (size_t)10*model_.nmp;
     s.ptmp_bytes = rows*s.ld*sizeof(double); s.ptmp = dalloc<double>(s, rows*s.ld);
     CK(cudaDeviceSynchronize());       /* dalloc's zero-fill runs on the legacy stream */
   }
@@ -531,7 +543,7 @@ void Engine::resort(Shard &s)
     CK(cudaGetLastError());
   };
   StateDev &st = s.st;
-  perm_rows(st.q[s.cur], 8, nq); perm_rows(st.qd[s.cur], 8, nq); perm_rows(st.qdd, 8, nq); perm_rows(st.u, 8, nl); perm_rows(st.fext, 8, 6*model_.nfext);
+  perm_rows(st.q[s.cur], 8, nq); perm_rows(st.qd[s.cur], 8, nq); perm_rows(st.qdd, 8, nq); perm_rows(st.u, 8, nl); perm_rows(st.fext, 8, 6*model_.nfext); perm_rows(st.mp, 8, 10*model_.nmp);
   perm_rows(st.piv_prev, 8, nq); perm_rows(st.piv_type, 4, 1); perm_rows(st.cflags, 8, nfw);
   perm_rows(st.cref, 8, 3*ns); perm_rows(st.cf, 8, 3*ns); perm_rows(st.status, 4, 1);
   int *pn = s.perm_buf[s.perm_cur ^ 1];
@@ -562,6 +574,7 @@ static ResetLayout reset_layout(const Shard &s, const ModelDev &m, int ld, int c
   for(int k=0;k<2;k++){ st.q[k] = (double*)take(8*nq*L); st.qd[k] = (double*)take(8*nq*L); }
   st.u = (double*)take(8*nl*L);
   if( s.st.fext ) st.fext = (double*)take(8*6*(size_t)m.nfext*L);
+  if( s.st.mp ) st.mp = (double*)take(8*10*(size_t)m.nmp*L);
   if( s.st.scratch ) st.scratch = (double*)take(8*(size_t)m.nscratch*L);
   if( s.st.ws ) st.ws = (double*)take(8*(L/32)*(size_t)m.ws_doubles);
   if( s.st.ws1 ) st.ws1 = (double*)take(8*(size_t)m.ws1_doubles*L);
@@ -590,7 +603,7 @@ void Engine::reset_chunk(Shard &s, int n, const int *envs, const double *q, cons
   const ResetLayout r = reset_layout(s, model_, ld, s.rcap, s.rbuf);
   const StateDev &sub = r.st;
   CK(cudaMemsetAsync(s.rbuf + r.zero_ofs, 0, r.zero_bytes, s.stream));
-  rkfd_reset_gather_kernel<<<ld/256, 256, 0, s.stream>>>(sub, s.st.u, s.ld, s.B, s.inv, envs, n, q, qd, u, nq, nl, s.st.fext, 6*model_.nfext);
+  rkfd_reset_gather_kernel<<<ld/256, 256, 0, s.stream>>>(sub, s.st.u, s.ld, s.B, s.inv, envs, n, q, qd, u, nq, nl, s.st.fext, 6*model_.nfext, s.st.mp, 10*model_.nmp);
   CK(cudaGetLastError());
   launch(s, sub, 0, 2, 0);                    /* rkFDUpdateInit's committing evaluation, on the sub-state */
   ResetRows rr; std::memset(&rr, 0, sizeof rr);
@@ -902,6 +915,24 @@ void Engine::set_ext_wrench_device(int si, const double *w)
   int prev = 0; CK(cudaGetDevice(&prev)); CK(cudaSetDevice(s.dev));
   /* the transposing scatter reads the caller's env-major rows through the slot permutation: no staging copy */
   xp_scatter(w, s.st.fext, s.B, 6*model_.nfext, s.ld, s.stream, s.perm);
+  CK(cudaGetLastError());
+  CK(cudaSetDevice(prev));
+}
+void Engine::set_mass_prop(const double *mp)
+{
+  if( model_.nmp <= 0 ) throw std::runtime_error("rokifd_b200: mass properties: no link is declared (rkFDBatchSetMassPropLinks)");
+  int prev = 0; CK(cudaGetDevice(&prev));
+  for(Shard *s : shards_){ CK(cudaSetDevice(s->dev)); h2d_scatter(*s, mp, 10*model_.nmp, s->st.mp); }
+  for(Shard *s : shards_){ CK(cudaSetDevice(s->dev)); CK(cudaStreamSynchronize(s->stream)); }
+  CK(cudaSetDevice(prev));
+}
+void Engine::set_mass_prop_device(int si, const double *mp)
+{
+  if( model_.nmp <= 0 ) throw std::runtime_error("rokifd_b200: mass properties: no link is declared (rkFDBatchSetMassPropLinks)");
+  if( si < 0 || si >= (int)shards_.size() ) throw std::runtime_error("rokifd_b200: mass properties: shard index out of range");
+  Shard &s = *shards_[si];
+  int prev = 0; CK(cudaGetDevice(&prev)); CK(cudaSetDevice(s.dev));
+  xp_scatter(mp, s.st.mp, s.B, 10*model_.nmp, s.ld, s.stream, s.perm);     /* through the slot permutation, as set_ext_wrench_device */
   CK(cudaGetLastError());
   CK(cudaSetDevice(prev));
 }

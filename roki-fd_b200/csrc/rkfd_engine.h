@@ -16,7 +16,8 @@ struct Shard;
 class Engine {
  public:
   /* devices empty -> the current device */
-  Engine(const ModelDev &model, int B, const std::vector<int> &devices);
+  /* mp_default: the model's own mass properties of the declared links ([nmp][10], build_model), needed when model.nmp > 0 */
+  Engine(const ModelDev &model, int B, const std::vector<int> &devices, const double *mp_default = nullptr);
   ~Engine();
   Engine(const Engine&) = delete;
   Engine &operator=(const Engine&) = delete;
@@ -78,6 +79,12 @@ class Engine {
    * declared link */
   void set_ext_wrench(const double *w);
   void set_ext_wrench_device(int shard, const double *w);
+  /* mass properties of the declared links (ModelDev::nmp), env-major [B][nmp][10]: (mass, centre of mass, inertia about the
+   * centre of mass xx xy xz yy yz zz), link axes.  set_mass_prop: host array, every shard, synchronous.  set_mass_prop_device:
+   * a device buffer [Bs][nmp][10] of shard `shard`, indexed by the environment local to the shard; stream-ordered, no
+   * allocation.  Both throw without a declared link; neither checks the values */
+  void set_mass_prop(const double *mp);
+  void set_mass_prop_device(int shard, const double *mp);
 
   /* link kinematics (rkfd_kin.cuh): world frames [B][nsel][12] (R row-major, p) and velocities [B][nsel][6] (linear, angular;
    * world axes) of the output columns of table `t`, from the committed state; a null output is neither computed nor written.

@@ -111,9 +111,9 @@ struct DevCtx {
  * variant has its own kernel symbol: two translation units instantiating the same template arguments with
  * different launch bounds would collide at link time and launch each other's module (and constant bank). */
 template <int BLOCK, bool GSCR, bool RIGID, int SPEC, int MINB>
-__global__ void __launch_bounds__(BLOCK, MINB) rkfd_step_kernel(StateDevHead sh, int cur, int mode, int nsteps, double *fext)
+__global__ void __launch_bounds__(BLOCK, MINB) rkfd_step_kernel(StateDevHead sh, int cur, int mode, int nsteps, double *fext, double *mp)
 {
-  StateDev st; static_cast<StateDevHead &>(st) = sh; st.fext = fext;
+  StateDev st; static_cast<StateDevHead &>(st) = sh; st.fext = fext; st.mp = mp;
   using Spec = typename SpecOf<SPEC>::type;
   constexpr bool TM = Spec::TM != 0;
   int e_ = blockIdx.x*BLOCK + threadIdx.x;

@@ -14,7 +14,7 @@ namespace rkfd {
 
 static void launch(const StateDev &st, int cur, int mode, int nsteps, int grid, size_t smem, cudaStream_t stream)
 {
-  rkfd_step_kernel<RKFD_BLOCK, RKFD_GSCR != 0, RKFD_RIGID != 0, RKFD_SPEC, RKFD_MINB><<<grid, RKFD_BLOCK, smem, stream>>>(st, cur, mode, nsteps, st.fext);
+  rkfd_step_kernel<RKFD_BLOCK, RKFD_GSCR != 0, RKFD_RIGID != 0, RKFD_SPEC, RKFD_MINB><<<grid, RKFD_BLOCK, smem, stream>>>(st, cur, mode, nsteps, st.fext, st.mp);
 }
 static int blocks_per_sm(size_t smem)
 {

@@ -22,6 +22,43 @@ struct S3 { double xx, xy, xz, yy, yz, zz; };               /* symmetric */
 struct V6 { V3 l, a; };                                      /* (linear, angular) */
 
 RKFD_HD V3 v3(double x, double y, double z){ V3 r; r.x=x; r.y=y; r.z=z; return r; }
+
+/* products and sums that the compiler may not contract into multiply-adds (the host build does not contract) */
+RKFD_HD double mul_rn(double a, double b){
+#if defined(__CUDA_ARCH__)
+  return __dmul_rn(a, b);
+#else
+  return a*b;
+#endif
+}
+RKFD_HD double add_rn(double a, double b){
+#if defined(__CUDA_ARCH__)
+  return __dadd_rn(a, b);
+#else
+  return a + b;
+#endif
+}
+RKFD_HD double sub_rn(double a, double b){
+#if defined(__CUDA_ARCH__)
+  return __dsub_rn(a, b);
+#else
+  return a - b;
+#endif
+}
+/* rigid-body inertia of a link about its origin from its mass m, centre of mass c and inertia Ic about c (link axes):
+ * mc = m c and Io = Ic - m [c x]^2 = Ic + m (|c|^2 E - c c^T).  build_model fills the constant table with it and Core::pass2
+ * forms per-environment values with it: the same operations in the same order, so that a link given the model's own values
+ * gets the table's values bit for bit */
+RKFD_HD void mass_prop_origin(double m, V3 c, const S3 &Ic, V3 &mc, S3 &Io){
+  const double c2 = add_rn(add_rn(mul_rn(c.x, c.x), mul_rn(c.y, c.y)), mul_rn(c.z, c.z));
+  mc.x = mul_rn(m, c.x); mc.y = mul_rn(m, c.y); mc.z = mul_rn(m, c.z);
+  Io.xx = add_rn(Ic.xx, mul_rn(m, sub_rn(c2, mul_rn(c.x, c.x))));
+  Io.xy = add_rn(Ic.xy, mul_rn(m, sub_rn(0.0, mul_rn(c.x, c.y))));
+  Io.xz = add_rn(Ic.xz, mul_rn(m, sub_rn(0.0, mul_rn(c.x, c.z))));
+  Io.yy = add_rn(Ic.yy, mul_rn(m, sub_rn(c2, mul_rn(c.y, c.y))));
+  Io.yz = add_rn(Ic.yz, mul_rn(m, sub_rn(0.0, mul_rn(c.y, c.z))));
+  Io.zz = add_rn(Ic.zz, mul_rn(m, sub_rn(c2, mul_rn(c.z, c.z))));
+}
 RKFD_HD V3 operator+(V3 a, V3 b){ return v3(a.x+b.x, a.y+b.y, a.z+b.z); }
 RKFD_HD V3 operator-(V3 a, V3 b){ return v3(a.x-b.x, a.y-b.y, a.z-b.z); }
 RKFD_HD V3 operator-(V3 a){ return v3(-a.x,-a.y,-a.z); }

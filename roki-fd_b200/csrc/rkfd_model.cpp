@@ -70,7 +70,7 @@ static bool box_sign_bit_order(double *v)
   return false;
 }
 
-bool build_model(const WorldHost &w, ModelDev &m, std::string &err)
+bool build_model(const WorldHost &w, ModelDev &m, std::string &err, std::vector<double> *mp_default)
 {
   std::memset(&m, 0, sizeof m);
   m.dt = w.dt; m.inv_dt = 1.0/w.dt; m.friction_weight = w.friction_weight; m.pyramid = w.pyramid; m.max_iter = w.max_iter; m.solver = w.solver; m.integrator = w.integrator;
@@ -87,6 +87,7 @@ bool build_model(const WorldHost &w, ModelDev &m, std::string &err)
   struct StatBox { BoxDev b; std::string stuff; int ord, slide; };
   std::vector<StatBox> boxes;
   std::vector<int> cell_ord, cell_slide, mbox_ord, mbox_slide;      /* registration order / slide entry (-1: none) of every cell and moving box */
+  std::vector<double> link_mp;                                       /* [nl][10]: mass properties of every link, the rows of StateDev::mp */
   int ord = 0;                                                       /* shapes in the order of rkFDChainReg: chains, links, shapes then boxes */
   auto add_slide = [&](const LinkHost::Slide *sl, const double *lR, const double *lp) -> int {
     if( !sl ) return -1;
@@ -134,7 +135,7 @@ bool build_model(const WorldHost &w, ModelDev &m, std::string &err)
       d.fext_row = -1;
       std::memcpy(d.Ro, l.Ro, sizeof d.Ro); std::memcpy(d.po, l.po, sizeof d.po);
       d.mass = l.mass;
-      for(int k=0;k<3;k++){ d.com[k] = l.com[k]; d.mc[k] = l.mass*l.com[k]; }
+      for(int k=0;k<3;k++) d.com[k] = l.com[k];
       { /* class of the constant rotation; entries within 1e-14 of {0,+-1} are snapped so that the structured
            transforms are exact signed permutations */
         static const double RI[9] = {1,0,0, 0,1,0, 0,0,1}, RP[9] = {1,0,0, 0,0,-1, 0,1,0}, RM[9] = {1,0,0, 0,0,1, 0,-1,0};
@@ -144,10 +145,14 @@ bool build_model(const WorldHost &w, ModelDev &m, std::string &err)
         d.rsg = d.rcls == RO_RXP ? 1.0 : ( d.rcls == RO_RXM ? -1.0 : 0.0 );
         for(int k=0;k<3;k++) d.pol[k] = d.Ro[k]*d.po[0] + d.Ro[3+k]*d.po[1] + d.Ro[6+k]*d.po[2];
       }
-      { /* Io = Ic - m [c x]^2 = Ic + m (|c|^2 E - c c^T) */
-        const double *c = l.com, c2 = c[0]*c[0]+c[1]*c[1]+c[2]*c[2]; double Io[9];
-        for(int r=0;r<3;r++) for(int q=0;q<3;q++) Io[3*r+q] = l.inertia[3*r+q] + l.mass*((r==q?c2:0.0) - c[r]*c[q]);
-        d.Io[0]=Io[0]; d.Io[1]=0.5*(Io[1]+Io[3]); d.Io[2]=0.5*(Io[2]+Io[6]); d.Io[3]=Io[4]; d.Io[4]=0.5*(Io[5]+Io[7]); d.Io[5]=Io[8];
+      { /* mc and Io from the symmetric part of Ic (a symmetric inertia is taken as it is) */
+        const double *I = l.inertia; S3 Ic, Io; V3 mc;
+        Ic.xx = I[0]; Ic.xy = 0.5*(I[1]+I[3]); Ic.xz = 0.5*(I[2]+I[6]); Ic.yy = I[4]; Ic.yz = 0.5*(I[5]+I[7]); Ic.zz = I[8];
+        mass_prop_origin(l.mass, v3(l.com[0], l.com[1], l.com[2]), Ic, mc, Io);
+        d.mc[0] = mc.x; d.mc[1] = mc.y; d.mc[2] = mc.z;
+        d.Io[0] = Io.xx; d.Io[1] = Io.xy; d.Io[2] = Io.xz; d.Io[3] = Io.yy; d.Io[4] = Io.yz; d.Io[5] = Io.zz;
+        const double row[10] = { l.mass, l.com[0], l.com[1], l.com[2], Ic.xx, Ic.xy, Ic.xz, Ic.yy, Ic.yz, Ic.zz };
+        link_mp.insert(link_mp.end(), row, row + 10);
       }
       d.stiffness = l.stiffness; d.viscosity = l.viscosity; d.coulomb = l.coulomb; d.sfriction = l.sfriction;
       d.brk_f = l.brk_f; d.brk_t = l.brk_t;
@@ -260,6 +265,18 @@ bool build_model(const WorldHost &w, ModelDev &m, std::string &err)
   }
   m.nfext = (int)w.fext_links.size();
   m.need_world = m.npair > 0 || m.nfext > 0;
+  /* links that take per-environment mass properties (rkFDBatchSetMassPropLinks): row k is link mp_links[k] */
+  if( (int)w.mp_links.size() > MAX_LINKS ){ err = "at most " + std::to_string(MAX_LINKS) + " links take mass properties (MAX_LINKS)"; return false; }
+  for(int i=0;i<MAX_LINKS;i++) m.mp_row[i] = -1;
+  if( mp_default ) mp_default->clear();
+  for(size_t k=0;k<w.mp_links.size();k++){
+    const int i = w.mp_links[k];
+    if( i < 0 || i >= nl ){ err = "mass properties: link index " + std::to_string(i) + " out of range [0, " + std::to_string(nl) + ")"; return false; }
+    if( m.mp_row[i] >= 0 ){ err = "mass properties: link " + std::to_string(i) + " listed twice"; return false; }
+    m.mp_row[i] = (int)k;
+    if( mp_default ) mp_default->insert(mp_default->end(), link_mp.begin() + 10*i, link_mp.begin() + 10*i + 10);
+  }
+  m.nmp = (int)w.mp_links.size();
 
   /* ---- topology flags and the scratch slot map */
   for(int i=0;i<nl;i++) if( m.link[i].parent >= 0 ) m.link[m.link[i].parent].nchild++;

@@ -69,11 +69,13 @@ struct WorldHost {
   double dt = 0.001, friction_weight = 100.0;
   int pyramid = 8, max_iter = 10, solver = S_VERT, integrator = 0;
   std::vector<int> fext_links;              /* links that take an external wrench, in the order of its input rows */
+  std::vector<int> mp_links;                /* links that take per-environment mass properties, in the order of their rows */
 };
 
 /* Flattens the world into `out`.  Returns false and fills `err` when a limit of the fused kernel is
- * exceeded or the topology is not supported. */
-bool build_model(const WorldHost &w, ModelDev &out, std::string &err);
+ * exceeded or the topology is not supported.  mp_default (optional): the model's own mass properties of the links of
+ * w.mp_links, [nmp][10] = (mass, centre of mass, inertia about it xx xy xz yy yz zz), the initial rows of StateDev::mp. */
+bool build_model(const WorldHost &w, ModelDev &out, std::string &err, std::vector<double> *mp_default = nullptr);
 
 /* Scratch map of the generic kernel.  tm = false: everything in the shared-memory column.  tm = true (worlds without
  * rigid pairs): (sin, cos, 1/D, u) of the 1-DoF joints and the integrator stage state move to the T space (tensor

@@ -127,6 +127,9 @@ struct ModelDev {
   MBoxDev mbox[MAX_MBOXES];
   PairDev pair[MAX_PAIRS];
   double vert[3 * MAX_VERTS];
+  /* per-environment mass properties (rkFDBatchSetMassPropLinks), appended so that no entry above moves */
+  int nmp;             /* links declared for per-environment mass properties */
+  int mp_row[MAX_LINKS];   /* >=0: row of link i's mass properties in StateDev::mp, else -1 */
 };
 
 /* Link table of the kinematics pass (rkfd_kin.cuh, rkFDBatchGetLinkFrames).  It is a __grid_constant__ kernel parameter, not
@@ -172,11 +175,13 @@ struct StateDevHead {
   unsigned char *work;    /* [ld] or null: work class of the environment's last rigid solve (Vert / Volume: pairs or contacts and
                            * active-set iterations), 0 = no solve; the engine's re-sort groups equal classes into warps */
 };
-/* The step kernel takes the head as its first parameter and fext as its last one (rkfd_kernel.cuh): its other parameters keep
- * their places in the parameter space, and kernels that never read fext compile to the code they had without it */
+/* The step kernel takes the head as its first parameter and fext and mp as its last ones (rkfd_kernel.cuh): its other
+ * parameters keep their places in the parameter space, and kernels that never read them compile to the code they had without them */
 struct StateDev : StateDevHead {
   double *fext;           /* [6*nfext][ld] or null: external wrench per declared link, (force, torque about the centre of mass),
                            * world axes (row 6*LinkDev::fext_row + k) */
+  double *mp;             /* [10*nmp][ld] or null: mass properties per declared link, (mass, centre of mass, inertia about the centre
+                           * of mass xx xy xz yy yz zz), link axes (row 10*ModelDev::mp_row[i] + k) */
 };
 
 }  // namespace rkfd
