@@ -1,7 +1,7 @@
-"""TEST-ONLY references for external wrenches (rkFDBatchSetExtWrench): the oracle with a wrench per link
-(tests/ext_wrench/ork_ext_wrench.c) and the host harness of the kernel core with StateDev::fext
-(tests/ext_wrench/hostsim_ext_wrench.cpp).  Both compile the unchanged oracle / harness sources into libraries of their own, in
-a temporary directory, and work on worlds and harness objects made by the usual ones."""
+"""TEST-ONLY reference for external wrenches (rkFDBatchSetExtWrench): the oracle with a wrench per link
+(tests/ext_wrench/ork_ext_wrench.c), which compiles the unchanged oracle source into a library of its own, in a temporary
+directory, and works on worlds made by the usual one.  The host harness of the kernel core takes the wrenches itself
+(hostsim_py.HostSim(..., ext_links=...))."""
 import atexit
 import ctypes as C
 import os
@@ -11,11 +11,9 @@ import tempfile
 
 import numpy as np
 
-from hostsim_py import HostSim
 from oracle.oracle import OracleWorld
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-_CSRC = os.path.join(os.path.dirname(_HERE), "roki-fd_b200", "csrc")
 _vp, _dp, _ip = C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_int)
 _LIBS = {}
 NDOF = {"fixed": 0, "revolute": 1, "prismatic": 1, "spherical": 3, "float": 6, "cylindrical": 2, "hooke": 2, "breakablefloat": 6}
@@ -126,35 +124,3 @@ def oracle_run(w, q, qd, u, links, W, nsteps):
         out[3][e] = env.pivot_bits(w)
     return out
 
-
-def hostsim_lib():
-    L = _build("libhostsim_ext_wrench.so", ["/usr/bin/g++", "-O2", "-mfma", "-ffp-contract=off", "-std=c++17", "-fPIC", "-shared",
-                                            "-I" + _CSRC, os.path.join(_HERE, "ext_wrench", "hostsim_ext_wrench.cpp"),
-                                            os.path.join(_CSRC, "rkfd_model.cpp")])
-    L.hostsim_ext_declare.argtypes = [_vp, C.c_int, _ip]
-    L.hostsim_ext_set.argtypes = [_vp, _dp]
-    L.hostsim_ext_nfext.argtypes = [_vp]
-    return L
-
-
-def hostsim(world, B, links=None, spec=None):
-    """a HostSim of the kernel core; links: the links that take an external wrench (set_ext_wrench(hs, W))"""
-    hs = HostSim(world, B, spec=spec)
-    if links is not None:
-        li = np.ascontiguousarray(links, np.int32).reshape(-1)
-        if hostsim_lib().hostsim_ext_declare(hs.h, li.shape[0], li.ctypes.data_as(_ip)) != 0:
-            raise RuntimeError("external wrench declaration refused")
-    return hs
-
-
-def spec_mask(hs):
-    from hostsim_py import lib
-    return lib().hostsim_spec_mask(hs.h)
-
-
-def set_ext_wrench(hs, W):
-    """W (B, nfext, 6): force at the centre of mass, torque about it, world axes"""
-    L = hostsim_lib()
-    W, pw = _d(W)
-    assert W.size == hs.B * 6 * L.hostsim_ext_nfext(hs.h)
-    L.hostsim_ext_set(hs.h, pw)

@@ -1,6 +1,7 @@
 /* hostsim.cpp - TEST-ONLY host harness: compiles the kernel core (roki-fd_b200/csrc/rkfd_core.cuh)
- * with g++ and runs it one environment at a time on the CPU, so that the arithmetic of the sm_100a
- * kernel can be checked against the oracle where no GPU exists (`-m "not gpu"` tests).
+ * and the link kinematics walk (rkfd_kin.cuh) with g++ and runs them one environment at a time on
+ * the CPU, so that the arithmetic of the sm_100a kernels can be checked against the oracle where no
+ * GPU exists (`-m "not gpu"` tests).
  * It is NOT part of the product: librokifd_b200.so does not contain it and nothing under
  * roki-fd_b200/ loads it.  The product path has no CPU fallback. */
 #include <cmath>
@@ -12,6 +13,7 @@
 #define RKFD_VOL_STATS
 static long long rkfd_vol_stats[8];
 #include "rkfd_core.cuh"
+#include "rkfd_kin.cuh"
 #include "rkfd_model.h"
 
 using namespace rkfd;
@@ -93,11 +95,17 @@ void hostsim_set_prp(HostSim *h, double dt, int pyramid, double fw, int max_iter
 { h->world.dt = dt; h->world.pyramid = pyramid; h->world.friction_weight = fw; h->world.max_iter = max_iter; h->world.solver = solver;
   if( solver == S_VOLUME ) h->world.cidef.L = 0.001; }
 void hostsim_set_integrator(HostSim *h, int integrator){ h->world.integrator = integrator; }
+/* links that take per-environment rows, in the order of the rows; kind 0: external wrench, 1: mass properties.  Before
+ * hostsim_finalize, which checks the list */
+void hostsim_declare(HostSim *h, int kind, int n, const int *links)
+{ (kind == 0 ? h->world.fext_links : h->world.mp_links).assign(links, links + n); }
 
-/* returns 0 on success */
+/* returns 0 on success.  As the engine: the external wrenches start at zero and the mass-property rows of every environment
+ * with the model's own values */
 int hostsim_finalize(HostSim *h, int B)
 {
-  if( !build_model(h->world, h->model, h->err) ) return 1;
+  std::vector<double> def;
+  if( !build_model(h->world, h->model, h->err, &def) ) return 1;
   const ModelDev &m = h->model; h->B = B;
   const int nq = m.nq > 0 ? m.nq : 1, nl = m.nl > 0 ? m.nl : 1, ns = m.nslot > 0 ? m.nslot : 1;
   StateDev &st = h->st; std::memset(&st, 0, sizeof st); st.B = B; st.ld = B;
@@ -106,6 +114,11 @@ int hostsim_finalize(HostSim *h, int B)
   st.piv_type = halloc<unsigned int>(h, B); st.cflags = halloc<unsigned long long>(h, (size_t)(m.nfw > 0 ? m.nfw : 1)*B);
   st.ws1 = halloc<double>(h, (size_t)(m.ws1_doubles > 0 ? m.ws1_doubles : 1)*B);
   st.cref = halloc<double>(h, (size_t)3*ns*B); st.cf = halloc<double>(h, (size_t)3*ns*B); st.status = halloc<int>(h, B);
+  if( m.nfext > 0 ) st.fext = halloc<double>(h, (size_t)6*m.nfext*B);
+  if( m.nmp > 0 ){
+    st.mp = halloc<double>(h, (size_t)10*m.nmp*B);
+    for(int k=0;k<10*m.nmp;k++) for(int e=0;e<B;e++) st.mp[(size_t)k*B+e] = def[k];
+  }
   return 0;
 }
 const char *hostsim_error(HostSim *h){ return h->err.c_str(); }
@@ -131,6 +144,20 @@ void hostsim_set_state(HostSim *h, const double *q, const double *qd, const doub
     if( u ) for(int j=0;j<nl;j++) h->st.u[(size_t)j*B+e] = u[(size_t)e*nl+j];
   }
 }
+/* the wrench of every environment, env-major w[B][nfext][6]: (force at the centre of mass, torque about it), world axes */
+void hostsim_ext_set(HostSim *h, const double *w)
+{
+  const int n = 6*h->model.nfext, B = h->B;
+  for(int e=0;e<B;e++) for(int k=0;k<n;k++) h->st.fext[(size_t)k*B+e] = w[(size_t)e*n+k];
+}
+int hostsim_ext_nfext(HostSim *h){ return h->model.nfext; }
+/* the mass properties of every environment, env-major mp[B][nmp][10] */
+void hostsim_mp_set(HostSim *h, const double *mp)
+{
+  const int n = 10*h->model.nmp, B = h->B;
+  for(int e=0;e<B;e++) for(int k=0;k<n;k++) h->st.mp[(size_t)k*B+e] = mp[(size_t)e*n+k];
+}
+int hostsim_mp_nmp(HostSim *h){ return h->model.nmp; }
 void hostsim_get_state(HostSim *h, double *q, double *qd, double *qdd)
 {
   const int nq = h->model.nq, B = h->B;
@@ -176,6 +203,40 @@ void hostsim_run(HostSim *h, int mode, int nsteps)
     h->last_ws = ctx.wsp;
   }
   if( mode == 0 && (nsteps & 1) ) h->cur ^= 1;
+}
+
+/* the kinematics walk of rkFDBatchGetLinkFrames on the model: frames [B][nlink][12] and velocities [B][nlink][6] (either may
+ * be null) of links[0..nlink) (null: all) at the env-major states q, qd [B][nq] and pivot words piv [B] (null: none broken).
+ * B is the caller's, not the harness's.  Returns 1 when kin_table refuses the list. */
+int hostsim_link_frames(HostSim *h, int B, const double *q, const double *qd, const unsigned *piv, int nlink, const int *links,
+                        double *frame, double *vel)
+{
+  KinDev t;
+  if( !kin_table(h->model, nlink, links, t, h->err) ) return 1;
+  const int nq = h->model.nq;
+  struct Row {
+    const double *qr, *qdr; unsigned pv;
+    double q(int k) const { return qr[k]; }
+    double qd(int k) const { return qdr[k]; }
+    unsigned piv() const { return pv; }
+  };
+  struct Keep {
+    std::vector<double> v;
+    double ld(int s, int c) const { return v[(size_t)s*KIN_KEEP + c]; }
+    void st(int s, int c, double x){ v[(size_t)s*KIN_KEEP + c] = x; }
+  };
+  struct Out {
+    double *f, *v;
+    void frame(int k, int c, double x){ f[12*k + c] = x; }
+    void vel(int k, int c, double x){ v[6*k + c] = x; }
+  };
+  for(int e=0;e<B;e++){
+    const Row S{q + (size_t)e*nq, qd + (size_t)e*nq, piv ? piv[e] : 0u};
+    Keep K; K.v.assign((size_t)KIN_KEEP*(t.nkeep + 1), std::nan(""));     /* read-before-write shows up as NaN */
+    Out O{frame ? frame + (size_t)e*12*nlink : nullptr, vel ? vel + (size_t)e*6*nlink : nullptr};
+    kin_walk(t, S, K, O, frame != nullptr, vel != nullptr);
+  }
+  return 0;
 }
 
 /* debugging aid: the rigid-contact workspace of the last environment processed */

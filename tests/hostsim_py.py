@@ -1,4 +1,4 @@
-"""ctypes wrapper of the TEST-ONLY host harness of the kernel core (tests/hostsim/hostsim.cpp)."""
+"""ctypes wrapper of the TEST-ONLY host harness of the kernel core and the link kinematics walk (tests/hostsim/hostsim.cpp)."""
 import ctypes as C
 import os
 import subprocess
@@ -20,7 +20,8 @@ def lib():
     if _LIB is None:
         so = os.path.join(_SRC, "libhostsim.so")
         deps = [os.path.join(_SRC, "hostsim.cpp")] + [os.path.join(_CSRC, f) for f in
-                                                     ("rkfd_core.cuh", "rkfd_volume.cuh", "rkfd_math.cuh", "rkfd_types.h", "rkfd_model.cpp", "rkfd_model.h")]
+                                                     ("rkfd_core.cuh", "rkfd_volume.cuh", "rkfd_kin.cuh", "rkfd_math.cuh", "rkfd_types.h",
+                                                      "rkfd_model.cpp", "rkfd_model.h")]
         if not os.path.exists(so) or any(os.path.getmtime(d) > os.path.getmtime(so) for d in deps):
             subprocess.check_call(["/usr/bin/g++", "-O2", "-mfma", "-ffp-contract=off", "-std=c++17", "-fPIC", "-shared", "-I" + _CSRC,
                                    os.path.join(_SRC, "hostsim.cpp"), os.path.join(_CSRC, "rkfd_model.cpp"), "-o", so])
@@ -31,6 +32,7 @@ def lib():
         L.hostsim_add_box.argtypes = [C.c_void_p, C.c_int, C.c_int, _dp, C.c_double, C.c_double, C.c_double]
         L.hostsim_add_contact_info.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int] + [C.c_double] * 6
         L.hostsim_set_prp.argtypes = [C.c_void_p, C.c_double, C.c_int, C.c_double, C.c_int, C.c_int]
+        L.hostsim_declare.argtypes = [C.c_void_p, C.c_int, C.c_int, _ip]
         L.hostsim_finalize.argtypes = [C.c_void_p, C.c_int]
         L.hostsim_error.restype = C.c_char_p
         L.hostsim_error.argtypes = [C.c_void_p]
@@ -38,9 +40,12 @@ def lib():
         L.hostsim_spec_match.argtypes = [C.c_void_p, C.c_int]
         L.hostsim_spec_mask.restype = C.c_uint
         L.hostsim_spec_mask.argtypes = [C.c_void_p]
-        for f in ("hostsim_nq", "hostsim_nl", "hostsim_nslot", "hostsim_nscratch", "hostsim_free"):
+        for f in ("hostsim_nq", "hostsim_nl", "hostsim_nslot", "hostsim_nscratch", "hostsim_ext_nfext", "hostsim_mp_nmp", "hostsim_free"):
             getattr(L, f).argtypes = [C.c_void_p]
         L.hostsim_set_state.argtypes = [C.c_void_p, _dp, _dp, _dp]
+        L.hostsim_ext_set.argtypes = [C.c_void_p, _dp]
+        L.hostsim_mp_set.argtypes = [C.c_void_p, _dp]
+        L.hostsim_link_frames.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 3 + [C.c_int] + [C.c_void_p] * 3
         L.hostsim_get_state.argtypes = [C.c_void_p, _dp, _dp, _dp]
         L.hostsim_get_contact.argtypes = [C.c_void_p, _ip, _ip, _dp, _dp]
         L.hostsim_get_pivot.argtypes = [C.c_void_p, _ip, _dp]
@@ -56,7 +61,10 @@ def _d(a):
 
 
 class HostSim:
-    def __init__(self, world, B, spec=None):
+    """B environments of `world` on the kernel core.  ext_links / mp_links: the links that take an external wrench
+    (set_ext_wrench, zero until set) / per-environment mass properties (set_mass_prop, the model's own values until set)"""
+
+    def __init__(self, world, B, spec=None, ext_links=None, mp_links=None):
         L = lib()
         links, nls = [], []
         for ch in world.chains:          # all chains (static ones included), chain-local parents
@@ -86,7 +94,11 @@ class HostSim:
         L.hostsim_set_prp(self.h, world.dt, world.pyramid, world.friction_weight, world.max_iter, SOLVER[world.solver])
         L.hostsim_set_integrator.argtypes = [C.c_void_p, C.c_int]
         L.hostsim_set_integrator(self.h, {"RKG": 0, "RK4": 1, "Euler": 2, "Heun": 3}[getattr(world, "integrator", "RKG")])
-        if L.hostsim_finalize(self.h, B) != 0:
+        for kind, links in ((0, ext_links), (1, mp_links)):
+            if links is not None:
+                li = np.ascontiguousarray(links, np.int32).reshape(-1)
+                L.hostsim_declare(self.h, kind, li.shape[0], li.ctypes.data_as(_ip))
+        if L.hostsim_finalize(self.h, B) != 0:       # also refuses a declared link list
             raise RuntimeError(L.hostsim_error(self.h).decode())
         self.B, self.nq, self.nl, self.nslot = B, L.hostsim_nq(self.h), L.hostsim_nl(self.h), L.hostsim_nslot(self.h)
         self.nscratch = L.hostsim_nscratch(self.h)
@@ -111,6 +123,35 @@ class HostSim:
         if u is not None:
             _, pu = _d(u)
         lib().hostsim_set_state(self.h, pq, pqd, pu)
+
+    def set_ext_wrench(self, W):
+        """W (B, nfext, 6): force at the centre of mass, torque about it, world axes"""
+        W, pw = _d(W)
+        assert W.size == self.B * 6 * lib().hostsim_ext_nfext(self.h)
+        lib().hostsim_ext_set(self.h, pw)
+
+    def set_mass_prop(self, MP):
+        """MP (B, nmp, 10)"""
+        MP, pm = _d(MP)
+        assert MP.size == self.B * 10 * lib().hostsim_mp_nmp(self.h)
+        lib().hostsim_mp_set(self.h, pm)
+
+    def link_frames(self, q, qd, piv_type=None, links=None, frames=True, vel=True):
+        """the kinematics walk of rkFDBatchGetLinkFrames: frames (B, n, 12) and velocities (B, n, 6) of `links` (None: all) at
+        env-major states of any B; piv_type: per-dof pivot bits (B, nq)"""
+        q, qd = np.ascontiguousarray(q, np.float64), np.ascontiguousarray(qd, np.float64)
+        B = q.shape[0]
+        pv = None
+        if piv_type is not None:
+            pv = (piv_type.astype(np.uint64) << np.arange(piv_type.shape[1], dtype=np.uint64)).sum(1).astype(np.uint32)
+        n = self.nl if links is None else len(links)
+        li = None if links is None else np.ascontiguousarray(links, np.int32)
+        fr = np.full((B, n, 12), np.nan) if frames else None
+        v = np.full((B, n, 6), np.nan) if vel else None
+        addr = lambda a: None if a is None else a.ctypes.data
+        if lib().hostsim_link_frames(self.h, B, q.ctypes.data, qd.ctypes.data, addr(pv), n, addr(li), addr(fr), addr(v)) != 0:
+            raise RuntimeError(lib().hostsim_error(self.h).decode())
+        return fr, v
 
     def get_state(self):
         n = max(self.nq, 1)

@@ -1,39 +1,11 @@
-"""TEST-ONLY helpers for per-environment mass properties (rkFDBatchSetMassProp): the host harness of the kernel core with
-StateDev::mp (tests/mass_prop/hostsim_mass_prop.cpp, compiled from the unchanged harness source into a library of its own, in a
-temporary directory) and the reference for an environment: the unchanged oracle on a copy of the world whose declared links
-carry that environment's mass, centre of mass and inertia."""
-import atexit
+"""TEST-ONLY helpers for per-environment mass properties (rkFDBatchSetMassProp): the reference for an environment, the
+unchanged oracle on a copy of the world whose declared links carry that environment's mass, centre of mass and inertia, and
+the rows the tests set.  The host harness of the kernel core takes the rows itself (hostsim_py.HostSim(..., mp_links=...))."""
 import copy
-import ctypes as C
-import os
-import shutil
-import subprocess
-import tempfile
 
 import numpy as np
 
-from hostsim_py import HostSim
 from oracle.oracle import OracleWorld
-
-_HERE = os.path.dirname(os.path.abspath(__file__))
-_CSRC = os.path.join(os.path.dirname(_HERE), "roki-fd_b200", "csrc")
-_vp, _dp, _ip = C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_int)
-_LIB = []
-
-
-def hostsim_lib():
-    if not _LIB:
-        tmp = tempfile.mkdtemp(prefix="rkfd_mass_prop_")
-        atexit.register(shutil.rmtree, tmp, True)
-        so = os.path.join(tmp, "libhostsim_mass_prop.so")
-        subprocess.check_call(["/usr/bin/g++", "-O2", "-mfma", "-ffp-contract=off", "-std=c++17", "-fPIC", "-shared", "-I" + _CSRC,
-                               os.path.join(_HERE, "mass_prop", "hostsim_mass_prop.cpp"), os.path.join(_CSRC, "rkfd_model.cpp"), "-o", so])
-        L = C.CDLL(so)
-        L.hostsim_mp_declare.argtypes = [_vp, C.c_int, _ip]
-        L.hostsim_mp_set.argtypes = [_vp, _dp]
-        L.hostsim_mp_nmp.argtypes = [_vp]
-        _LIB.append(L)
-    return _LIB[0]
 
 
 def row(mass, com, inertia):
@@ -46,30 +18,6 @@ def own_rows(w, links):
     """(n, 10): the model's own mass properties of `links`"""
     fl = w.flat_links()
     return np.array([row(fl[l].mass, fl[l].com, 0.5 * (np.asarray(fl[l].inertia) + np.asarray(fl[l].inertia).T)) for l in links])
-
-
-def hostsim(world, B, links=None, spec=None, ext_links=None):
-    """a HostSim of the kernel core; links: the links that take mass properties (set_mass_prop(hs, MP)), ext_links: the links that
-    take an external wrench (ext_wrench_py.set_ext_wrench after this)"""
-    hs = HostSim(world, B, spec=spec)
-    if ext_links is not None:
-        from ext_wrench_py import hostsim_lib as ext_lib
-        li = np.ascontiguousarray(ext_links, np.int32).reshape(-1)
-        if ext_lib().hostsim_ext_declare(hs.h, li.shape[0], li.ctypes.data_as(_ip)) != 0:
-            raise RuntimeError("external wrench declaration refused")
-    if links is not None:
-        li = np.ascontiguousarray(links, np.int32).reshape(-1)
-        if hostsim_lib().hostsim_mp_declare(hs.h, li.shape[0], li.ctypes.data_as(_ip)) != 0:
-            raise RuntimeError("mass property declaration refused")
-    return hs
-
-
-def set_mass_prop(hs, MP):
-    """MP (B, nmp, 10)"""
-    L = hostsim_lib()
-    MP = np.ascontiguousarray(MP, np.float64)
-    assert MP.size == hs.B * 10 * L.hostsim_mp_nmp(hs.h)
-    L.hostsim_mp_set(hs.h, MP.ctypes.data_as(_dp))
 
 
 def world_with(w, links, rows):

@@ -10,9 +10,10 @@ import rokifd_b200  # noqa: F401
 from rokifd_b200 import capi
 from rokifd_b200 import chains as ch
 import ref_numpy as rn
-from ext_wrench_py import OracleEnvWrench, oracle_run, hostsim, set_ext_wrench, spec_mask
+from ext_wrench_py import OracleEnvWrench, oracle_run
 from hostsim_py import HostSim
 from oracle.oracle import OracleWorld
+from workloads import brick_wall_world, free_body, workload
 
 NDOF = rn.NDOF
 
@@ -72,11 +73,6 @@ def test_oracle_matches_newton_euler(seed):
         assert np.allclose(qdd, ref, rtol=1e-9, atol=1e-9 * max(1.0, np.abs(ref).max())), (seed, root)
 
 
-def free_body(com=(0.03, -0.02, 0.05)):
-    I = np.array([[0.02, 0.003, -0.001], [0.003, 0.03, 0.002], [-0.001, 0.002, 0.04]])
-    return ch.World(chains=[ch.ChainModel("body", [ch.Link(name="b", jtype="float", mass=1.7, com=np.array(com), inertia=I)])])
-
-
 def test_hovering_body_stays_put():
     """f = (0, 0, m g) at the centre of mass cancels gravity: a free body at rest stays at rest, 1,000 steps"""
     w = free_body()
@@ -122,64 +118,22 @@ def test_axis_torque_equals_motor_torque():
     assert np.allclose(a1, a2, rtol=0, atol=1e-12 * max(1.0, np.abs(a1).max())), np.abs(a1 - a2).max()
 
 
-def brick_wall_world():
-    from test_kernel_core_host import brick_wall
-    return ch.World(chains=[brick_wall([200.0, 200.0, 20.0], [200.0, 200.0, 200.0]), ch.floor_soft()],
-                    contact_info=[ch.ContactInfo("soft", "wall", "elastic", E=1000.0, V=10.0)])
-
-
 @pytest.mark.parametrize("push,breaks", [(30.0, True), (10.0, False)])
 def test_push_breaks_a_joint(push, breaks):
     """brick wall whose outer joint gives way at 20 N: a sideways push on the outer brick above the threshold breaks it in the
     committing evaluation; below, it holds (so does everything under gravity alone).  Host harness and oracle agree."""
-    w = brick_wall_world()
+    w = brick_wall_world([200.0, 200.0, 20.0], [200.0, 200.0, 200.0])
     B = 2
     q = np.zeros((B, w.nq)); qd = np.zeros((B, w.nq)); u = np.zeros((B, w.nl))
     W = np.zeros((B, 1, 6)); W[0, 0, 1] = push
     oq, oqd, oqdd, opiv = oracle_run(w, q, qd, u, [3], W, 0)
     assert opiv[0, 12] == int(breaks) and opiv[1, 12] == 0 and (opiv[:, [0, 6]] == 0).all()
-    hs = hostsim(w, B, [3])
-    hs.set_state(q, qd, u); set_ext_wrench(hs, W); hs.eval(ref=True)
+    hs = HostSim(w, B, ext_links=[3])
+    hs.set_state(q, qd, u); hs.set_ext_wrench(W); hs.eval(ref=True)
     assert (hs.get_pivot()[0] == opiv).all()
 
 
 # ---- the generic kernel core against the oracle --------------------------------------------------------------------------
-def workload(name):
-    """(world, links, sampler(B, seed) -> (q, qd, u, W), tolerance on q and q' relative to their largest entry)"""
-    if name == "arm_box_floor":
-        from test_kernel_core_host import flat_world, flat_states
-        w, q0 = flat_world(name, soft=True)
-        links = [3, 2]
-
-        def sample(B, seed):
-            q, qd, u = flat_states(name, w, q0, B, seed=seed)
-            return q, qd, u, np.random.default_rng(seed).uniform(-3, 3, (B, 2, 6))
-        return w, links, sample, 1e-9
-    if name == "c4_volume":
-        w = ch.world_c4_volume()
-
-        def sample(B, seed):
-            q, qd, u = ch.sample_c4_standing(w, B, seed=seed)
-            W = np.zeros((B, 1, 6)); W[:, 0, :2] = np.random.default_rng(seed).uniform(-40, 40, (B, 2))   # a shove on the trunk
-            return q, qd, u, W
-        return w, [0], sample, 1e-6
-    if name.startswith("c5"):
-        w = ch.world_c5(base_z=0.3, solver="MLCP" if name == "c5_mlcp" else "Vert")
-
-        def sample(B, seed):
-            q, qd, u = ch.sample_state(w, B, seed=seed)
-            W = np.random.default_rng(seed).uniform(-1, 1, (B, 2, 6)); W[:, 0, 2] -= 30.0      # the tip pushed into the floor
-            return q, qd, u, W
-        return w, [7, 4], sample, 1e-9 if name == "c5_mlcp" else 1e-7
-    w = ch.world_c3(base_z=0.3)
-
-    def sample(B, seed):
-        q, qd, u = ch.sample_state(w, B, seed=seed)
-        W = np.random.default_rng(seed).uniform(-10, 10, (B, 2, 6)); W[:, 0, 2] -= 20.0
-        return q, qd, u, W
-    return w, [7, 3], sample, 1e-9
-
-
 @pytest.mark.parametrize("integrator", ["RKG", "RK4"])
 @pytest.mark.parametrize("name", ["c3", "arm_box_floor", "c5_mlcp", "c5_vert", "c4_volume"])
 def test_core_matches_oracle(name, integrator):
@@ -187,8 +141,8 @@ def test_core_matches_oracle(name, integrator):
     w.integrator = integrator
     B, n = 6, 30
     q, qd, u, W = sample(B, 5)
-    hs = hostsim(w, B, links)
-    hs.set_state(q, qd, u); set_ext_wrench(hs, W); hs.eval(ref=True); hs.step(n)
+    hs = HostSim(w, B, ext_links=links)
+    hs.set_state(q, qd, u); hs.set_ext_wrench(W); hs.eval(ref=True); hs.step(n)
     hq, hqd, _ = hs.get_state()
     oq, oqd, _, _ = oracle_run(w, q, qd, u, links, W, n)
     assert (hs.get_status() == 0).all()
@@ -208,10 +162,10 @@ def test_zero_wrench_is_bit_identical(name):
     q, qd, u, _ = sample(B, 9)
     runs = []
     for decl in (None, links):
-        hs = hostsim(w, B, decl)
+        hs = HostSim(w, B, ext_links=decl)
         hs.set_state(q, qd, u)
         if decl:
-            set_ext_wrench(hs, np.zeros((B, len(links), 6)))
+            hs.set_ext_wrench(np.zeros((B, len(links), 6)))
         hs.eval(ref=True); hs.step(20)
         runs.append(hs.get_state() + hs.get_contact()[3:])
     for a, b in zip(*runs):
@@ -221,7 +175,7 @@ def test_zero_wrench_is_bit_identical(name):
 def test_declared_world_takes_no_arm_specialisation():
     w = ch.world_c3(base_z=0.3)
     assert HostSim(w, 1).spec_mask != 0
-    assert spec_mask(hostsim(w, 1, [7])) == 0
+    assert HostSim(w, 1, ext_links=[7]).spec_mask == 0
 
 
 # ---- C-ABI argument checks (no device needed) --------------------------------------------------------------------------

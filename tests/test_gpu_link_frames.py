@@ -5,50 +5,18 @@ import numpy as np
 import pytest
 
 import rokifd_b200  # noqa: F401
-from rokifd_b200 import chains as ch
-from test_link_frames_host import assert_frames_close, broken_links, oracle_frames, random_world
-from test_gpu_reset import brick_wall_world, brick_wall_states, num_shards, snapshot, assert_same, pick
+from gpu_batch import capi, start, steps, snapshot, assert_same, pick, num_shards  # noqa: F401
+from workloads import assert_frames_close, broken_links, oracle_frames, world
 
 pytestmark = pytest.mark.gpu
 
-
-@pytest.fixture(scope="module")
-def capi():
-    from rokifd_b200 import capi as c
-    assert c.device_count() > 0, "no CUDA device: the product path has no CPU fallback"
-    return c
+BATCH = {"c2": 1024, "c3": 1024, "c4": 256, "c5_mlcp": 1024, "arm_box_floor": 512, "random_tree": 256, "brick_wall": 256}
 
 
 def setup(name):
     """(world, B, sampler(B, seed) -> (q, qd, u))"""
-    if name == "arm_box_floor":
-        from test_kernel_core_host import flat_world, flat_states
-        w, q0 = flat_world(name, soft=True)
-        return w, 512, lambda B, seed: flat_states(name, w, q0, B, seed=seed)
-    if name == "brick_wall":
-        w = brick_wall_world()
-        return w, 256, lambda B, seed: brick_wall_states(w, B, seed)
-    if name == "random_tree":
-        w = random_world(11)
-        return w, 256, lambda B, seed: ch.sample_state(w, B, seed=seed)
-    if name == "c4":
-        w = ch.world_c4_penalty()
-        return w, 256, lambda B, seed: ch.sample_c4_standing(w, B, seed=seed)
-    w = {"c2": ch.world_c2, "c3": lambda: ch.world_c3(base_z=0.3), "c5_mlcp": lambda: ch.world_c5(base_z=0.3, solver="MLCP")}[name]()
-    return w, 1024, lambda B, seed: ch.sample_state(w, B, seed=seed)
-
-
-def start(capi, w, q, qd, u, devices=None, resort=None):
-    fd, _ = capi.create_world(w, B=q.shape[0], devices=devices)
-    if resort is not None:
-        fd.batch_set_resort_interval(resort)
-    fd.batch_set_state(q, qd); fd.batch_set_motor_input(u); fd.update_init()
-    return fd
-
-
-def steps(fd, k):
-    for _ in range(k):         # one call per step: the engine re-sorts between calls
-        fd.update()
+    w, sample = world(name)
+    return w, BATCH[name], sample
 
 
 @pytest.mark.parametrize("name", ["c2", "c3", "c4", "c5_mlcp", "arm_box_floor", "random_tree", "brick_wall"])

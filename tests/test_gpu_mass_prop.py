@@ -8,48 +8,27 @@ import pytest
 import rokifd_b200  # noqa: F401
 from rokifd_b200 import chains as ch
 import ref_numpy as rn
+from gpu_batch import capi, start, steps, state  # noqa: F401
 from mass_prop_py import oracle_run_mp, own_rows, randomise
-from test_gpu_ext_wrench import setup as wrench_setup, LINKS, TOL
+from workloads import world
 
 pytestmark = pytest.mark.gpu
 
-
-@pytest.fixture(scope="module")
-def capi():
-    from rokifd_b200 import capi as c
-    assert c.device_count() > 0, "no CUDA device: the product path has no CPU fallback"
-    return c
+LINKS = {"c2": [7], "c3": [7, 3], "c4": [0, 3], "c4_volume": [0], "c5_mlcp": [7, 4], "c5_vert": [7], "arm_box_floor": [3, 2],
+         "random_tree": [0, 5, 12], "brick_wall": [3]}
+TOL = {"c5_vert": 1e-7, "c4_volume": 1e-6}
+BATCH = {"c2": 1024, "c3": 1024, "c4": 256, "c4_volume": 512, "c5_mlcp": 1024, "c5_vert": 512, "arm_box_floor": 512,
+         "random_tree": 256, "brick_wall": 256}
 
 
 def setup(name):
     """(world, B, sampler(B, seed) -> (q, qd, u, MP)); MP: per-environment mass properties of LINKS[name]"""
-    w, B, sample_w = wrench_setup(name)
+    w, states = world(name)
 
     def sample(B, seed):
-        q, qd, u, _ = sample_w(B, seed)
+        q, qd, u = states(B, seed)
         return q, qd, u, randomise(w, LINKS[name], B, seed + 2000)
-    return w, B, sample
-
-
-def start(capi, w, q, qd, u, links, MP, devices=None, resort=None):
-    fd, _ = capi.create_world(w, B=q.shape[0], devices=devices)
-    if resort is not None:
-        fd.batch_set_resort_interval(resort)
-    if links is not None:
-        fd.batch_set_mass_prop_links(links)
-        if MP is not None:
-            fd.batch_set_mass_prop(MP)
-    fd.batch_set_state(q, qd); fd.batch_set_motor_input(u); fd.update_init()
-    return fd
-
-
-def steps(fd, k):
-    for _ in range(k):         # one call per step: the engine re-sorts between calls
-        fd.update()
-
-
-def state(fd):
-    return fd.batch_get_state() + (fd.batch_get_status(),) + tuple(fd.batch_get_contact())
+    return w, BATCH[name], sample
 
 
 @pytest.mark.parametrize("name", list(LINKS))
@@ -58,7 +37,7 @@ def test_matches_oracle(capi, name):
     B += 37                   # a ragged batch: the last block is partly padding
     q, qd, u, MP = sample(B, 3)
     links = LINKS[name]
-    fd = start(capi, w, q, qd, u, links, MP)
+    fd = start(capi, w, q, qd, u, mp=(links, MP))
     n = 40
     steps(fd, n)
     gq, gqd, _ = fd.batch_get_state()
@@ -68,7 +47,7 @@ def test_matches_oracle(capi, name):
     for a, b, what in ((gq[sel], oq, "q"), (gqd[sel], oqd, "q'")):
         err = np.abs(a - b).max() / max(np.abs(b).max(), 1.0)
         assert err < TOL.get(name, 1e-9), (name, what, err)
-    ref = start(capi, w, q, qd, u, None, None)
+    ref = start(capi, w, q, qd, u)
     steps(ref, n)
     assert np.abs(ref.batch_get_state()[0] - gq).max() > 1e-6          # the mass properties moved the worlds
     fd.destroy(); ref.destroy()
@@ -77,7 +56,7 @@ def test_matches_oracle(capi, name):
 def test_declared_world_runs_the_generic_kernel(capi):
     w, B, sample = setup("c3")
     q, qd, u, MP = sample(256, 1)
-    plain, decl = start(capi, w, q, qd, u, None, None), start(capi, w, q, qd, u, [7], MP[:, :1])
+    plain, decl = start(capi, w, q, qd, u), start(capi, w, q, qd, u, mp=([7], MP[:, :1]))
     assert plain.kernel_variant()[3] == 5
     assert decl.kernel_variant()[3] in (0, 11)
     plain.destroy(); decl.destroy()
@@ -91,13 +70,13 @@ def test_own_values_are_bit_identical(capi, name, explicit, monkeypatch):
     w, B, sample = setup(name)
     q, qd, u, _ = sample(B, 4)
     links = LINKS[name]
-    decl = start(capi, w, q, qd, u, links, np.repeat(own_rows(w, links)[None], B, axis=0) if explicit else None)
+    decl = start(capi, w, q, qd, u, mp=(links, np.repeat(own_rows(w, links)[None], B, axis=0) if explicit else None))
     variant = decl.kernel_variant()
     steps(decl, 40)
     s_decl = state(decl)
     decl.destroy()            # one engine per variant at a time: the two worlds' scratch columns differ in size
     monkeypatch.setenv("RKFD_SPEC", str(variant[3]))
-    plain = start(capi, w, q, qd, u, None, None)
+    plain = start(capi, w, q, qd, u)
     assert plain.kernel_variant() == variant
     steps(plain, 40)
     for a, b in zip(s_decl, state(plain)):
@@ -110,9 +89,9 @@ def test_rows_follow_the_slots(capi):
     w, _, sample = setup("c3")
     B = 4096
     q, qd, u, MP = sample(B, 5)
-    runs = [start(capi, w, q, qd, u, [7, 3], MP, resort=r) for r in (1, 0)] + [start(capi, w, q, qd, u, [7, 3], MP, devices=[0, 0])]
+    runs = [start(capi, w, q, qd, u, resort=r, mp=([7, 3], MP)) for r in (1, 0)] + [start(capi, w, q, qd, u, devices=[0, 0], mp=([7, 3], MP))]
     if capi.device_count() >= 2:
-        runs.append(start(capi, w, q, qd, u, [7, 3], MP, devices=[0, 1]))
+        runs.append(start(capi, w, q, qd, u, devices=[0, 1], mp=([7, 3], MP)))
     for fd in runs:
         steps(fd, 30)
     assert runs[0].resort_count > 0
@@ -130,7 +109,7 @@ def test_device_setter_equals_host_setter(capi):
     B = 2048
     q, qd, u, MP = sample(B, 6)
     MP2 = randomise(w, [7, 3], B, 99)
-    a, b = start(capi, w, q, qd, u, [7, 3], MP), start(capi, w, q, qd, u, [7, 3], MP)
+    a, b = start(capi, w, q, qd, u, mp=([7, 3], MP)), start(capi, w, q, qd, u, mp=([7, 3], MP))
     steps(a, 20); steps(b, 20)                                  # re-sorted slots by now
     assert a.resort_count > 0
     a.batch_set_mass_prop(MP2)
@@ -156,7 +135,7 @@ def test_pending_values_enter_the_first_evaluation(capi):
     fd.batch_set_state(q, qd); fd.batch_set_motor_input(u); fd.update_init()
     with pytest.raises(RuntimeError, match="before rkFDUpdateInit"):
         fd.batch_set_mass_prop_links([7])
-    plain = start(capi, w, q, qd, u, None, None)
+    plain = start(capi, w, q, qd, u)
     gqdd, pqdd = fd.batch_get_state()[2], plain.batch_get_state()[2]
     _, _, oqdd = oracle_run_mp(w, q, qd, u, [7, 3], MP, 0)
     assert np.abs(gqdd - oqdd).max() < 1e-9 * max(np.abs(oqdd).max(), 1.0)
@@ -170,12 +149,12 @@ def test_reset_keeps_the_mass_properties(capi, name):
     w, B, sample = setup(name)
     q, qd, u, MP = sample(B, 8)
     links = LINKS[name]
-    fd, twin = start(capi, w, q, qd, u, links, MP), start(capi, w, q, qd, u, links, MP)
+    fd, twin = start(capi, w, q, qd, u, mp=(links, MP)), start(capi, w, q, qd, u, mp=(links, MP))
     steps(fd, 20); steps(twin, 20)
     envs = np.arange(3, B, 7)
     q2, qd2, u2, _ = sample(B, 9)
     fd.batch_reset_envs(envs, q2[envs], qd2[envs], u2[envs])
-    fresh = start(capi, w, q2[envs], qd2[envs], u2[envs], links, MP[envs])
+    fresh = start(capi, w, q2[envs], qd2[envs], u2[envs], mp=(links, MP[envs]))
     steps(fd, 20); steps(twin, 20); steps(fresh, 20)
     others = np.setdiff1d(np.arange(B), envs)
     sf, st_, sn = state(fd), state(twin), state(fresh)
@@ -196,7 +175,7 @@ def test_boxes_of_different_masses_settle_at_their_own_depth(capi):
     MP = np.repeat(own_rows(w, [0])[None], B, axis=0)
     MP[:, 0, 0] = m; MP[:, 0, 4:] *= (m / 0.5)[:, None]
     q = np.tile([0, 0, 0.05 + 1e-4, 0, 0, 0], (B, 1)); qd = np.zeros((B, 6))
-    fd = start(capi, w, q, qd, np.zeros((B, 1)), [0], MP)
+    fd = start(capi, w, q, qd, np.zeros((B, 1)), mp=([0], MP))
     fd.update_n(4000)
     gq, gqd, _ = fd.batch_get_state()
     depth = 0.05 - gq[:, 2]

@@ -7,15 +7,10 @@ import pytest
 
 import rokifd_b200  # noqa: F401
 from rokifd_b200 import chains as ch
+from gpu_batch import capi  # noqa: F401
+from workloads import brick_wall_world, flat_world, flat_states, mm_world, mm_states, slide_worlds, slide_states
 
 pytestmark = pytest.mark.gpu
-
-
-@pytest.fixture(scope="module")
-def capi():
-    from rokifd_b200 import capi as c
-    assert c.device_count() > 0, "no CUDA device: the product path has no CPU fallback"
-    return c
 
 
 def relerr(a, b):
@@ -703,7 +698,6 @@ def test_reference_model_files(capi, oracle, name, soft, solver):
     arm_2DoF.ztk + box.ztk + floor.ztk (example/chain/arm_box_test.c) with penalty contact, box.ztk on floor_hardsoft.ztk
     (example/chain/boxdrop_hardsoft_test.c), crawler.ztk with both tracks in slide mode on the soft half of floor_hardsoft.ztk (the
     reference's fake crawler): one committing evaluation (1e-9) and 50 free-running steps."""
-    from test_kernel_core_host import flat_world, flat_states
     w, q0 = flat_world(name, solver=solver, soft=soft)
     B = 256
     if name == "boxdrop_hardsoft":
@@ -738,7 +732,6 @@ def test_environment_resort_is_invisible(capi, name):
     inputs are written between the sorts.  The Volume world sorts every step (its default), the Vert world every 4."""
     intervals = (0, 7)
     if name == "arm_box_floor":
-        from test_kernel_core_host import flat_world, flat_states
         w, q0 = flat_world(name, soft=True)
         B = 3000
         q, qd, u = flat_states(name, w, q0, B)
@@ -784,7 +777,6 @@ def test_moving_vs_moving_contact(capi, oracle, kind):
     relative velocity of both links rkfd_util.c:42-60, force on one and its opposite on the other rkfd_util.c:268-282):
     three free boxes landing on each other (example/chain/boxdrop_test.c) and an arm pushing a free box
     (example/chain/arm_box_test.c), penalty contact, 200 free-running steps against the oracle."""
-    from test_kernel_core_host import mm_world, mm_states
     w = mm_world(kind)
     B = 512
     q, qd, u = mm_states(kind, w, B)
@@ -810,7 +802,6 @@ def test_rigid_moving_vs_moving_contact(capi, oracle, kind, solver):
     info gives example/chain/arm_box_test.c and boxdrop_test.c) - A couples the two links / chains (rkfd_vert.c:125-185,
     rkfd_mlcp.c:76-142): relative point acceleration / velocity (rkfd_util.c:42-60, 103-118), probes with the opposite unit force
     on the partner, opposite wrenches.  The committing evaluation and 100 free-running steps against the oracle."""
-    from test_kernel_core_host import mm_world, mm_states
     w = mm_world(kind, solver)
     # the dense Vert QP serves the environments of a warp one after the other, every active-set iteration with a Jacobi
     # eigen-decomposition in the per-warp workspace: small batch (two boxes lying flat on each other - 8 rigid contacts,
@@ -850,7 +841,6 @@ def test_slide_mode(capi, oracle, name):
     (rkFDShape3DSetSlideMode / -Vel / -Axis on a shape of the registered chain), belt velocity in the relative contact velocity
     (rkfd_util.c:26-40), anchors of sticking contacts riding on the belt (:218-237); penalty, MLCP and Vert; 400 steps against
     the oracle."""
-    from test_kernel_core_host import slide_worlds, slide_states
     w = slide_worlds()[name]()
     B = 256
     q, qd, u = slide_states(w, B)
@@ -869,9 +859,7 @@ def test_slide_mode(capi, oracle, name):
 def test_breakable_float_joint(capi, oracle):
     """SURVEY.md section 8(f)2: the breakable float joint of example/model/wall.ztk:51-95 ([EXT A-17]): a cantilever of three
     bricks whose middle joint gives way under gravity; 400 steps against the oracle."""
-    from test_kernel_core_host import brick_wall
-    w = ch.World(chains=[brick_wall([200.0, 4.0, 10.0], [200.0, 0.3, 10.0]), ch.floor_soft()],
-                 contact_info=[ch.ContactInfo("soft", "wall", "elastic", E=1000.0, V=10.0)])
+    w = brick_wall_world([200.0, 4.0, 10.0], [200.0, 0.3, 10.0])
     B = 256
     rng = np.random.default_rng(0)
     q = np.zeros((B, w.nq)); qd = np.zeros((B, w.nq)); u = np.zeros((B, w.nl))

@@ -6,89 +6,19 @@ import pytest
 
 import rokifd_b200  # noqa: F401
 from rokifd_b200 import chains as ch
+from gpu_batch import capi, start, steps, snapshot, assert_same, pick, num_shards  # noqa: F401
+from workloads import world
 
 pytestmark = pytest.mark.gpu
 
-
-@pytest.fixture(scope="module")
-def capi():
-    from rokifd_b200 import capi as c
-    assert c.device_count() > 0, "no CUDA device: the product path has no CPU fallback"
-    return c
-
-
-def brick_wall_world():
-    from test_kernel_core_host import brick_wall
-    return ch.World(chains=[brick_wall([200.0, 4.0, 10.0], [200.0, 0.3, 10.0]), ch.floor_soft()],
-                    contact_info=[ch.ContactInfo("soft", "wall", "elastic", E=1000.0, V=10.0)])
-
-
-def brick_wall_states(w, B, seed):
-    rng = np.random.default_rng(seed)
-    q = np.zeros((B, w.nq)); qd = np.zeros((B, w.nq)); u = np.zeros((B, w.nl))
-    q[:, 9:12] = rng.uniform(-0.05, 0.05, (B, 3))
-    return q, qd, u
+BATCH = {"c2": 4096, "c3": 4096, "c4_penalty": 2048, "c4_volume": 2048, "c5_mlcp": 4096, "c5_vert": 4096, "arm_box_floor": 2048,
+         "brick_wall": 256}
 
 
 def setup(name):
     """(world, B, sampler(B, seed) -> (q, qd, u), the world re-sorts its slots)"""
-    if name == "arm_box_floor":
-        from test_kernel_core_host import flat_world, flat_states
-        w, q0 = flat_world(name, soft=True)
-        return w, 2048, lambda B, seed: flat_states(name, w, q0, B, seed=seed), True
-    if name == "brick_wall":
-        w = brick_wall_world()
-        return w, 256, lambda B, seed: brick_wall_states(w, B, seed), True
-    if name in ("c4_volume", "c4_penalty"):
-        w = ch.world_c4_volume() if name == "c4_volume" else ch.world_c4_penalty()
-        return w, 2048, lambda B, seed: ch.sample_c4_standing(w, B, seed=seed), True
-    w = {"c2": ch.world_c2, "c3": lambda: ch.world_c3(base_z=0.3), "c5_mlcp": lambda: ch.world_c5(base_z=0.3, solver="MLCP"),
-         "c5_vert": lambda: ch.world_c5(base_z=0.3, solver="Vert")}[name]()
-    return w, 4096, lambda B, seed: ch.sample_state(w, B, seed=seed), name != "c2"
-
-
-def start(capi, w, q, qd, u, devices=None):
-    fd, _ = capi.create_world(w, B=q.shape[0], devices=devices)
-    fd.batch_set_state(q, qd); fd.batch_set_motor_input(u); fd.update_init()
-    return fd
-
-
-def steps(fd, k):
-    for _ in range(k):         # one call per step: the engine re-sorts between calls
-        fd.update()
-
-
-def snapshot(fd):
-    q, qd, qdd = fd.batch_get_state()
-    a, t, r, f = fd.batch_get_contact()
-    pt, pp = fd.batch_get_pivot()
-    return dict(q=q, qd=qd, qdd=qdd, active=a, kinetic=t, ref=r, f=f, piv_type=pt, piv_prev=pp, status=fd.batch_get_status())
-
-
-def assert_same(x, xi, y, yi, what):
-    """environments xi of snapshot x are bit-identical to environments yi of snapshot y (anchors and forces on active slots)"""
-    act = y["active"][yi] == 1
-    for k in x:
-        a, b = x[k][xi], y[k][yi]
-        if k in ("ref", "f"):
-            a, b = a * act[:, :, None], b * act[:, :, None]
-        assert np.array_equal(a, b), "%s: %s differs in %d environments" % (what, k, int((a != b).reshape(len(a), -1).any(1).sum()))
-
-
-def pick(B, frac, seed):
-    """an unsorted subset of ~frac * B environments that contains 0 and B-1"""
-    rng = np.random.default_rng(seed)
-    envs = rng.choice(np.arange(1, B - 1), max(int(frac * B) - 2, 0), replace=False)
-    envs = np.concatenate([envs, [0, B - 1]]).astype(np.int32)
-    rng.shuffle(envs)
-    return envs
-
-
-def num_shards(capi, fd):
-    n = 0
-    while capi.lib().rkFDBatchDevicePtr(fd.h, n, 0, None, None):
-        n += 1
-    return n
+    w, sample = world(name)
+    return w, BATCH[name], sample, name != "c2"
 
 
 def check_reset(capi, name, with_u, frac=0.1, devices=None, B=None):

@@ -8,6 +8,7 @@ import pytest
 
 import rokifd_b200  # noqa: F401
 import variant_matrix as vm
+from gpu_batch import capi  # noqa: F401
 
 pytestmark = pytest.mark.gpu
 
@@ -18,13 +19,6 @@ NORACLE = 48
 # kernel with its scratch in device memory, the generic kernel in shared memory only
 REFERENCES = [{"RKFD_SPEC": "0"}, {"RKFD_SPEC": "0", "RKFD_FORCE_GSCR": "1", "RKFD_FORCE_BLOCK": "64"},
               {"RKFD_SPEC": "0", "RKFD_FORCE_SMEM": "1"}]
-
-
-@pytest.fixture(scope="module")
-def capi():
-    from rokifd_b200 import capi as c
-    assert c.device_count() > 0, "no CUDA device: the product path has no CPU fallback"
-    return c
 
 
 @pytest.fixture(scope="module")

@@ -1,13 +1,14 @@
 """The sm_100a kernel core (roki-fd_b200/csrc/rkfd_core.cuh) compiled for the host by the test-only
 harness tests/hostsim, against the oracle.  This checks the kernel ARITHMETIC where no GPU exists;
 the GPU parity tests proper are in test_gpu_parity.py (-m gpu) and go through the C-ABI."""
-import os
 import numpy as np
 import pytest
 
 import rokifd_b200  # noqa: F401
 from rokifd_b200 import chains as ch
 from hostsim_py import HostSim
+from workloads import (MM_CI, brick_wall, brick_wall_world, flat_world, flat_states, mm_world, mm_states, slide_worlds,
+                       slide_states)
 
 
 def relerr(a, b):
@@ -503,34 +504,6 @@ def test_volume_pair_limit_is_flagged():
 
 
 # ---- the reference's own model files (tests/golden/flat_*.txt: what the C-ABI makes of example/model/*.ztk) -------------
-GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-
-
-def flat_world(name, solver=None, soft=False):
-    desc = ch.load_flat(os.path.join(GOLD, "flat_%s.txt" % name))
-    w = ch.world_from_flat(desc)
-    if solver:
-        w.solver = solver
-    if soft:      # every pair elastic (contactinfo.ztk's soft/body record): the penalty path on the reference's geometry
-        for ci in w.contact_info:
-            ci.type, ci.E, ci.V = "elastic", 1000.0, 10.0
-    return w, np.array(desc["init.q[0]"])
-
-
-def flat_states(name, w, q0, B, seed=0):
-    rng = np.random.default_rng(seed)
-    q = np.tile(q0, (B, 1)); qd = rng.uniform(-0.05, 0.05, (B, w.nq)); u = np.zeros((B, w.nl))
-    if name.startswith("crawler"):         # crawler.ztk on the SOFT half of floor_hardsoft.ztk (y < 0), tracks on the floor
-        q[:, 0:2] = np.array([0.0, -1.0]) + rng.uniform(-0.05, 0.05, (B, 2)); q[:, 2] = rng.uniform(-0.002, 0.004, B)    # (the body's frame: already holds z = 0.13)
-        q[:, 3:6] = rng.uniform(-0.02, 0.02, (B, 3))
-    elif name.startswith("mighty"):        # the humanoid near its registered standing pose, soles on the floor
-        q[:, 6:] += 0.002 * rng.uniform(-1, 1, (B, w.nq - 6))
-    else:                                  # arm_box_test.c: arm swung down towards the floor, box dropped next to it
-        q[:, :2] = rng.uniform(-0.3, 0.3, (B, 2)) + np.array([np.pi / 2, 0.0]); qd[:, :2] = rng.uniform(-2, 2, (B, 2))
-        q[:, 2:5] = np.array([0.0, 0.6, 0.06]) + rng.uniform(-0.02, 0.02, (B, 3)); q[:, 5:8] = rng.uniform(-0.3, 0.3, (B, 3))
-    return q, qd, u
-
-
 def test_reference_crawler_drives_in_slide_mode(oracle):
     """The reference's example/model/crawler.ztk (float body + two fixed track links, 20-vertex polyhedra) on floor_hardsoft.ztk with
     both tracks in slide mode (set through rkFDShape3DSetSlideMode/-Vel/-Axis when tests/golden/flat_crawler_on_hardsoft.txt was
@@ -571,55 +544,6 @@ def test_reference_models_step_like_the_oracle(oracle, name, soft):
 
 
 # ---- moving-vs-moving collision (SURVEY.md section 8(f)3): vertices of a cell against a box carried by another link ----------
-def mm_box(name, stuff="body"):
-    """box.ztk as a `type: box` shape: 8 collision vertices AND a box target for other bodies' vertices."""
-    return ch.ChainModel(name, [ch.Link(name="link#00", jtype="float", mass=0.5, stuff=stuff, inertia=np.eye(3) * 8.33e-4,
-                                        boxes=[((0.0, 0.0, 0.0), 0.1, 0.1, 0.1)])])
-
-
-MM_CI = [ch.ContactInfo("soft", "body", "elastic", E=1000.0, V=10.0, SF=0.5, KF=0.3),
-         ch.ContactInfo("body", "body", "elastic", E=2000.0, V=20.0, SF=0.5, KF=0.3)]
-
-
-# the same bodies with RIGID contact info between them (what the reference's default contact info gives arm_box_test.c and
-# boxdrop_test.c): the pair couples two chains in A (rkfd_vert.c:125-185, rkfd_mlcp.c:76-142)
-MM_CI_RIGID = [ch.ContactInfo("soft", "body", "elastic", E=1000.0, V=10.0, SF=0.5, KF=0.3),
-               ch.ContactInfo("body", "body", "rigid", K=1000.0, L=0.01, SF=0.5, KF=0.3)]
-
-
-def mm_world(kind, solver="Vert"):
-    rigid = kind.endswith("_rigid")
-    ci = MM_CI_RIGID if rigid else MM_CI
-    if kind.startswith("box_stack"):          # example/chain/boxdrop_test.c: boxes landing on each other (self pairs unregistered)
-        nb = 2 if rigid else 3                # rigid: 2 boxes (3 x 8 x 2 + 16 = 32 slots is the limit of the vertex solvers)
-        return ch.World(chains=[mm_box(n) for n in "abc"[:nb]] + [ch.floor_soft()], contact_info=ci, solver=solver)
-    arm = ch.arm_2dof()              # example/chain/arm_box_test.c: the arm pushes a free box lying on the floor
-    arm.links[2].boxes = [((0.2, 0.0, 0.0), 0.3, 0.1, 0.1)]
-    return ch.World(chains=[arm, mm_box("box"), ch.floor_soft()], contact_info=ci, solver=solver)
-
-
-def mm_states(kind, w, B, seed=0):
-    rng = np.random.default_rng(seed)
-    q = np.zeros((B, w.nq)); qd = np.zeros((B, w.nq)); u = np.zeros((B, w.nl))
-    if kind.startswith("box_stack"):
-        for k in range(w.nq // 6):
-            o = 6 * k
-            q[:, o:o + 2] = rng.uniform(-0.02, 0.02, (B, 2)); q[:, o + 2] = 0.05 + 0.105 * k + rng.uniform(0.0, 0.01, B)
-            q[:, o + 3:o + 6] = rng.uniform(-0.1, 0.1, (B, 3)); qd[:, o:o + 6] = rng.uniform(-0.2, 0.2, (B, 6))
-    else:
-        q[:, 0] = rng.uniform(-0.3, 0.3, B); q[:, 1] = rng.uniform(-0.3, 0.3, B); qd[:, :2] = rng.uniform(-1, 1, (B, 2))
-        # the free box starts in the path of the forearm's box primitive (link 2, centre (0.2, 0, 0) in its frame)
-        from oracle import oracle as orc
-        ow = orc.OracleWorld(w)
-        for b in range(B):
-            e = ow.env(); e.set_state(q[b], qd[b]); e.eval(False)
-            Rs, ps = e.link_frames(); R, p = Rs[2], ps[2]
-            q[b, 2:5] = p + R @ np.array([0.2, 0.0, 0.0]) + R @ np.array([0.0, 0.09, 0.0]) + rng.uniform(-0.005, 0.005, 3)
-        q[:, 5:8] = rng.uniform(-0.2, 0.2, (B, 3))
-        u[:, 1:3] = rng.uniform(-6, 6, (B, 2))
-    return q, qd, u
-
-
 @pytest.mark.parametrize("kind,solver", [("box_stack_rigid", "MLCP"), ("box_stack_rigid", "Vert"), ("arm_pushes_box_rigid", "MLCP"), ("arm_pushes_box_rigid", "Vert")])
 def test_rigid_moving_vs_moving_contact_matches_oracle(oracle, kind, solver):
     """Rigid contact info between two MOVING links: relative acceleration / velocity of the two links at the contact, probes with
@@ -710,23 +634,12 @@ def test_two_dof_joints_under_the_rigid_contact_solvers(oracle, solver):
     assert (err < 1e-8).all(), err
 
 
-def brick_wall(fth, tth):
-    """wall.ztk-like: a fixed base and three bricks sticking out sideways, held by breakable float joints (example/model/wall.ztk:51-95)."""
-    links = [ch.Link(name="base", jtype="fixed", mass=1.0, inertia=np.eye(3) * 1e-2, org_p=np.array([0, 0, 1.0]), stuff="wall")]
-    for k in range(3):
-        links.append(ch.Link(name="b%d" % k, jtype="breakablefloat", parent=k, mass=0.25, com=np.array([0.05, 0, 0]),
-                             inertia=np.diag([2.6e-4, 4.2e-4, 2.6e-4]), org_p=np.array([0.1, 0, 0]), stuff="wall",
-                             break_force=fth[k], break_torque=tth[k], shapes=[ch.box_verts(0.1, 0.05, 0.05, center=(0.05, 0, 0))]))
-    return ch.ChainModel("wall", links)
-
-
 def test_breakable_float_joint(oracle):
     """[EXT A-17] breakable float: rigid while the wrench it transmits (IA a + pA in the committing evaluation) stays under its
     thresholds, a float joint afterwards.  A cantilever of three bricks under gravity: the middle joint (0.3 N m) gives way at
     the first committing evaluation - the two outer bricks fall as ONE body (the joint between them holds: 10 N m), the inner
     brick stays.  The physics: the torque at the middle joint is the weight of two bricks at their lever arms."""
-    w = ch.World(chains=[brick_wall([200.0, 4.0, 10.0], [200.0, 0.3, 10.0]), ch.floor_soft()],
-                 contact_info=[ch.ContactInfo("soft", "wall", "elastic", E=1000.0, V=10.0)])
+    w = brick_wall_world([200.0, 4.0, 10.0], [200.0, 0.3, 10.0])
     B = 6
     rng = np.random.default_rng(0)
     q = np.zeros((B, w.nq)); qd = np.zeros((B, w.nq)); u = np.zeros((B, w.nl))
@@ -748,34 +661,6 @@ def test_breakable_float_joint(oracle):
 
 
 # ---- slide mode of collision cells (SURVEY.md section 8(f)4: the "fake crawler" of rkfd_sim.c:386-440) -------------------------
-def slide_worlds():
-    def belt(stuff, vel):       # a conveyor: static box whose link origin lies far below it, belt axis y -> surface velocity +x
-        l = ch.Link(name="belt", jtype="fixed", stuff=stuff, org_p=np.array([0, 0, -100.0]), boxes=[((0, 0, 100 - 0.2), 50.0, 5.0, 0.4)])
-        l.slides = {0: (vel, (0.0, 1.0, 0.0))}
-        return ch.ChainModel("belt", [l])
-
-    def mbox(name, slide=None):
-        l = ch.Link(name="b", jtype="float", mass=0.5, stuff="body", inertia=np.eye(3) * 8.33e-4, shapes=[ch.box_verts(0.1, 0.1, 0.1)])
-        if slide:
-            l.slides = {0: slide}
-        return ch.ChainModel(name, [l])
-    el = [ch.ContactInfo("soft", "body", "elastic", E=1000.0, V=10.0, SF=0.5, KF=0.3)]
-    rg = [ch.ContactInfo("soft", "body", "rigid", K=1000.0, L=0.01, SF=0.5, KF=0.3)]
-    return {
-        "belt_registered_second_penalty": lambda: ch.World(chains=[mbox("box"), belt("soft", 0.5)], contact_info=el),
-        "belt_registered_first_penalty": lambda: ch.World(chains=[belt("soft", 0.5), mbox("box")], contact_info=el),
-        "crawler_box_on_plain_floor_penalty": lambda: ch.World(chains=[mbox("box", (0.3, (0.0, 1.0, 0.0))), ch.floor_soft()], contact_info=el),
-        "belt_mlcp": lambda: ch.World(chains=[mbox("box"), belt("soft", 0.5)], contact_info=rg, solver="MLCP"),
-        "belt_registered_first_vert": lambda: ch.World(chains=[belt("soft", 0.5), mbox("box")], contact_info=rg, solver="Vert"),
-    }
-
-
-def slide_states(w, B, seed=1):
-    rng = np.random.default_rng(seed)
-    q = np.zeros((B, 6)); q[:, 2] = 0.05 + rng.uniform(0, 0.01, B); q[:, 3:6] = rng.uniform(-0.05, 0.05, (B, 3))
-    return q, rng.uniform(-0.2, 0.2, (B, 6)), np.zeros((B, w.nl))
-
-
 @pytest.mark.parametrize("name", list(slide_worlds()))
 def test_slide_mode_matches_oracle(oracle, name):
     """Cells in slide mode: belt velocity in the relative contact velocity (rkFDLinkAddSlideVel, rkfd_util.c:26-40) and anchors of

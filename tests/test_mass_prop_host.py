@@ -11,10 +11,9 @@ import rokifd_b200  # noqa: F401
 from rokifd_b200 import capi
 from rokifd_b200 import chains as ch
 import ref_numpy as rn
-from ext_wrench_py import set_ext_wrench, spec_mask
 from hostsim_py import HostSim
-from mass_prop_py import hostsim, set_mass_prop, oracle_run_mp, own_rows, randomise, row
-from test_ext_wrench_host import free_body, workload
+from mass_prop_py import oracle_run_mp, own_rows, randomise, row
+from workloads import free_body, workload
 
 
 def spd(rng, scale):
@@ -38,8 +37,8 @@ def test_pendulum_matches_parallel_axis_formula():
     rng = np.random.default_rng(11)
     q = rng.uniform(-3, 3, (B, 1)); qd = np.zeros((B, 1)); u = np.zeros((B, 2))
     MP = np.array([[row(rng.uniform(0.3, 5.0), rng.uniform(-0.3, 0.3, 3), spd(rng, 0.05))] for _ in range(B)])
-    hs = hostsim(w, B, [1])
-    hs.set_state(q, qd, u); set_mass_prop(hs, MP); hs.eval(ref=True)
+    hs = HostSim(w, B, mp_links=[1])
+    hs.set_state(q, qd, u); hs.set_mass_prop(MP); hs.eval(ref=True)
     hqdd = hs.get_state()[2]
     _, _, oqdd = oracle_run_mp(w, q, qd, u, [1], MP, 0)
     Ro = ch.rot_x(np.pi / 2)
@@ -60,8 +59,8 @@ def test_hovering_body_with_its_own_mass_stays_put():
     q = np.tile([0.1, -0.2, 0.5, 0.3, -0.4, 0.2], (B, 1)); qd = np.zeros((B, 6))
     MP = np.array([[row(rng.uniform(0.5, 4.0), rng.uniform(-0.1, 0.1, 3), spd(rng, 0.03))] for _ in range(B)])
     W = np.zeros((B, 1, 6)); W[:, 0, 2] = MP[:, 0, 0] * rn.G
-    hs = hostsim(w, B, [0], ext_links=[0])
-    hs.set_state(q, qd, np.zeros((B, 1))); set_mass_prop(hs, MP); set_ext_wrench(hs, W)
+    hs = HostSim(w, B, ext_links=[0], mp_links=[0])
+    hs.set_state(q, qd, np.zeros((B, 1))); hs.set_mass_prop(MP); hs.set_ext_wrench(W)
     hs.eval(ref=True); hs.step(200)
     hq, hqd, hqdd = hs.get_state()
     assert np.abs(hq - q).max() < 1e-12 and np.abs(hqd).max() < 1e-12 and np.abs(hqdd).max() < 1e-12
@@ -84,8 +83,8 @@ def test_core_matches_oracle(name, integrator):
     w, q, qd, u, MP, tol = sample_mp(name, B, 5)
     w.integrator = integrator
     links = LINKS[name]
-    hs = hostsim(w, B, links)
-    hs.set_state(q, qd, u); set_mass_prop(hs, MP); hs.eval(ref=True); hs.step(n)
+    hs = HostSim(w, B, mp_links=links)
+    hs.set_state(q, qd, u); hs.set_mass_prop(MP); hs.eval(ref=True); hs.step(n)
     hq, hqd, _ = hs.get_state()
     oq, oqd, _ = oracle_run_mp(w, q, qd, u, links, MP, n)
     assert (hs.get_status() == 0).all()
@@ -106,10 +105,10 @@ def test_own_values_are_bit_identical(name):
     links = LINKS[name]
     runs = []
     for decl, explicit in ((None, False), (links, False), (links, True)):
-        hs = hostsim(w, B, decl)
+        hs = HostSim(w, B, mp_links=decl)
         hs.set_state(q, qd, u)
         if explicit:
-            set_mass_prop(hs, np.repeat(own_rows(w, links)[None], B, axis=0))
+            hs.set_mass_prop(np.repeat(own_rows(w, links)[None], B, axis=0))
         hs.eval(ref=True); hs.step(20)
         runs.append(hs.get_state() + hs.get_contact()[3:] + (hs.get_pivot()[0],))
     for r in runs[1:]:
@@ -117,10 +116,27 @@ def test_own_values_are_bit_identical(name):
             assert np.array_equal(a, b)
 
 
+def test_declared_links_without_rows_step_like_the_undeclared_world():
+    """links declared for external wrenches and mass properties and no rows set: the harness starts them as the engine does
+    (zero wrenches, the model's own values), so the committing evaluation and 20 steps on the generic core are bit for bit
+    those of the undeclared world"""
+    w = ch.world_c3(base_z=0.1)
+    B = 4
+    q, qd, u = ch.sample_state(w, B, seed=9)
+    runs = []
+    for decl in (None, [7]):
+        hs = HostSim(w, B, ext_links=decl, mp_links=decl)
+        hs.set_state(q, qd, u); hs.eval(ref=True); hs.step(20)
+        runs.append(hs.get_state() + hs.get_contact()[3:] + (hs.get_pivot()[0],))
+    assert np.abs(runs[0][3]).max() > 0             # in contact
+    for a, b in zip(*runs):
+        assert np.array_equal(a, b)
+
+
 def test_declared_world_takes_no_arm_specialisation():
     w = ch.world_c3(base_z=0.3)
     assert HostSim(w, 1).spec_mask != 0
-    assert spec_mask(hostsim(w, 1, [7])) == 0
+    assert HostSim(w, 1, mp_links=[7]).spec_mask == 0
 
 
 # ---- C-ABI argument checks (no device needed) --------------------------------------------------------------------------

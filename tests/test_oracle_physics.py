@@ -7,6 +7,7 @@ import pytest
 import rokifd_b200  # noqa: F401
 from rokifd_b200 import chains as ch
 import ref_numpy as rn
+from workloads import slide_worlds
 
 
 def _world(chain, **kw):
@@ -596,7 +597,6 @@ def test_slide_mode_conveyor_and_crawler(oracle):
     speed 0.5 m/s, penalty contact) is dragged until it rides along at the belt speed and then STICKS (static friction: its
     anchors ride on the belt); (2) a box whose own cell is in slide mode propels itself over a plain floor in the opposite
     direction of its belt's surface velocity at the contact (a crawler), approaching the belt speed."""
-    from test_kernel_core_host import slide_worlds
     W = slide_worlds()
     e = oracle.OracleWorld(W["belt_registered_first_penalty"]()).env()
     q = np.zeros(6); q[2] = 0.05

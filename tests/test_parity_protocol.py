@@ -14,6 +14,7 @@ import pytest
 
 import rokifd_b200  # noqa: F401
 from rokifd_b200 import chains as ch
+from workloads import flat_world, flat_states, mm_world, mm_states
 
 pytestmark = pytest.mark.gpu
 B, H = 4096, 100
@@ -41,13 +42,11 @@ def _c4():
 
 
 def _flat(name, soft, solver=None):
-    from test_kernel_core_host import flat_world, flat_states
     w, q0 = flat_world(name, solver=solver, soft=soft)
     return (w,) + tuple(flat_states(name, w, q0, B, seed=20260418))
 
 
 def _mm(kind, solver="Vert"):
-    from test_kernel_core_host import mm_world, mm_states
     w = mm_world(kind, solver)
     return (w,) + tuple(mm_states(kind, w, B, seed=20260418))
 

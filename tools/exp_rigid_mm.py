@@ -2,7 +2,7 @@
 import sys, os, time; sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__)))); sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests"))
 import numpy as np, rokifd_b200
 from rokifd_b200 import capi, chains as ch
-from test_kernel_core_host import mm_world, mm_states
+from workloads import mm_world, mm_states
 B = int(sys.argv[1]) if len(sys.argv) > 1 else 32
 for kind, solver in (("arm_pushes_box_rigid", "MLCP"), ("box_stack_rigid", "MLCP"), ("arm_pushes_box_rigid", "Vert"), ("box_stack_rigid", "Vert")):
     w = mm_world(kind, solver)
