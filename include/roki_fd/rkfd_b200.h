@@ -387,6 +387,39 @@ __ROKI_FD_EXPORT long long rkFDBatchResetKernelCount(rkFD *fd);       /* gather,
 __ROKI_FD_EXPORT int rkFDBatchGetLinkFrames(rkFD *fd, int nlink, const int *links, double *frame, double *vel);
 __ROKI_FD_EXPORT int rkFDBatchGetLinkFramesDevice(rkFD *fd, int shard, int nlink, const int *links, double *frame, double *vel);
 __ROKI_FD_EXPORT long long rkFDBatchLinkFrameKernelCount(rkFD *fd);   /* kinematics launches of the calls so far */
+/* Contact wrench on links: for foot-contact observations, penalties on links that should not touch, an emulated wrist
+ * force/torque sensor.  w[env][k][6] is the net contact wrench on link links[k] from the last committing evaluation, the one
+ * whose forces rkFDBatchGetContactForce reports: the force, then the torque about the link origin (the p of
+ * rkFDBatchGetLinkFrames), both in world axes.  The reference point is the origin, not the centre of mass, because the centre
+ * of mass may differ per environment (rkFDBatchSetMassProp); the torque about another point x adds (o - x) x f, o being the
+ * origin.  The sum holds exactly the contact wrenches that evaluation pushed onto the link:
+ *   - elastic vertex contacts whose force was applied: a penalty force pointing into the surface, dot(f, n) < 0, is reported by
+ *     rkFDBatchGetContactForce but was never applied, and is left out;
+ *   - rigid vertex contacts of the MLCP and Vert solvers;
+ *   - both sides of a pair between two moving links: the vertex's link takes +f, the link carrying the box -f at the same point;
+ *   - the pair wrenches of the Volume solver, shifted from the volume centre to the link origin.
+ * It holds no external wrench (rkFDBatchSetExtWrench), gravity or joint torque; the reaction on static links is dropped, as in
+ * the reference.  A link without contact gets a zero row.
+ * Links: indices in [0, rkFDBatchLinkNum), duplicates allowed; links = NULL means all links and needs nlink ==
+ * rkFDBatchLinkNum; nlink = 0 does nothing.  nlink < 0 or > 32, an index out of range, or w = NULL with nlink > 0 is refused:
+ * a refused call writes nothing and launches nothing.
+ * Accuracy: vertex positions are recomputed from the committed q with the joint model of rkFDBatchGetLinkFrames (fresh sin/cos,
+ * where the committing evaluation rotated them), so results agree with that evaluation to rounding, not bit for bit.  The
+ * dot(f, n) < 0 decision is the kernel's: against a static box the normal is an exact column of the box rotation and the two
+ * agree except where a vertex lies within rounding of two faces (the choice of face can flip); against a box on a moving link
+ * they can differ only where |f . n| is at rounding level.
+ * Volume solver: when an environment's status word has bit 2 (more colliding pairs than the solver takes), a dropped pair's
+ * contact slots hold forces of an earlier evaluation, and its rows include them: the rows of links with Volume pairs are then
+ * unspecified.  The same holds for a pair with a vertex inside the box whose clipped contact volume is empty.
+ * rkFDBatchGetLinkContactWrench: a host array, global environment index, every shard; synchronous.
+ * rkFDBatchGetLinkContactWrenchDevice: a device buffer [Bs][nlink][6] on the device of shard `shard`, indexed by the environment
+ * local to the shard (the engine maps its re-sorted slots itself); stream-ordered on the engine's stream, without a host
+ * synchronisation or an allocation.
+ * Both need rkFDUpdateInit, write nothing of the engine's state and launch one kernel per shard they cover
+ * (rkFDBatchLinkContactKernelCount). */
+__ROKI_FD_EXPORT int rkFDBatchGetLinkContactWrench(rkFD *fd, int nlink, const int *links, double *w);
+__ROKI_FD_EXPORT int rkFDBatchGetLinkContactWrenchDevice(rkFD *fd, int shard, int nlink, const int *links, double *w);
+__ROKI_FD_EXPORT long long rkFDBatchLinkContactKernelCount(rkFD *fd);   /* launches of the calls so far */
 /* External wrenches: a force and a torque applied to links of every environment, for pushes, disturbances, tethers, drag or
  * forces from another model.  The reference has no such input (it clears every link's wrench list at each evaluation).
  * rkFDBatchSetExtWrenchLinks declares which links take one, before rkFDUpdateInit: links[0..n) are link indices in

@@ -85,7 +85,9 @@ def lib():
         "rkFDBatchResetEnvs": (ci, [vp, ci, vp, vp, vp, vp]), "rkFDBatchResetEnvsDevice": (ci, [vp, ci, ci, vp, vp, vp, vp]),
         "rkFDBatchResetKernelCount": (C.c_longlong, [vp]),
         "rkFDBatchGetLinkFrames": (ci, [vp, ci, vp, vp, vp]), "rkFDBatchGetLinkFramesDevice": (ci, [vp, ci, ci, vp, vp, vp]),
-        "rkFDBatchLinkFrameKernelCount": (C.c_longlong, [vp]), "rkFDBatchKernelVariant": (ci, [vp, ci, _ip]),
+        "rkFDBatchLinkFrameKernelCount": (C.c_longlong, [vp]), "rkFDBatchGetLinkContactWrench": (ci, [vp, ci, vp, vp]),
+        "rkFDBatchGetLinkContactWrenchDevice": (ci, [vp, ci, ci, vp, vp]), "rkFDBatchLinkContactKernelCount": (C.c_longlong, [vp]),
+        "rkFDBatchKernelVariant": (ci, [vp, ci, _ip]),
         "rkFDBatchSetExtWrenchLinks": (ci, [vp, ci, vp]), "rkFDBatchSetExtWrench": (ci, [vp, vp]), "rkFDBatchSetExtWrenchDevice": (ci, [vp, ci, vp]),
         "rkFDBatchSetMassPropLinks": (ci, [vp, ci, vp]), "rkFDBatchSetMassProp": (ci, [vp, vp]), "rkFDBatchSetMassPropDevice": (ci, [vp, ci, vp]),
         "rkFDB200DescribeModel": (ci, [vp, C.c_char_p, ci]), "rkFDBatchLastError": (C.c_char_p, []), "rkFDBatchDeviceCount": (ci, []), "rkFDB200MeasureFp64": (ci, [_dp]),
@@ -489,6 +491,33 @@ class RkFD:
     @property
     def link_frame_kernel_count(self):
         return lib().rkFDBatchLinkFrameKernelCount(self.h)
+
+    def batch_get_link_contact_wrench(self, links=None):
+        """rkFDBatchGetLinkContactWrench: net contact wrench (B, n, 6) of the last committing evaluation on links (indices in
+        flat_links() order; None: all links) - force, then torque about the link origin, world axes."""
+        if links is None:
+            n, pl = self.link_num, None
+        else:
+            pl = np.ascontiguousarray(links, np.int32).reshape(-1)
+            n = pl.shape[0]
+        w = np.zeros((self.env_num, n, 6))
+        self._ck(lib().rkFDBatchGetLinkContactWrench(self.h, n, _ptr(pl), _ptr(w)))
+        return w
+
+    def batch_get_link_contact_wrench_device(self, shard, links, ptr):
+        """rkFDBatchGetLinkContactWrenchDevice: the raw device address (e.g. torch CUDA tensor .data_ptr()) of float64
+        w[Bs][n][6] of shard `shard`, indexed by the shard's local environment; stream-ordered on the engine's stream.  links: a
+        host list of link indices (None: all links)."""
+        if links is None:
+            n, pl = self.link_num, None
+        else:
+            pl = np.ascontiguousarray(links, np.int32).reshape(-1)
+            n = pl.shape[0]
+        self._ck(lib().rkFDBatchGetLinkContactWrenchDevice(self.h, shard, n, _ptr(pl), _ptr(ptr)))
+
+    @property
+    def link_contact_kernel_count(self):
+        return lib().rkFDBatchLinkContactKernelCount(self.h)
 
     def batch_set_ext_wrench_links(self, links):
         """rkFDBatchSetExtWrenchLinks (before update_init): the links (indices in flat_links() order) that take an external

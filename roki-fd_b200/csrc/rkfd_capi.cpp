@@ -602,6 +602,25 @@ extern "C" int rkFDBatchGetLinkFramesDevice(rkFD *fd, int shard, int nlink, cons
   TRY(fi->engine->link_frames(shard, t, frame, vel));
 }
 extern "C" long long rkFDBatchLinkFrameKernelCount(rkFD *fd){ FDImpl *fi = FI(fd); return ( fi && fi->engine ) ? fi->engine->link_frame_kernels() : 0; }
+/* net contact wrench on selected links (Engine::link_contact_wrench): what the last committing evaluation pushed onto them */
+extern "C" int rkFDBatchGetLinkContactWrench(rkFD *fd, int nlink, const int *links, double *w)
+{
+  BATCH_GUARD(fd); NEED_ENGINE();
+  LcwDev t; std::string err;
+  if( !link_contact_table(fi->engine->model(), nlink, links, t, err) ) return fail("rkFDBatchGetLinkContactWrench: " + err);
+  if( nlink > 0 && !w ) return fail("rkFDBatchGetLinkContactWrench: w is needed");
+  TRY(fi->engine->link_contact_wrench_host(t, w));
+}
+extern "C" int rkFDBatchGetLinkContactWrenchDevice(rkFD *fd, int shard, int nlink, const int *links, double *w)
+{
+  BATCH_GUARD(fd); NEED_ENGINE();
+  if( shard < 0 || shard >= fi->engine->num_shards() ) return fail("rkFDBatchGetLinkContactWrenchDevice: shard index out of range");
+  LcwDev t; std::string err;
+  if( !link_contact_table(fi->engine->model(), nlink, links, t, err) ) return fail("rkFDBatchGetLinkContactWrenchDevice: " + err);
+  if( nlink > 0 && !w ) return fail("rkFDBatchGetLinkContactWrenchDevice: w is needed");
+  TRY(fi->engine->link_contact_wrench(shard, t, w));
+}
+extern "C" long long rkFDBatchLinkContactKernelCount(rkFD *fd){ FDImpl *fi = FI(fd); return ( fi && fi->engine ) ? fi->engine->link_contact_kernels() : 0; }
 /* external wrenches on declared links (Engine::set_ext_wrench): an input held like the motor input */
 extern "C" int rkFDBatchSetExtWrenchLinks(rkFD *fd, int n, const int *links)
 {

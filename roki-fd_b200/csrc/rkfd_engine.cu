@@ -19,6 +19,7 @@
 
 #include "rkfd_kernel.cuh"
 #include "rkfd_kin.cuh"
+#include "rkfd_link_contact.cuh"
 #include "rkfd_model.h"
 
 namespace rkfd {
@@ -225,6 +226,36 @@ __global__ void __launch_bounds__(KIN_MAX_THREADS) rkfd_link_frames_kernel(const
   for(int i=tid; i<ne*vw; i+=nb){ const int e = i/vw, c = i - e*vw; vel[(size_t)(perm ? perm[e0 + e] : e0 + e)*vw + c] = tv[e*vs + c]; }
 }
 
+/* ---- link contact wrenches (rkFDBatchGetLinkContactWrench) -------------------------------------------------------------
+ * The walk of rkfd_link_frames_kernel over the frame columns of the table (frames only), then link_contact_reduce
+ * (rkfd_link_contact.cuh) over the cf rows of the listed slots.  Frames, keep slots and the output rows live in shared memory;
+ * the block writes its output tile environment by environment through perm, as rkfd_link_frames_kernel does. */
+struct LcwFrDev { const double *tf; __device__ double fr(int k, int c) const { return tf[12*k + c]; } };
+struct LcwCfDev {
+  const double *cf; int ld, sl;
+  __device__ double f(int s, int a) const { return __ldg(cf + (size_t)(3*s + a)*ld + sl); }
+};
+struct LcwOutDev { double *tw; __device__ double &w(int k, int c){ return tw[6*k + c]; } };
+__global__ void __launch_bounds__(KIN_MAX_THREADS) rkfd_link_contact_wrench_kernel(const __grid_constant__ LcwDev t, const double * __restrict__ vert,
+                                                                                   const double * __restrict__ q, const unsigned int * __restrict__ piv,
+                                                                                   const double * __restrict__ cf, const int * __restrict__ perm,
+                                                                                   int B, int ld, double * __restrict__ w)
+{
+  extern __shared__ double kin_smem[];
+  const int nb = blockDim.x, tid = threadIdx.x, e0 = blockIdx.x*nb, sl = e0 + tid;
+  const int ww = 6*t.nsel, ws = ww | 1, fs = t.kin.nsel ? (12*t.kin.nsel | 1) : 0;
+  double *tw = kin_smem, *tf = tw + (size_t)nb*ws, *keep = tf + (size_t)nb*fs;
+  if( sl < B ){
+    const KinSrcDev S{q, q, piv, ld, sl}; KinKeepDev K{keep + tid, nb}; KinOutDev O{tf + (size_t)tid*fs, nullptr};
+    kin_walk(t.kin, S, K, O, true, false);
+    const LcwFrDev F{tf + (size_t)tid*fs}; const LcwCfDev C{cf, ld, sl}; LcwOutDev W{tw + (size_t)tid*ws};
+    link_contact_reduce(t, vert, F, C, W);
+  }
+  __syncthreads();
+  const int ne = min(nb, B - e0);
+  for(int i=tid; i<ne*ww; i+=nb){ const int e = i/ww, c = i - e*ww; w[(size_t)(perm ? perm[e0 + e] : e0 + e)*ww + c] = tw[e*ws + c]; }
+}
+
 /* rows k0..k0+n-1 of an SoA array <- one value per row, every environment (rkFDChainSetDis/SetVel and
  * rkJointMotorSetInput on a running simulator: the reference's cell windows alias fd->dis/vel, rkfd_sim.c:277-287) */
 __global__ void rkfd_fill_rows_kernel(double * __restrict__ dst, int ld, int B, int n, const double * __restrict__ vals)
@@ -318,6 +349,8 @@ struct Shard {
   char *rbuf = nullptr; int rcap = 0;
   /* link kinematics: the host path's device outputs (allocated on first use, grown when a call needs more) */
   double *kbuf = nullptr; size_t kcap = 0; bool kin_smem_attr = false;
+  /* link contact wrenches: the model's vertex coordinates (worlds with cells; uploaded once, so the device call allocates nothing) */
+  double *vert = nullptr; bool lcw_smem_attr = false;
   std::vector<void*> allocs;
 };
 
@@ -404,6 +437,10 @@ Engine::Engine(const ModelDev &model, int B, const std::vector<int> &devices, co
     if( (unsigned long long)nmax*(unsigned long long)s->ld >= (1ull << 32) )
       throw std::runtime_error("rokifd_b200: rows x environments per device exceed 2^32 elements - spread the batch over more devices (rkFDBatchSetDevices)");
     s->nstage = (size_t)nmax*s->B; if( s->nstage < 256 ) s->nstage = 256; s->dstage = dalloc<double>(*s, s->nstage);
+    if( model.ncell > 0 ){
+      s->vert = dalloc<double>(*s, (size_t)3*model.nvert);
+      CK(cudaMemcpy(s->vert, model.vert, (size_t)3*model.nvert*sizeof(double), cudaMemcpyHostToDevice));
+    }
     if( st.mp ){    /* every slot, the padding [B, ld) too, starts with the model's own mass properties */
       CK(cudaMemcpy(s->dstage, mp_default, (size_t)10*model.nmp*sizeof(double), cudaMemcpyHostToDevice));
       rkfd_fill_rows_kernel<<<s->ld/256, 256>>>(st.mp, s->ld, s->ld, 10*model.nmp, s->dstage);
@@ -681,6 +718,15 @@ void Engine::kin_launch(Shard &s, const KinDev &t, double *frame, double *vel)
   kin_kernels_++;
 }
 
+/* Shard::kbuf holds at least n doubles (the host paths' device outputs) */
+static void kbuf_reserve(Shard &s, size_t n)
+{
+  if( n <= s.kcap ) return;
+  CK(cudaStreamSynchronize(s.stream));      /* an earlier call's copies may still read the old buffer */
+  CK(cudaFree(s.kbuf)); s.kbuf = nullptr; s.kcap = 0;
+  CK(cudaMalloc(&s.kbuf, n*sizeof(double))); s.kcap = n;
+}
+
 void Engine::link_frames(int si, const KinDev &t, double *frame, double *vel)
 {
   if( si < 0 || si >= (int)shards_.size() ) throw std::runtime_error("rokifd_b200: link frames: shard index out of range");
@@ -697,16 +743,49 @@ void Engine::link_frames_host(const KinDev &t, double *frame, double *vel)
   int prev = 0; CK(cudaGetDevice(&prev));
   for(Shard *s : shards_){
     CK(cudaSetDevice(s->dev));
-    const size_t need = (size_t)s->B*((frame ? fw : 0) + (vel ? vw : 0));
-    if( need > s->kcap ){
-      CK(cudaStreamSynchronize(s->stream));      /* an earlier call's copies may still read the old buffer */
-      CK(cudaFree(s->kbuf)); s->kbuf = nullptr; s->kcap = 0;
-      CK(cudaMalloc(&s->kbuf, need*sizeof(double))); s->kcap = need;
-    }
+    kbuf_reserve(*s, (size_t)s->B*((frame ? fw : 0) + (vel ? vw : 0)));
     double *df = frame ? s->kbuf : nullptr, *dv = vel ? s->kbuf + ( frame ? (size_t)s->B*fw : 0 ) : nullptr;
     kin_launch(*s, t, df, dv);
     if( frame ) CK(cudaMemcpyAsync(frame + (size_t)s->e0*fw, df, (size_t)s->B*fw*sizeof(double), cudaMemcpyDeviceToHost, s->stream));
     if( vel ) CK(cudaMemcpyAsync(vel + (size_t)s->e0*vw, dv, (size_t)s->B*vw*sizeof(double), cudaMemcpyDeviceToHost, s->stream));
+  }
+  for(Shard *s : shards_){ CK(cudaSetDevice(s->dev)); CK(cudaStreamSynchronize(s->stream)); }
+  CK(cudaSetDevice(prev));
+}
+
+void Engine::lcw_launch(Shard &s, const LcwDev &t, double *w)
+{
+  const size_t per_env = sizeof(double)*((size_t)(6*t.nsel | 1) + ( t.kin.nsel ? (size_t)(12*t.kin.nsel | 1) : 0 ) + (size_t)KIN_KEEP*t.kin.nkeep);
+  int nb = KIN_MAX_THREADS;
+  while( nb > 32 && nb*per_env > KIN_TILE_BYTES ) nb >>= 1;
+  const size_t smem = nb*per_env;
+  if( smem > 227*1024 ) throw std::runtime_error("rokifd_b200: link contact wrench: the tile does not fit in shared memory");
+  if( smem > 48*1024 && !s.lcw_smem_attr ){
+    CK(cudaFuncSetAttribute(rkfd_link_contact_wrench_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227*1024)); s.lcw_smem_attr = true; }
+  rkfd_link_contact_wrench_kernel<<<(s.B + nb - 1)/nb, nb, smem, s.stream>>>(t, s.vert, s.st.q[s.cur], s.st.piv_type, s.st.cf, s.perm, s.B, s.ld, w);
+  CK(cudaGetLastError());
+  lcw_kernels_++;
+}
+
+void Engine::link_contact_wrench(int si, const LcwDev &t, double *w)
+{
+  if( si < 0 || si >= (int)shards_.size() ) throw std::runtime_error("rokifd_b200: link contact wrench: shard index out of range");
+  if( t.nsel == 0 ) return;
+  int prev = 0; CK(cudaGetDevice(&prev)); CK(cudaSetDevice(shards_[si]->dev));
+  lcw_launch(*shards_[si], t, w);
+  CK(cudaSetDevice(prev));
+}
+
+void Engine::link_contact_wrench_host(const LcwDev &t, double *w)
+{
+  if( t.nsel == 0 ) return;
+  const size_t ww = 6*(size_t)t.nsel;
+  int prev = 0; CK(cudaGetDevice(&prev));
+  for(Shard *s : shards_){
+    CK(cudaSetDevice(s->dev));
+    kbuf_reserve(*s, (size_t)s->B*ww);
+    lcw_launch(*s, t, s->kbuf);
+    CK(cudaMemcpyAsync(w + (size_t)s->e0*ww, s->kbuf, (size_t)s->B*ww*sizeof(double), cudaMemcpyDeviceToHost, s->stream));
   }
   for(Shard *s : shards_){ CK(cudaSetDevice(s->dev)); CK(cudaStreamSynchronize(s->stream)); }
   CK(cudaSetDevice(prev));

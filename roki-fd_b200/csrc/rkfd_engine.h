@@ -95,6 +95,15 @@ class Engine {
   void link_frames_host(const KinDev &t, double *frame, double *vel);
   long long link_frame_kernels() const { return kin_kernels_; }     /* kinematics launches (one per shard and call) */
 
+  /* net contact wrench [B][nsel][6] (force, torque about the link origin; world axes) of the last committing evaluation on the
+   * output columns of table `t` (rkfd_link_contact.cuh), from the committed q and the contact forces.  Nothing of the engine's
+   * state is written.  link_contact_wrench: a device buffer of shard `shard`, indexed by the environment local to the shard;
+   * stream-ordered on the shard's stream, no allocation.  link_contact_wrench_host: a host array, global environment index,
+   * every shard; synchronous */
+  void link_contact_wrench(int shard, const LcwDev &t, double *w);
+  void link_contact_wrench_host(const LcwDev &t, double *w);
+  long long link_contact_kernels() const { return lcw_kernels_; }   /* launches (one per shard and call) */
+
   /* the step-kernel variant shard `shard` launches: v = (block, gscr, rigid, spec, minb); throws on a bad shard index */
   void kernel_variant(int shard, int v[5]) const;
 
@@ -104,11 +113,12 @@ class Engine {
   void resort(Shard &s);
   void reset_chunk(Shard &s, int n, const int *envs, const double *q, const double *qd, const double *u);
   void kin_launch(Shard &s, const KinDev &t, double *frame, double *vel);
+  void lcw_launch(Shard &s, const LcwDev &t, double *w);
   int resort_interval_ = 0;
   ModelDev model_, model_tm_;     /* model_tm_: the same table with the tensor-memory scratch map (generic TM kernel) */
   int B_;
   std::vector<Shard*> shards_;
-  long long launches_ = 0, resort_kernels_ = 0, reset_kernels_ = 0, kin_kernels_ = 0;
+  long long launches_ = 0, resort_kernels_ = 0, reset_kernels_ = 0, kin_kernels_ = 0, lcw_kernels_ = 0;
   int id_;
 };
 

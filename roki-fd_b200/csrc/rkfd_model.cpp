@@ -389,4 +389,43 @@ bool kin_table(const ModelDev &m, int nlink, const int *links, KinDev &t, std::s
   return true;
 }
 
+bool link_contact_table(const ModelDev &m, int nlink, const int *links, LcwDev &t, std::string &err)
+{
+  std::memset(&t, 0, sizeof t);
+  if( !kin_table(m, nlink, links, t.kin, err) ) return false;     /* the list rules of rkFDBatchGetLinkFrames */
+  t.nsel = nlink;
+  int cols[MAX_LINKS], ncol = 0, colof[MAX_LINKS];
+  for(int i=0;i<MAX_LINKS;i++) colof[i] = -1;
+  auto col = [&](int i){ if( colof[i] < 0 ){ colof[i] = ncol; cols[ncol++] = i; } return colof[i]; };
+  for(int b=0;b<m.nbox;b++){ LcwBoxDev &x = t.box[b]; const BoxDev &s = m.box[b];
+    std::memcpy(x.R, s.R, sizeof x.R); std::memcpy(x.p, s.p, sizeof x.p); std::memcpy(x.half, s.half, sizeof x.half); x.col = -1; }
+  for(int b=0;b<m.nmbox;b++){ LcwBoxDev &x = t.box[m.nbox + b]; const MBoxDev &s = m.mbox[b];
+    std::memcpy(x.R, s.R, sizeof x.R); std::memcpy(x.p, s.p, sizeof x.p); std::memcpy(x.half, s.half, sizeof x.half); x.col = -1; }
+  for(int k=0;k<nlink;k++){
+    const int i = links ? links[k] : k;
+    t.first[k] = k; t.ocol[k] = -1;
+    for(int j=0;j<k;j++) if( ( links ? links[j] : j ) == i ){ t.first[k] = j; break; }
+    if( t.first[k] != k ) continue;
+    for(int p=0;p<m.npair;p++){
+      const PairDev &pr = m.pair[p]; const CellDev &cl = m.cell[pr.cell];
+      const bool vol = m.solver == S_VOLUME && pr.type == C_RIGID;
+      if( vol && !pr.volbox ) continue;          /* watched only: no wrench */
+      const bool vside = cl.link == i, bside = pr.mbox >= 0 && m.mbox[pr.mbox].link == i;
+      if( !vside && !bside ) continue;
+      LcwTermDev &e = t.term[t.nterm++];
+      e.kind = vol ? LCW_VOL : ( vside ? LCW_VERT : LCW_BOX ); e.elastic = pr.type == C_ELASTIC;
+      e.sofs = pr.sofs; e.vofs = cl.vofs; e.nvert = cl.nvert; e.vcol = col(cl.link); e.acc = k;
+      e.box = pr.mbox >= 0 ? m.nbox + pr.mbox : pr.box;
+      if( pr.mbox >= 0 ) t.box[e.box].col = col(m.mbox[pr.mbox].link);
+    }
+    t.ocol[k] = colof[i];
+  }
+  for(int k=0;k<nlink;k++) t.ocol[k] = t.ocol[t.first[k]];
+  /* the walk over the frame columns (distinct links: at most MAX_LINKS) */
+  KinDev kin;
+  if( !kin_table(m, ncol, cols, kin, err) ) return false;
+  t.kin = kin;
+  return true;
+}
+
 }  // namespace rkfd

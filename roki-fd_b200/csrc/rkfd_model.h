@@ -88,5 +88,11 @@ void model_layout(ModelDev &m, bool tm);
  * (nlink < 0 or > MAX_LINKS, an index out of range). */
 bool kin_table(const ModelDev &m, int nlink, const int *links, KinDev &t, std::string &err);
 
+/* Table of the link contact-wrench readout (rkfd_link_contact.cuh) for output columns links[0..nlink): the same list rules and
+ * refusals as kin_table.  Per requested link, the (pair, side) terms that push a contact wrench onto it: the vertex slots of its
+ * cells (not the rigid non-box cells of the Volume solver, which push nothing), the box side of moving pairs whose box it
+ * carries, and its Volume box pairs; then the kinematics table of the links whose frames those terms need. */
+bool link_contact_table(const ModelDev &m, int nlink, const int *links, LcwDev &t, std::string &err);
+
 }  // namespace rkfd
 #endif

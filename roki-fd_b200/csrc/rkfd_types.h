@@ -154,6 +154,30 @@ struct KinDev {
 };
 constexpr int KIN_KEEP = 18;    /* Rw (9), pw (3), linear and angular velocity in link axes (3 + 3) */
 
+/* Contact table of the link contact-wrench readout (rkfd_link_contact.cuh, rkFDBatchGetLinkContactWrench): a __grid_constant__
+ * kernel parameter like KinDev, ~12 KB at the limits.  `kin` walks the links whose frames the readout needs (its output columns
+ * are "frame columns"): the requested links that carry cells or boxes in a pair, and the vertex-side links of moving pairs whose
+ * box sits on a requested link.  A term is one (pair, side) that pushes a wrench onto a requested link. */
+struct LcwBoxDev {
+  double R[9], p[3], half[3];   /* static box: world frame; box on a moving link: frame in that link (MBoxDev) */
+  int col;                      /* frame column of the carrying link, -1: static box */
+  int pad_;
+};
+enum LcwKind : int { LCW_VERT = 0,   /* vertex slots of a cell on the link: +f at the vertex */
+                     LCW_BOX = 1,    /* box of a moving pair on the link: -f at the vertex of the other link */
+                     LCW_VOL = 2 };  /* Volume box pair: slots (force, torque about the centre, centre) */
+struct LcwTermDev { int kind, elastic, sofs, vofs, nvert, vcol, box, acc; };   /* acc: output column that accumulates */
+constexpr int LCW_MAX_TERMS = 2*MAX_PAIRS;    /* a pair acts on at most two links */
+struct LcwDev {
+  KinDev kin;
+  int nsel;                     /* output columns (requested links, duplicates included) */
+  int nterm;
+  int first[MAX_LINKS];         /* output column k repeats column first[k] (== k: its own accumulator) */
+  int ocol[MAX_LINKS];          /* frame column of the link of output column k (the torque's reference point), -1: no term */
+  LcwBoxDev box[MAX_BOXES + MAX_MBOXES];   /* static boxes, then the boxes of moving links */
+  LcwTermDev term[LCW_MAX_TERMS];
+};
+
 /* Per-environment state in HBM, structure-of-arrays with the environment index fastest:
  * element (k, e) of an array lives at base[k*ld + e].  Thread e of a warp therefore reads
  * consecutive 8-byte words: every load/store is one fully coalesced 256-byte request. */
